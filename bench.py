@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- PDE-layer forward+backward throughput on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--layer NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--layer NAME] [--dump-outputs DIR]
 
 One "step" = one forward + backward pass of the PDE layer over one batch of synthetic input
 (u, g_out ~ N(0,1), seeded).  Headline workload: fashion_mnist.DiffusionLayer (BASELINE.json
@@ -11,9 +11,14 @@ latency; the config-batch latency is reported beside it.  Unit: cell-updates = B
 per step.  Under torchrun every rank runs its own batch (weak scaling; the only exchange is the
 all-reduce of the coefficient gradients) and rank 0 prints ONE JSON line.
 
-Every one of the K timed "steps" is INNER back-to-back passes (config.inner_repeats, sized so that the
-timed region lasts about a second: clock samples and event resolution mean something); ms_per_step
-is the time of ONE pass.  Beside the default-init weights the same batch is timed with perturbed
+The timed region is the K steps back to back inside one CUDA-event bracket (--inner N makes every
+step N passes; ms_per_step is the time of ONE pass).  At the headline batch a pass takes ~3.5 ms on a
+B200 (1000 W limit), so a window of about a second, with enough NVML clock samples for `clocks` and
+`issue_frac`, takes K ~ 300; with fewer samples `issue_frac` uses the maximum SM clock.
+--dump-outputs DIR writes what the last timed step handed its caller -- the layer output, grad_input
+and the coefficient gradients -- as DIR/<name>.npy (float32; a fixed, seeded sample of the batch where the full arrays would exceed
+64 MB), so that two builds can be compared output for output on identical inputs.
+Beside the default-init weights the same batch is timed with perturbed
 weights that put cells outside both clamp edges (`clamped`: the masked / in-sweep smoothing-adjoint
 path), and at N = 1 the CPU leg doubles as a parity self-check: the oracle runs on the very batch the
 GPU was timed on and `parity_rel_err` holds the worst relative error per output.
@@ -177,6 +182,47 @@ class ClockSampler:
                 "sm_max_mhz": self.max_mhz, "reasons": sorted(self.reasons), "samples": len(self.samples)}
 
 
+DUMP_BYTES = 64_000_000
+
+
+def timed_inputs(B, shape, dev, rank=0):
+    """The seeded batch of the timed path: input u and upstream gradient g, the same on every run with the same
+    arguments, and the generator they came from (the script-batch section keeps drawing from it)."""
+    import torch
+    gen = torch.Generator(device=dev).manual_seed(1234 + rank)
+    u = torch.randn(B, *shape, device=dev, generator=gen)
+    g = torch.randn(B, *shape, device=dev, generator=gen)
+    return u, g, gen
+
+
+def dump_rows(B, keep):
+    """The batch rows --dump-outputs keeps when it cannot keep all B: a fixed, seeded sample, in batch order."""
+    import numpy as np
+    return np.sort(np.random.default_rng(0).choice(B, size=keep, replace=False))
+
+
+def dump_outputs(out_dir, y, grad_input, layer):
+    """Write the arrays one forward + backward hands its caller as out_dir/<name>.npy (float32):
+    `out`, `grad_input` and `grad_<parameter>`.  The coefficient gradients are written whole; `out` and
+    `grad_input` keep a fixed, seeded sample of the batch (same rows in both, in batch order) when the
+    full arrays would take more than DUMP_BYTES in all."""
+    import numpy as np
+    import torch
+    grads = {"grad_" + n: p.grad for n, p in layer.named_parameters() if p.grad is not None}
+    batched = {"out": y, "grad_input": grad_input}
+    batched = {k: v for k, v in batched.items() if v is not None}
+    B = y.shape[0]
+    row_bytes = sum(v[0].numel() * 4 for v in batched.values())
+    room = DUMP_BYTES - sum(g.numel() * 4 + 1024 for g in grads.values()) - 1024 * len(batched)   # + .npy headers
+    keep = min(B, max(1, room // row_bytes))
+    if keep < B:
+        idx = torch.from_numpy(dump_rows(B, keep)).to(y.device)
+        batched = {k: v.detach().index_select(0, idx) for k, v in batched.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in {**batched, **grads}.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 # ------------------------------------------------------------------------------------------ b200
 def run_b200(args):
     import numpy as np
@@ -207,9 +253,7 @@ def run_b200(args):
     # same layer, weights perturbed so that cells sit outside both clamp edges (tests/cases.make_params)
     c_pert = K.case("bench_clamped_" + args.layer, kind, B=B, perturb=True, **ctor)
     layer_c = runners.make_cuda_layer(c_pert, device=dev)
-    gen = torch.Generator(device=dev).manual_seed(1234 + rank)
-    u = torch.randn(B, C, H, W, device=dev, generator=gen)
-    g = torch.randn(B, C, H, W, device=dev, generator=gen)
+    u, g, gen = timed_inputs(B, (C, H, W), dev, rank)
     info = P._cabi.device_info()
 
     def grads():
@@ -237,23 +281,18 @@ def run_b200(args):
     sampler = ClockSampler(index=local).start() if rank == 0 else None
     for _ in range(max(args.warmup, 3)):
         step(x)
+    inner = args.inner
     sync_all()
-    # passes per timed "step": enough for a timed region of about a second (same on every rank)
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    e0.record()
+    # one more untimed pass: the host enqueues the first timed one while the device runs it, so the bracket
+    # opens on a busy device instead of timing the host's way to the first launch
     step(x)
-    e1.record()
-    torch.cuda.synchronize()
-    t = torch.tensor([e0.elapsed_time(e1)], device=dev, dtype=torch.float64)
-    if world > 1:
-        dist.all_reduce(t, op=dist.ReduceOp.MAX)
-    inner = args.inner or max(1, min(256, int(-(-args.min_seconds * 1e3 // (args.steps * max(float(t.item()), 1e-3))))))
-    sync_all()
     if sampler:
         sampler.begin()
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    for _ in range(args.steps * inner):
+    for _ in range(args.steps * inner - 1):
         step(x)
+    y_last = step(x)
     e1.record()
     sync_all()
     clocks = sampler.stop() if sampler else None
@@ -264,6 +303,9 @@ def run_b200(args):
     ms_total = float(t.item())
     ms_per_step = ms_total / (args.steps * inner)
     value = world * cells * nsteps / (ms_per_step * 1e-3) / 1e9
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, y_last, x.grad, layer)
+    del y_last
 
     # ----------------------------------------- per-kernel timing through the C ABI (roofline)
     def time_phase(fn, n):
@@ -818,13 +860,18 @@ def main():
     ap.add_argument("--layer", default="fashion", choices=sorted(LAYERS))
     ap.add_argument("--batch", type=int, default=0, help="per-GPU batch (default: roofline-size batch of the layer)")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
-    ap.add_argument("--inner", type=int, default=0, help="passes per timed step (default: sized for --min-seconds)")
-    ap.add_argument("--min-seconds", type=float, default=1.0, help="target length of the timed region")
+    ap.add_argument("--inner", type=int, default=1, help="back-to-back passes per timed step")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (--impl b200)")
     ap.add_argument("--all-layers", type=int, default=1, help="also time the other layers (N=1 only)")
     ap.add_argument("--train", type=int, default=1, help="also time a whole-model training step (img/s)")
     ap.add_argument("--train-model", default="cifar10")
     ap.add_argument("--train-batch", type=int, default=512, help="per-GPU batch of the training step")
     args = ap.parse_args()
+    if args.steps < 1 or args.inner < 1:
+        ap.error("--steps and --inner must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU path: it needs --impl b200")
     if args.impl == "reference":
         run_reference(args)
     else:

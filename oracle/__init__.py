@@ -8,9 +8,8 @@ Only ``tests/``, ``__graft_entry__.smoke()`` and ``bench.py``'s cpu_baseline / -
 reference legs may import this package.  The product (``cnn-with-pde_b200/``) never does.
 
 Parity pinning: the reference has no tests or golden vectors of its own, so this oracle
-is pinned against the reference's Python modules imported unmodified
-(``tests/test_oracle_vs_reference.py``, runs where ``/root/reference`` exists) and against
-fixtures generated from them (``tests/golden/make_golden.py``).
+is pinned against fixtures generated from the reference's Python modules imported
+unmodified (``tests/golden/make_golden.py``).
 """
 from __future__ import annotations
 

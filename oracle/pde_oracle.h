@@ -6,9 +6,8 @@
  * --impl reference legs.  Nothing under cnn-with-pde_b200/ may include, link or call it.
  *
  * Pinning: the reference ships no tests or golden vectors ("parity unpinned" by the
- * reference itself, SURVEY.md section 8c).  This oracle is pinned instead against the
- * reference's own Python modules imported unmodified in the build container
- * (tests/test_oracle_vs_reference.py) and against fixtures generated from them
+ * reference itself, SURVEY.md section 8c).  This oracle is pinned instead against
+ * fixtures generated from the reference's own Python modules imported unmodified
  * (tests/golden/make_golden.py -> tests/golden/ npz files).
  *
  * The file pde_oracle.c is compiled twice (REAL=float / REAL=double); every entry point

@@ -1,5 +1,4 @@
 """CPU-only tests: C-ABI surface, drop-in contract of the modules, schedule, sharding."""
-import inspect
 import os
 import re
 
@@ -8,7 +7,7 @@ import pytest
 import torch
 
 from . import cases as K
-from . import refload, runners
+from . import runners
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -111,67 +110,6 @@ def test_state_dict_layout(kind):
     layer = _ours(kind)()
     assert list(layer.state_dict().keys()) == EXPECTED_KEYS[kind]
     assert all(v.dtype == torch.float32 for v in layer.state_dict().values())
-
-
-@pytest.mark.reference
-@pytest.mark.skipif(not refload.available(), reason="reference not present")
-@pytest.mark.parametrize("kind", sorted(EXPECTED_KEYS))
-def test_drop_in_contract_against_reference_class(kind):
-    script, cls = K.REF_CLASS[kind]
-    Ref = getattr(refload.load(script), cls)
-    Ours = _ours(kind)
-    # constructor: same parameter names, order and defaults
-    assert str(inspect.signature(Ref.__init__)) == str(inspect.signature(Ours.__init__))
-    # same init values AND the same RNG draws under the same seed
-    torch.manual_seed(99)
-    ref = refload.quiet(Ref)
-    torch.manual_seed(99)
-    ours = Ours()
-    sr, so = ref.state_dict(), ours.state_dict()
-    assert list(sr.keys()) == list(so.keys())
-    for k in sr:
-        assert sr[k].shape == so[k].shape and sr[k].dtype == so[k].dtype, k
-        assert torch.equal(sr[k], so[k]), k
-    assert [n for n, _ in ref.named_parameters()] == [n for n, _ in ours.named_parameters()]
-    # state dicts load across in both directions
-    ours.load_state_dict(sr)
-    ref.load_state_dict(so)
-    # plain attributes the training / plotting code reads
-    for attr in ("dx", "dy", "dt", "num_steps", "size", "channels", "stability_eps", "Nx", "Ny", "Lx", "Ly",
-                 "T", "Nt", "max_coeff", "use_implicit"):
-        if hasattr(ref, attr):
-            assert getattr(ours, attr) == getattr(ref, attr), attr
-    # helper methods give identical tensors
-    with torch.no_grad():
-        for p in list(ref.parameters()):
-            p.add_(0.3 * torch.randn_like(p))
-        ours.load_state_dict(ref.state_dict())
-        if hasattr(ref, "get_alpha_beta_at_time"):
-            for t in (0.0, 0.0037, 1.2):
-                for a, b in zip(ref.get_alpha_beta_at_time(t), ours.get_alpha_beta_at_time(t)):
-                    assert torch.equal(a, b)
-        if hasattr(ref, "get_numerical_stability_info"):
-            assert ref.get_numerical_stability_info() == ours.get_numerical_stability_info()
-        if kind == "tiny":
-            # the dormant methods (tiny_imagenet.py:88-233) exist with the reference's signatures; the general
-            # Thomas helper (arbitrary bands, PyTorch, off the path) gives the reference's numbers
-            for m in ("implicit_diffusion_step", "solve_implicit_x", "solve_implicit_y", "thomas_algorithm_batch",
-                      "diffuse_x_explicit", "diffuse_y_explicit"):
-                assert str(inspect.signature(getattr(Ref, m))) == str(inspect.signature(getattr(Ours, m))), m
-            a, b, c, d = (torch.rand(5, 9) + 0.1 for _ in range(4))
-            assert torch.equal(ref.thomas_algorithm_batch(a, b + 3, c, d), ours.thomas_algorithm_batch(a, b + 3, c, d))
-        if kind == "emotion":
-            assert torch.equal(ref.alpha(ref.y), ours.alpha(ours.y))
-            assert torch.equal(ref.beta(ref.x), ours.beta(ours.x))
-        if hasattr(ref, "apply_channel_mixing"):
-            x = torch.randn(2, 3, 32, 32)
-            assert torch.allclose(ref.apply_channel_mixing(x), ours.apply_channel_mixing(x), atol=1e-6)
-        if hasattr(ref, "apply_channel_coupling"):
-            x = torch.randn(2, 3, 32, 32)
-            assert torch.allclose(ref.apply_channel_coupling(x), ours.apply_channel_coupling(x), atol=1e-6)
-        if hasattr(ref, "smooth_coefficients"):
-            x = torch.randn(5, 28)
-            assert torch.allclose(ref.smooth_coefficients(x), ours.smooth_coefficients(x), atol=1e-7)
 
 
 def test_modules_reject_cpu_input_loudly():
