@@ -1503,8 +1503,8 @@ int forward_multi(int n, const pde_adi_desc *d, const void *const *tables, const
     }
     const int grid = deal_blocks(n, d, props.sm_count * per_sm, nitems, &m);   // the branches share the resident set
     if (debug_enabled())
-        fprintf(stderr, "[pde_b200] split fwd multi plan: n=%d N=%d C=%d P=%d Q=%d threads=%d smem=%zu occ=%d grid=%d\n", n, d[0].N,
-                d[0].C, p.P, p.Qf, p.threads, smem, per_sm, grid);
+        fprintf(stderr, "[pde_b200] split fwd multi plan: n=%d N=%d C=%d chan_op=%d P=%d Q=%d threads=%d smem=%zu occ=%d grid=%d\n", n,
+                d[0].N, d[0].C, d[0].chan_op, p.P, p.Qf, p.threads, smem, per_sm, grid);
     void *params[] = {&m};
     PDE_CUDA_TRY(cudaLaunchKernel(kern, dim3(grid), dim3(p.threads), params, smem, st));
     return cuda_last_error();
@@ -1528,6 +1528,9 @@ int backward_multi(int n, const pde_adi_desc *d, const void *const *tables, cons
     MultiArgs m{};
     m.n = n;
     const int grid = deal_blocks(n, d, props.sm_count * b.occ, b.nitems, &m);
+    if (debug_enabled())
+        fprintf(stderr, "[pde_b200] split bwd multi plan: n=%d N=%d C=%d chan_op=%d P=%d occ=%d grid=%d\n", n, d[0].N, d[0].C,
+                d[0].chan_op, p.P, b.occ, grid);
     FinishJob jobs[PDE_MAX_BRANCHES];
     for (int i = 0; i < n; ++i) {
         WsLayout w;
