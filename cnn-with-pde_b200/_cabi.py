@@ -14,7 +14,8 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # PDE_B200_LIB points at another build of the same library (A/B timing of kernel variants)
 LIB_PATH = os.environ.get("PDE_B200_LIB") or os.path.join(_HERE, "libpde_b200.so")
 MAX_SWEEPS = 192
-MAX_CHANNELS = 4
+MAX_CHANNELS = 4          # channels of the register-resident implicit kernels
+ADI_MAX_CHANNELS = 64     # bound of AdiDesc.C (implicit family)
 MAX_BRANCHES = 4
 ABI_VERSION = 3
 ERR_INVALID, ERR_UNSUPPORTED, ERR_WORKSPACE = -1, -2, -3   # include/pde_b200.h

@@ -1127,7 +1127,7 @@ static int validate(const pde_adi_desc *d) {
     if (d->B < 0 || d->C < 1 || d->N < 2 || d->steps < 0) return PDE_ERR_INVALID;
     if (d->chan_op < 0 || d->chan_op > 2) return PDE_ERR_INVALID;
     if (d->steps * sweeps_per_step(*d) > PDE_MAX_SWEEPS) return PDE_ERR_UNSUPPORTED;
-    if (d->C > PDE_MAX_CHANNELS) return PDE_ERR_UNSUPPORTED;
+    if (d->C > PDE_MAX_CHANNELS) return wide::serves(*d) ? PDE_OK : PDE_ERR_UNSUPPORTED;   // adi_wide.cu
     switch (d->N) {
         case 8: case 12: case 16: case 20: case 24: case 28: case 32: break;   // kernels compiled per plane edge
         default:
@@ -1270,7 +1270,7 @@ using namespace pde::adi;
 
 extern "C" size_t pde_adi_tables_bytes(const pde_adi_desc *d) {
     if (validate(d) != PDE_OK) return 0;
-    if (generic::serves(*d)) return generic::tables_bytes(*d);
+    if (generic::serves(*d) || wide::serves(*d)) return generic::tables_bytes(*d);   // one table layout for both
     // header | tables of adi.cu | tables of adi_split.cu (always reserved: the size does not depend
     // on which implementation a call ends up using)
     return (size_t)kHeaderBytes + (4 * table_elems(*d) + split::table_floats(*d)) * sizeof(float);
@@ -1284,13 +1284,14 @@ static size_t legacy_workspace_bytes(const pde_adi_desc *d) {
 
 extern "C" size_t pde_adi_checkpoint_bytes(const pde_adi_desc *d) {
     if (validate(d) != PDE_OK) return 0;
-    if (generic::serves(*d)) return 0;   // its backward pass replays the trajectory
+    if (generic::serves(*d) || wide::serves(*d)) return 0;   // their backward pass replays the trajectory
     return split::supported(*d) ? split::checkpoint_bytes(*d) : 0;
 }
 
 extern "C" size_t pde_adi_backward_saved_workspace_bytes(const pde_adi_desc *d) {
     if (validate(d) != PDE_OK) return 0;
     if (generic::serves(*d)) return generic::workspace_bytes(*d);
+    if (wide::serves(*d)) return wide::workspace_bytes(*d);
     if (split::supported(*d)) return split::workspace_bytes(*d);
     return legacy_workspace_bytes(d);
 }
@@ -1298,6 +1299,7 @@ extern "C" size_t pde_adi_backward_saved_workspace_bytes(const pde_adi_desc *d) 
 extern "C" size_t pde_adi_backward_workspace_bytes(const pde_adi_desc *d) {
     if (validate(d) != PDE_OK) return 0;
     if (generic::serves(*d)) return generic::workspace_bytes(*d);
+    if (wide::serves(*d)) return wide::workspace_bytes(*d);
     if (split::supported(*d)) return split::workspace_bytes(*d) + split::checkpoint_bytes(*d) + 256;
     return legacy_workspace_bytes(d);
 }
@@ -1346,7 +1348,7 @@ extern "C" int pde_adi_prepare(const pde_adi_desc *d, const pde_adi_schedule *sc
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const int S = d->steps * sweeps_per_step(*d);
     if (S == 0) return PDE_OK;   // zero steps: identity, no tables
-    if (generic::serves(*d))
+    if (generic::serves(*d) || wide::serves(*d))   // gprepare_kernel is channel-count agnostic
         return generic::prepare(*d, *sched, ab, bb, atc, btc, static_cast<char *>(tables), st);
     SlotMap sm;
     make_slot_map(*d, *sched, &sm);
@@ -1371,7 +1373,7 @@ static int multi_validate(int n, const pde_adi_desc *d) {
     for (int i = 0; i < n; ++i) {
         const int rc = validate(&d[i]);
         if (rc) return rc;
-        if (generic::serves(d[i])) return PDE_ERR_UNSUPPORTED;   // single-layer calls only
+        if (generic::serves(d[i]) || wide::serves(d[i])) return PDE_ERR_UNSUPPORTED;   // single-layer calls only
     }
     if (d[0].B == 0) return PDE_OK;
     return split::multi_compatible(n, d) ? PDE_OK : PDE_ERR_UNSUPPORTED;
@@ -1479,6 +1481,8 @@ extern "C" int pde_adi_forward_train(const pde_adi_desc *d, const void *tables, 
     if (d->skip && !skipw) return PDE_ERR_INVALID;
     if (generic::serves(*d))   // scalar accesses: no alignment requirement (odd plane edges)
         return generic::forward(*d, static_cast<const char *>(tables), u, chan, skipw, out, static_cast<cudaStream_t>(stream));
+    if (wide::serves(*d))
+        return wide::forward(*d, static_cast<const char *>(tables), u, chan, skipw, out, static_cast<cudaStream_t>(stream));
     if (!aligned16(u) || !aligned16(out)) return PDE_ERR_INVALID;
     // with checkpoints to write: the half-line kernel (its backward twin needs them); plain
     // inference: the whole-line kernel below, which is the faster forward (DESIGN.md section 4)
@@ -1558,6 +1562,9 @@ extern "C" int pde_adi_backward_saved(const pde_adi_desc *d, const void *tables,
     if (generic::serves(*d))
         return generic::backward(*d, static_cast<const char *>(tables), u, gout, chan, skipw, gin, g_ab, g_bb, g_atc, g_btc,
                                  g_chan, g_skip, workspace, workspace_bytes, st);
+    if (wide::serves(*d))
+        return wide::backward(*d, static_cast<const char *>(tables), u, gout, chan, skipw, gin, g_ab, g_bb, g_atc, g_btc,
+                              g_chan, g_skip, workspace, workspace_bytes, st);
     if (!aligned16(u) || !aligned16(gout) || (gin && !aligned16(gin))) return PDE_ERR_INVALID;
     if (d->B > 0 && split::supported(*d)) {
         const char *tb = static_cast<const char *>(tables);

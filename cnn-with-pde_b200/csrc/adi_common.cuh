@@ -185,5 +185,16 @@ int backward(const pde_adi_desc &d, const char *tables, const float *u, const fl
              float *g_skip, void *workspace, size_t workspace_bytes, cudaStream_t st);
 }  // namespace generic
 
+// adi_wide.cu: 5 ... PDE_ADI_MAX_CHANNELS channels, any edge 2 ... 128 (tables: generic::prepare / tables_bytes)
+namespace wide {
+bool serves(const pde_adi_desc &d);
+size_t workspace_bytes(const pde_adi_desc &d);          // accumulators + per-slot sweep history; 0 without a device
+int forward(const pde_adi_desc &d, const char *tables, const float *u, const float *chan, const float *skipw, float *out,
+            cudaStream_t st);
+int backward(const pde_adi_desc &d, const char *tables, const float *u, const float *gout, const float *chan,
+             const float *skipw, float *gin, float *g_ab, float *g_bb, float *g_atc, float *g_btc, float *g_chan,
+             float *g_skip, void *workspace, size_t workspace_bytes, cudaStream_t st);
+}  // namespace wide
+
 }  // namespace adi
 }  // namespace pde

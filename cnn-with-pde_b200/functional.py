@@ -150,9 +150,9 @@ class _AdiPlan:
         if self.tables_bytes == 0:
             raise _cabi.PdeB200Error(
                 f"unsupported implicit-layer configuration (size={cfg.N}, channels={cfg.C}, steps={cfg.steps}); "
-                "supported: size 2 ... 128 with channels <= 4 while channels * size * (size | 1) * 4 bytes <= 200 KB "
-                "and channels * size <= 384, "
-                "at most 64 Strang / 96 Lie steps")
+                "supported: size 2 ... 128 with channels * size * (size | 1) * 4 bytes <= 200 KB, "
+                f"channels <= {_cabi.ADI_MAX_CHANNELS} (channels <= {_cabi.MAX_CHANNELS} also needs channels * size <= 384 "
+                "unless size is 8, 12, ... 32), at most 64 Strang / 96 Lie steps")
         self.sched = adi_schedule(cfg.steps, cfg.dt, cfg.hx, cfg.hy, cfg.lie)
         self.sref = byref(self.sched)
         self.ckpt_bytes = L.pde_adi_checkpoint_bytes(self.dref)

@@ -41,7 +41,8 @@ extern "C" {
 #define PDE_ERR_WORKSPACE (-3)    /* workspace / table buffer too small or misaligned       */
 
 #define PDE_MAX_SWEEPS 192        /* 64 Strang steps or 96 Lie steps                        */
-#define PDE_MAX_CHANNELS 4        /* channel-mix registers per thread                       */
+#define PDE_MAX_CHANNELS 4        /* channels of the register-resident implicit kernels     */
+#define PDE_ADI_MAX_CHANNELS 64   /* bound of pde_adi_desc.C (implicit family)              */
 
 int pde_b200_abi_version(void);
 const char *pde_b200_error_string(int code);
@@ -56,11 +57,15 @@ int pde_b200_device_info(int *sm_count, int *cc_major, int *cc_minor, size_t *l2
  * thomas_solver_batch[_optimized], apply_channel_{mixing,coupling}).
  * ------------------------------------------------------------------------------------- */
 typedef struct pde_adi_desc {
-    int32_t B, C, N;          /* batch, channels (<= PDE_MAX_CHANNELS), plane edge H == W == N:
-                                 2 ... 128 while C * N * (N | 1) * 4 bytes <= 200 KB (one sample's
-                                 planes in one block's shared memory) and C * N <= 384 (a thread
-                                 per line); 8, 12, ... 32 have kernels compiled for them, the
-                                 rest share run-time-sized ones                                 */
+    int32_t B, C, N;          /* batch, channels, plane edge H == W == N.
+                                 C <= PDE_MAX_CHANNELS: N = 8, 12, ... 32 have kernels compiled
+                                 for them; any other N in 2 ... 128 while C * N * (N | 1) * 4
+                                 bytes <= 200 KB (one sample's planes in one block's shared
+                                 memory) and C * N <= 384 (a thread per line).
+                                 PDE_MAX_CHANNELS < C <= PDE_ADI_MAX_CHANNELS: any N in 2 ... 128
+                                 while C * N * (N | 1) * 4 bytes <= 200 KB (e.g. C <= 48 at 32 x 32,
+                                 12 at 64 x 64); no checkpoints (the backward pass replays), no
+                                 pde_adi_multi_* (PDE_ERR_UNSUPPORTED)                          */
     int32_t steps;            /* num_steps                                                   */
     int32_t lie;              /* 0 Strang x(dt/2) y(dt) x(dt/2); 1 Lie x(dt/2) y(dt/2)        */
     int32_t smooth;           /* 3-tap replicate smoothing of the clamped map along the sweep */
@@ -114,7 +119,7 @@ int pde_adi_forward(const pde_adi_desc *d, const void *tables, const float *u,
  * that is the state at the end of every step ("checkpoints": pde_adi_checkpoint_bytes(d) bytes,
  * 256-byte aligned, opaque layout), so that the backward kernel does not recompute the forward
  * trajectory.  pde_adi_checkpoint_bytes returns 0 when the configuration is served by kernels
- * that rebuild the trajectory themselves (plane edges other than 28 / 32, four channels); ckpt may
+ * that rebuild the trajectory themselves (plane edges other than 28 / 32, four or more channels); ckpt may
  * then be NULL.  pde_adi_backward (no ckpt) stays valid for every configuration: it makes the
  * checkpoints itself inside its (then batch-sized) workspace.  pde_adi_backward_saved needs
  * pde_adi_backward_saved_workspace_bytes(d) bytes of workspace when ckpt != NULL and
