@@ -17,7 +17,7 @@ ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 INCLUDE = os.path.join(ROOT, "include")
 LIB = os.path.join(HERE, "libpde_b200.so")
-SOURCES = ["cabi.cu", "adi.cu", "adi_split.cu", "adi_generic.cu", "adi_wide.cu", "explicit.cu", "tiny_split.cu"]
+SOURCES = ["cabi.cu", "adi.cu", "adi_split.cu", "adi_generic.cu", "adi_wide.cu", "explicit.cu", "tiny_split.cu", "tiny_tiled.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-lineinfo", "-std=c++17",

@@ -19,6 +19,8 @@
 #include <cuda_bf16.h>
 
 #include "common.cuh"
+#include "tiny_step.cuh"
+#include "tiny_tiled.cuh"
 
 namespace pde {
 namespace expl {
@@ -65,11 +67,6 @@ __device__ __forceinline__ float widen1(const __nv_bfloat16 *p) {
     return __uint_as_float((unsigned)(*reinterpret_cast<const unsigned short *>(p)) << 16);
 }
 
-__device__ __forceinline__ float clamp_alpha(const pde_tiny_desc &d, float raw, bool *inside) {
-    *inside = raw >= d.cmin && raw <= d.cmax;
-    return raw < d.cmin ? d.cmin : (raw > d.cmax ? d.cmax : raw);
-}
-
 struct Strip {
     float4 c, up, dn;
     float lf, rt;
@@ -112,12 +109,6 @@ __device__ __forceinline__ float4 lap0_scaled(const Strip &s, float k) {
     r.z = (((s.up.z * k + c1) + (-4.0f * c2)) + c3) + s.dn.z * k;
     r.w = (((s.up.w * k + c2) + (-4.0f * c3)) + rt) + s.dn.w * k;
     return r;
-}
-
-__device__ __forceinline__ float blend1(float u, float sc, float adt, float lap, float bl) {
-    const float v = u * sc;
-    const float w = fmaf(adt, lap, v);
-    return fmaf(bl, w - u, u);
 }
 
 // one explicit step of a whole plane: src in shared memory, dst in shared or global memory
@@ -374,6 +365,30 @@ static int tiny_grid(const pde_tiny_desc *d, const DeviceProps &props, size_t sm
         if (grid < d->C) grid = d->C;
     }
     return (int)(grid < 1 ? 1 : grid);
+}
+
+// Which kernels serve one pass of a tiny configuration with B > 0: the whole-plane ring kernels keep every
+// configuration they serve (tiny_validate and tiny_plan both pass), the tiled kernels (tiny_tiled.cu) take the
+// rest of their domain, anything else is PDE_ERR_UNSUPPORTED.  The launches and the workspace query all ask here.
+static int tiny_route(const pde_tiny_desc *d, bool bwd, int io_bytes, int max_smem, bool *tiled, int *stages,
+                      size_t *smem) {
+    const int rc = tiny_validate(d, io_bytes);
+    if (rc == PDE_ERR_INVALID) return rc;
+    *tiled = rc != PDE_OK || tiny_plan(d, bwd, max_smem, stages, smem, io_bytes) != PDE_OK;
+    return *tiled && !tiled::tiny_tiled_domain(d) ? PDE_ERR_UNSUPPORTED : PDE_OK;
+}
+
+// the checks that come before the batch is looked at: B = 0 is a no-op wherever some kernel could serve B > 0
+static int tiny_precheck(const pde_tiny_desc *d, int io_bytes) {
+    const int rc = tiny_validate(d, io_bytes);
+    if (rc == PDE_ERR_UNSUPPORTED && tiled::tiny_tiled_domain(d)) return PDE_OK;
+    return rc;
+}
+
+// pointers a kernel may be handed: 16-byte aligned for the ring kernels' vector loads and bulk copies, element
+// aligned for the tiled kernels
+static bool tiny_aligned(const void *p, bool tiled, int io_bytes) {
+    return tiled ? (reinterpret_cast<uintptr_t>(p) % (uintptr_t)io_bytes) == 0 : aligned16(p);
 }
 
 // ==========================================================================================
@@ -659,30 +674,42 @@ using namespace pde::expl;
 
 // ------------------------------------------------------------------------------------------ tiny
 extern "C" size_t pde_tiny_backward_workspace_bytes(const pde_tiny_desc *d) {
-    if (tiny_validate(d) != PDE_OK) return 0;
-    // one (alpha, scaling) partial pair per block; blocks <= 8 per SM
+    if (tiny_precheck(d, 4) != PDE_OK) return 0;
     DeviceProps props;
     if (query_props(&props) != PDE_OK) return 0;
+    // one query serves both I/O types: the tiled kernels' need wherever either backward pass goes there
+    bool tiled32 = false, tiled16 = false;
+    int stages;
+    size_t smem;
+    const bool ok32 = tiny_route(d, true, 4, props.max_smem_optin, &tiled32, &stages, &smem) == PDE_OK;
+    const bool ok16 = tiny_route(d, true, 2, props.max_smem_optin, &tiled16, &stages, &smem) == PDE_OK;
+    if ((ok32 && tiled32) || (ok16 && tiled16)) return tiled::tiny_tiled_workspace_bytes(d, props.sm_count);
+    if (!ok32 && !ok16) return 0;
+    // one (alpha, scaling) partial pair per block; blocks <= 8 per SM
     return ((size_t)props.sm_count * 8 + (size_t)d->C) * 2 * sizeof(float) + 256;
 }
 
 template <typename T>
 static int tiny_forward_impl(const pde_tiny_desc *d, const void *u, const float *alpha_base, const float *channel_scaling,
                              void *out, void *stream) {
-    int rc = tiny_validate(d, (int)sizeof(T));
+    constexpr int io = (int)sizeof(T);
+    int rc = tiny_precheck(d, io);
     if (rc) return rc;
     if (d->B == 0) return PDE_OK;   // empty batch: a no-op, its tensor pointers may be NULL
     if (!u || !alpha_base || !channel_scaling || !out) return PDE_ERR_INVALID;
-    if (!aligned16(u) || !aligned16(out)) return PDE_ERR_INVALID;
     DeviceProps props;
     rc = query_props(&props);
     if (rc) return rc;
     TinyArgs a{};
+    size_t smem;
+    bool tiled;
+    rc = tiny_route(d, false, io, props.max_smem_optin, &tiled, &a.stages, &smem);
+    if (rc) return rc;
+    if (!tiny_aligned(u, tiled, io) || !tiny_aligned(out, tiled, io)) return PDE_ERR_INVALID;
+    if (tiled)
+        return tiled::tiny_tiled_forward(d, io, u, alpha_base, channel_scaling, out, props, static_cast<cudaStream_t>(stream));
     a.d = *d; a.u = u; a.alpha = alpha_base; a.scal = channel_scaling; a.out = out;
     a.nplanes = d->B * d->C;
-    size_t smem;
-    rc = tiny_plan(d, false, props.max_smem_optin, &a.stages, &smem, (int)sizeof(T));
-    if (rc) return rc;
     const int grid = tiny_grid(d, props, smem, false);
     rc = kernel_info(reinterpret_cast<const void *>(tiny_fwd_kernel<T>), smem, nullptr);
     if (rc) return rc;
@@ -694,7 +721,8 @@ template <typename T>
 static int tiny_backward_impl(const pde_tiny_desc *d, const void *u, const void *gout, const float *alpha_base,
                               const float *channel_scaling, void *gin, float *g_alpha_base, float *g_channel_scaling,
                               void *workspace, size_t workspace_bytes, void *stream) {
-    int rc = tiny_validate(d, (int)sizeof(T));
+    constexpr int io = (int)sizeof(T);
+    int rc = tiny_precheck(d, io);
     if (rc) return rc;
     if (!g_alpha_base || !g_channel_scaling) return PDE_ERR_INVALID;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -704,17 +732,22 @@ static int tiny_backward_impl(const pde_tiny_desc *d, const void *u, const void 
         return PDE_OK;
     }
     if (!u || !gout || !alpha_base || !channel_scaling) return PDE_ERR_INVALID;
-    if (!aligned16(u) || !aligned16(gout) || (gin && !aligned16(gin))) return PDE_ERR_INVALID;
     DeviceProps props;
     rc = query_props(&props);
     if (rc) return rc;
     TinyArgs a{};
+    size_t smem;
+    bool tiled;
+    rc = tiny_route(d, true, io, props.max_smem_optin, &tiled, &a.stages, &smem);
+    if (rc) return rc;
+    if (!tiny_aligned(u, tiled, io) || !tiny_aligned(gout, tiled, io) || (gin && !tiny_aligned(gin, tiled, io)))
+        return PDE_ERR_INVALID;
+    if (tiled)
+        return tiled::tiny_tiled_backward(d, io, u, gout, alpha_base, channel_scaling, gin, g_alpha_base, g_channel_scaling,
+                                          workspace, workspace_bytes, props, st);
     a.d = *d; a.u = u; a.gout = gout; a.alpha = alpha_base; a.scal = channel_scaling; a.gin = gin;
     a.need_gin = gin != nullptr;
     a.nplanes = d->B * d->C;
-    size_t smem;
-    rc = tiny_plan(d, true, props.max_smem_optin, &a.stages, &smem, (int)sizeof(T));
-    if (rc) return rc;
     const int grid = tiny_grid(d, props, smem, true);
     const size_t need = (size_t)grid * 2 * sizeof(float) + 256;
     if (!workspace || workspace_bytes < need) return PDE_ERR_WORKSPACE;

@@ -462,6 +462,8 @@ class _EmotionFunction(torch.autograd.Function):
         if gout.dtype != torch.float32:
             gout = gout.float()
         d, dref, ws_bytes = ctx.plan
+        if ws_bytes == 0:
+            raise _tiny_refused(d)
         with _guard(u0.device):
             ws = _bytes(ws_bytes, u0.device)
             gin = torch.empty_like(u0) if ctx.needs_input_grad[0] else None
@@ -485,10 +487,25 @@ class TinyConfig:
     blend: float = 0.1
 
 
+def _tiny_refused(d) -> "_cabi.PdeB200Error":
+    return _cabi.PdeB200Error(
+        f"unsupported tiny_imagenet diffusion configuration (channels={d.C}, H={d.H}, W={d.W}, steps={d.steps}); "
+        "supported: any H, W 1 ... 4096 with at most 16 steps and channels <= 1024 (smaller planes take more steps "
+        "while a sample's plane and its step states fit a block's shared memory)")
+
+
+def _tiny_check(rc: int, d, what: str):
+    if rc == _cabi.ERR_UNSUPPORTED:
+        raise _tiny_refused(d)
+    _cabi.check(rc, what)
+
+
 @functools.lru_cache(maxsize=256)
 def _tiny_plan(cfg: TinyConfig, shape, device_index: int):
     B, C, H, W = shape
     d = _cabi.TinyDesc(B, C, H, W, cfg.steps, cfg.dt, cfg.cmin, cfg.cmax, cfg.blend)
+    # 0 where no backward pass serves d; the forward may still be served (small planes beyond 16 steps), so only
+    # the backward refuses on it
     return d, byref(d), _cabi.lib().pde_tiny_backward_workspace_bytes(byref(d))
 
 
@@ -513,7 +530,7 @@ class _TinyFunction(torch.autograd.Function):
         fwd = L.pde_tiny_forward_bf16 if ctx.bf16 else L.pde_tiny_forward
         with _guard(u.device):
             out = torch.empty_like(u)
-            _cabi.check(fwd(plan[1], _ptr(u), _ptr(al), _ptr(sc), _ptr(out), _stream(u.device)),
+            _tiny_check(fwd(plan[1], _ptr(u), _ptr(al), _ptr(sc), _ptr(out), _stream(u.device)), plan[0],
                         "pde_tiny_forward")
         ctx.plan = plan
         ctx.save_for_backward(u, al, sc)
@@ -529,14 +546,16 @@ class _TinyFunction(torch.autograd.Function):
             gout = gout.to(u.dtype)
         C = u.shape[1]
         d, dref, ws_bytes = ctx.plan
+        if ws_bytes == 0:
+            raise _tiny_refused(d)
         with _guard(u.device):
             ws = _bytes(ws_bytes, u.device)
             gin = torch.empty_like(u) if ctx.needs_input_grad[0] else None
             ga = torch.empty(C, dtype=torch.float32, device=u.device)
             gs = torch.empty(C, dtype=torch.float32, device=u.device)
             bwd = L.pde_tiny_backward_bf16 if ctx.bf16 else L.pde_tiny_backward
-            _cabi.check(bwd(dref, _ptr(u), _ptr(gout), _ptr(al), _ptr(sc), _ptr(gin), _ptr(ga),
-                                            _ptr(gs), _ptr(ws), ws_bytes, _stream(u.device)), "pde_tiny_backward")
+            _tiny_check(bwd(dref, _ptr(u), _ptr(gout), _ptr(al), _ptr(sc), _ptr(gin), _ptr(ga),
+                            _ptr(gs), _ptr(ws), ws_bytes, _stream(u.device)), d, "pde_tiny_backward")
         return gin, ga, gs, None
 
 

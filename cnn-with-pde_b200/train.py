@@ -15,9 +15,12 @@ optimiser recipe is reproduced (SURVEY.md section 2, row 14):
     svhn       SVHN.py:300-406                   AdamW 1e-2, wd 1e-4               CE                256
     emotion    emotion_recognition.py:265-415    AdamW 1e-3, wd 1e-4               CE                 64
 
-every loop clips the gradient norm at 1.0.  Weak scaling: --batch is the per-GPU batch.
+every loop clips the gradient norm at 1.0.  Weak scaling: --batch is the per-GPU batch.  --image-size N trains
+the tiny_imagenet ResNet on N x N images (it ends in a global average pool, so any size works; 224 is ImageNet's);
+the other models' heads are sized for their images, so they refuse it.
 
     python train.py --model cifar10 --batch 512 --steps 50
+    python train.py --model tiny --image-size 224 --batch 64 --steps 20 --graph
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 \
         --master-port 29511 train.py --model cifar10 --batch 512 --steps 50
 
@@ -135,9 +138,19 @@ def _dist_env():
 
 def run(model_name: str, batch: int, steps: int, warmup: int, graph: bool = False, amp: bool = False,
         seed: int = 1234, pool: int = 4, quiet: bool = False, sync: str = "flat", nccl_in_graph: bool = False,
-        no_dropout: bool = False, keep_model: bool = False):
+        no_dropout: bool = False, keep_model: bool = False, image_size: int | None = None):
     """Train `steps` timed steps (after `warmup`) of `model_name` at per-GPU batch `batch` on the
-    current rank's GPU; returns a dict with whole-job img/s (max-over-ranks device time)."""
+    current rank's GPU; returns a dict with whole-job img/s (max-over-ranks device time).
+    `image_size` (tiny only) trains on image_size x image_size images instead of the recipe's 64 x 64."""
+    r = _recipes()[model_name]
+    shape = r.shape
+    if image_size is not None:
+        if model_name != "tiny":
+            raise ValueError(f"--image-size: only the tiny model takes other image sizes (its ResNet ends in a global "
+                             f"average pool); {model_name}'s classifier head is sized for {r.shape[1]} x {r.shape[2]}")
+        if image_size < 1:
+            raise ValueError(f"--image-size must be positive, got {image_size}")
+        shape = (r.shape[0], image_size, image_size)
     world, rank, local = _dist_env()
     if not torch.cuda.is_available():
         raise RuntimeError("train.py needs a CUDA device: the PDE layers have no CPU fallback")
@@ -147,7 +160,6 @@ def run(model_name: str, batch: int, steps: int, warmup: int, graph: bool = Fals
     if world > 1 and not dist.is_initialized():
         dist.init_process_group("nccl", device_id=dev)
         own_pg = True
-    r = _recipes()[model_name]
     torch.manual_seed(seed)            # identical initial weights on every rank
     model = r.build().to(dev)
     model.train()
@@ -168,7 +180,7 @@ def run(model_name: str, batch: int, steps: int, warmup: int, graph: bool = Fals
     torch.cuda.current_stream().wait_stream(side)
 
     gen = torch.Generator(device=dev).manual_seed(seed + 1 + rank)   # a different shard per rank
-    xs = [torch.randn(batch, *r.shape, device=dev, generator=gen) for _ in range(pool)]
+    xs = [torch.randn(batch, *shape, device=dev, generator=gen) for _ in range(pool)]
     ys = [torch.randint(0, r.classes, (batch,), device=dev, generator=gen) for _ in range(pool)]
     x_in, y_in = xs[0].clone(), ys[0].clone()
     loss_out = torch.zeros((), device=dev)
@@ -263,7 +275,7 @@ def run(model_name: str, batch: int, steps: int, warmup: int, graph: bool = Fals
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     ms = float(ms.item())
     out = {
-        "model": model_name, "n_gpus": world, "batch_per_gpu": batch, "global_batch": batch * world,
+        "model": model_name, "image_shape": list(shape), "n_gpus": world, "batch_per_gpu": batch, "global_batch": batch * world,
         "steps": steps, "warmup": warmup, "ms_per_step": ms / max(steps, 1),
         "img_per_s": batch * world * steps / (ms * 1e-3) if ms > 0 else 0.0,
         "loss": float(loss_out.item()), "cuda_graph": bool(graphs), "autocast": amp, "optimizer_steps": state["done"],
@@ -293,11 +305,12 @@ def main(argv=None):
     ap.add_argument("--sync", choices=("flat", "ddp"), default="flat", help="gradient sync for N > 1")
     ap.add_argument("--nccl-in-graph", action="store_true", help="capture the all-reduce inside the CUDA graph (opt-in)")
     ap.add_argument("--seed", type=int, default=1234)
+    ap.add_argument("--image-size", type=int, default=None, help="tiny only: train on N x N images (e.g. 224)")
     a = ap.parse_args(argv)
     batch = a.batch or _recipes()[a.model].batch
     t0 = time.time()
     out = run(a.model, batch, a.steps, a.warmup, graph=a.graph, amp=a.amp, seed=a.seed, sync=a.sync,
-              nccl_in_graph=a.nccl_in_graph)
+              nccl_in_graph=a.nccl_in_graph, image_size=a.image_size)
     if int(os.environ.get("RANK", "0")) == 0:
         print(f"# {out['img_per_s']:.0f} img/s on {out['n_gpus']} GPU(s), {out['ms_per_step']:.3f} ms/step, "
               f"wall {time.time() - t0:.1f} s", flush=True)

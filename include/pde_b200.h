@@ -201,6 +201,19 @@ int pde_emotion_backward(const pde_emo_desc *d, const float *u0, const float *go
 /* ---------------------------------------------------------------------------------------
  * Explicit family, zero ghosts, per-channel scalars.  Replaces ImprovedDiffusionLayer.forward
  * and simple_diffusion_step, tiny_imagenet.py:34-72.
+ *
+ * Domain: 1 <= H, W <= 4096 (any combination: odd sizes and rectangles), 0 <= steps <= 16,
+ * 1 <= C <= 1024, fp32 and bf16 I/O.  Smaller planes also take more than 16 steps where the
+ * whole-plane kernels hold a plane and its step states in one block's shared memory.  Two kernel
+ * families serve it, chosen per pass: the whole-plane ring kernels wherever they fit (W % 4 == 0,
+ * for bf16 also H * W % 8 == 0, and the plane plus its step states within shared memory), the tiled
+ * kernels everywhere else in the domain.  Anything else is PDE_ERR_UNSUPPORTED; B = 0 is a no-op
+ * wherever the domain or the whole-plane kernels serve the descriptor.
+ * Alignment: where the whole-plane kernels serve a pass, u / out / gout / gin must be 16-byte
+ * aligned; where the tiled kernels do, element alignment is enough (4 bytes fp32, 2 bytes bf16), so a
+ * batch slice such as x[1:] of a plane with W % 4 != 0 can be passed as it is.
+ * pde_tiny_backward_workspace_bytes serves both I/O types: the largest of what the fp32 and bf16
+ * backward passes need, 0 for a descriptor neither serves.
  * ------------------------------------------------------------------------------------- */
 typedef struct pde_tiny_desc {
     int32_t B, C, H, W, steps;
@@ -217,7 +230,7 @@ int pde_tiny_backward(const pde_tiny_desc *d, const float *u, const float *gout,
                       void *workspace, size_t workspace_bytes, void *stream);
 
 /* bf16-I/O variants (SURVEY.md section 8f rank 3): u, out, gout, gin are bfloat16 planes in the same NCHW
- * layout (H * W a multiple of 8); arithmetic, parameters and parameter gradients stay fp32 and the
+ * layout (the whole-plane kernels need H * W a multiple of 8; the tiled ones take any plane); arithmetic, parameters and parameter gradients stay fp32 and the
  * results are rounded to nearest even once, on the way out.  This is the one layer of the reference that
  * is bound by HBM bandwidth, so halving the bytes per cell is what a half-precision pipeline gains from it.
  * Workspace size: pde_tiny_backward_workspace_bytes. */
