@@ -11,8 +11,10 @@
 // walking its own row and a thread walking its own column both hit 32 distinct banks); 64 threads own
 // a plane, thread t solves row t (x sweep) and then column t (y sweep) in registers.  The pivots do not
 // depend on the line, the plane or the sample: one thread per axis factorises once per block.  Both
-// sweeps of the ADI step run on-chip: one HBM read and one HBM write per cell.
+// sweeps of the ADI step run on-chip: one HBM read and one HBM write per cell.  Larger planes, up to 4096 x 4096,
+// go to the line-streaming kernels of tiny_split_tiled.cu (tsplit_on_chip decides).
 #include "common.cuh"
+#include "tiny_split_tiled.cuh"
 
 namespace pde {
 namespace tsplit {
@@ -119,6 +121,9 @@ __global__ void __launch_bounds__(kThreads) tiny_split_kernel(const Args a) {
     }
 }
 
+// the plane fits tiny_split_kernel's tile; every other plane of the domain takes the line-streaming kernels
+inline bool tsplit_on_chip(const pde_tiny_split_desc *d) { return d->H <= kMaxN && d->W <= kMaxN; }
+
 }  // namespace tsplit
 }  // namespace pde
 
@@ -126,12 +131,13 @@ using namespace pde;
 
 extern "C" int pde_tiny_split(const pde_tiny_split_desc *d, const float *u, float *out, void *stream) {
     if (!d || d->B < 0 || d->H < 1 || d->W < 1 || d->mode < 0 || d->mode > 4) return PDE_ERR_INVALID;
-    if (d->H > tsplit::kMaxN || d->W > tsplit::kMaxN) return PDE_ERR_UNSUPPORTED;
+    if (d->H > tsplit_tiled::kMaxEdge || d->W > tsplit_tiled::kMaxEdge) return PDE_ERR_UNSUPPORTED;
     if (d->B == 0) return PDE_OK;
     if (!u || !out) return PDE_ERR_INVALID;
     DeviceProps props;
     int rc = query_props(&props);
     if (rc) return rc;
+    if (!tsplit::tsplit_on_chip(d)) return tsplit_tiled::tiny_split_tiled(d, u, out, props, static_cast<cudaStream_t>(stream));
     int per_sm = 1;
     rc = cached_occupancy(reinterpret_cast<const void *>(tsplit::tiny_split_kernel), tsplit::kThreads, 0, &per_sm);
     if (rc) return rc;

@@ -624,8 +624,8 @@ def tiny_split(method: str, u, coeff_x: float = 0.0, coeff_y: float = 0.0, dt: f
     if u.dim() != 3:
         raise ValueError(f"{method}: expected (B, H, W) planes, got shape {tuple(u.shape)}")
     B, H, W = u.shape
-    if H > 64 or W > 64:
-        raise _cabi.PdeB200Error(f"{method}: planes up to 64 x 64 are built, got {H} x {W}")
+    if H > 4096 or W > 4096:
+        raise _cabi.PdeB200Error(f"{method}: planes up to 4096 x 4096 are built, got {H} x {W}")
     u = _autocast_to_fp32(u)
     d = _tiny_split_desc(TINY_SPLIT_MODES[method], B, H, W, float(coeff_x), float(coeff_y), float(dt), float(eps))
     return _TinySplitFunction.apply(u, d)

@@ -246,8 +246,15 @@ int pde_tiny_backward_bf16(const pde_tiny_desc *d, const void *u, const void *go
  * implicit_diffusion_step (:88-102), solve_implicit_x / _y (:104-157, with the clamp(denom) Thomas
  * variant of :159-190) and diffuse_x_explicit / diffuse_y_explicit (:199-233).  The reference stores
  * `use_implicit` (:21) and never reads it, so no forward reaches them; these entry points serve a
- * caller that does.  u, out: [B][H][W] planes, H, W <= 64.  All five maps are linear in u and
- * self-adjoint: the gradient with respect to u is the same call on the upstream gradient.
+ * caller that does.  All five maps are linear in u and self-adjoint: the gradient with respect to
+ * u is the same call on the upstream gradient.
+ * Domain: u, out: [B][H][W] fp32 planes, 1 <= H, W <= 4096, any B (B = 0 is a no-op); larger
+ * planes are PDE_ERR_UNSUPPORTED.  Planes with H <= 64 and W <= 64 are solved whole in one
+ * block's shared memory (one HBM read and write per cell, u and out may be one buffer); every
+ * other plane goes to line-streaming kernels, one lane per line, that park the forward
+ * elimination in out (modes 0-2 may run in place; in modes 3-4 u and out must not overlap).
+ * Both give the same results bit for bit on a line both can hold.  u and out need only be
+ * 4-byte aligned.  The library allocates nothing.
  * ------------------------------------------------------------------------------------- */
 #define PDE_TINY_SPLIT_ADI 0          /* x solve with cx, then y solve with cy                  */
 #define PDE_TINY_SPLIT_IMPLICIT_X 1
