@@ -19,6 +19,8 @@
 #include <cuda_bf16.h>
 
 #include "common.cuh"
+#include "emo_profile.cuh"
+#include "emotion_halo.cuh"
 #include "tiny_step.cuh"
 #include "tiny_tiled.cuh"
 
@@ -404,22 +406,6 @@ struct EmoArgs {
     int need_gin;
 };
 
-// a_i = 0.5 dt (w1 + w2 sin 2 pi y_i + w3 sin 4 pi y_i) / dx^2     emotion_recognition.py:76-77
-// b_j =     dt (w1 + w2 cos 2 pi x_j + w3 cos 4 pi x_j) / dy^2     emotion_recognition.py:79-80
-// evaluated in the reference's order with correctly rounded fp32 ops (no contraction).
-__device__ __forceinline__ void emo_profile(const pde_emo_desc &d, const float *__restrict__ w6,
-                                            const float *__restrict__ xs, const float *__restrict__ ys, int i,
-                                            float *a, float *b) {
-    const float two_pi = (float)(2.0 * 3.141592653589793), four_pi = (float)(4.0 * 3.141592653589793);
-    const float y = ys[i], x = xs[i];
-    const float s1 = sinf(__fmul_rn(two_pi, y)), s2 = sinf(__fmul_rn(four_pi, y));
-    const float c1 = cosf(__fmul_rn(two_pi, x)), c2 = cosf(__fmul_rn(four_pi, x));
-    const float sa = __fadd_rn(__fadd_rn(w6[0], __fmul_rn(w6[1], s1)), __fmul_rn(w6[2], s2));
-    const float sb = __fadd_rn(__fadd_rn(w6[3], __fmul_rn(w6[4], c1)), __fmul_rn(w6[5], c2));
-    *a = __fdiv_rn(__fmul_rn(d.half_dt, sa), d.dx2);
-    *b = __fdiv_rn(__fmul_rn(d.dt, sb), d.dy2);
-}
-
 // interior of the padded plane <- global plane (coalesced), then the reflected ghost ring
 __device__ __forceinline__ void emo_load_padded(const float *__restrict__ g, float *buf, float *buf2, int N,
                                                 int tid, int nthreads) {
@@ -637,6 +623,16 @@ static int emo_validate(const pde_emo_desc *d) {
     return PDE_OK;
 }
 
+// Which kernels serve an emotion descriptor: every plane edge up to kEmoMaxN keeps the whole-plane kernels below
+// (and their answers), larger planes within halo::emo_halo_domain go to emotion_halo.cu, anything else is
+// PDE_ERR_UNSUPPORTED.  Both launches and the workspace query ask here.
+static int emo_route(const pde_emo_desc *d, bool *halo) {
+    const int rc = emo_validate(d);
+    *halo = rc == PDE_ERR_UNSUPPORTED;
+    if (rc == PDE_ERR_INVALID) return rc;
+    return *halo && !halo::emo_halo_domain(d) ? PDE_ERR_UNSUPPORTED : PDE_OK;
+}
+
 static int emo_threads(int N) {
     const int rb = (N + kEmoRows - 1) / kEmoRows;
     return ((N * rb + 31) / 32) * 32;
@@ -788,7 +784,9 @@ extern "C" int pde_tiny_backward_bf16(const pde_tiny_desc *d, const void *u, con
 
 // --------------------------------------------------------------------------------------- emotion
 extern "C" size_t pde_emotion_backward_workspace_bytes(const pde_emo_desc *d) {
-    if (emo_validate(d) != PDE_OK) return 0;
+    bool halo;
+    if (emo_route(d, &halo) != PDE_OK) return 0;
+    if (halo) return halo::emo_halo_workspace_bytes(d);
     DeviceProps props;
     if (query_props(&props) != PDE_OK) return 0;
     const size_t generic = (size_t)props.sm_count * 4 * 2 * kEmoMaxN * sizeof(float) + 256;
@@ -801,13 +799,15 @@ extern "C" size_t pde_emotion_backward_workspace_bytes(const pde_emo_desc *d) {
 
 extern "C" int pde_emotion_forward(const pde_emo_desc *d, const float *u0, const float *w6, const float *xs,
                                    const float *ys, float *out, void *stream) {
-    int rc = emo_validate(d);
+    bool halo;
+    int rc = emo_route(d, &halo);
     if (rc) return rc;
     if (d->B == 0) return PDE_OK;   // empty batch: a no-op, its tensor pointers may be NULL
     if (!u0 || !w6 || !xs || !ys || !out) return PDE_ERR_INVALID;
     DeviceProps props;
     rc = query_props(&props);
     if (rc) return rc;
+    if (halo) return halo::emo_halo_forward(d, u0, w6, xs, ys, out, props, static_cast<cudaStream_t>(stream));
     EmoArgs a{};
     a.d = *d; a.u0 = u0; a.w6 = w6; a.xs = xs; a.ys = ys; a.out = out;
     if (emo_use_tiled(d))
@@ -825,7 +825,8 @@ extern "C" int pde_emotion_forward(const pde_emo_desc *d, const float *u0, const
 extern "C" int pde_emotion_backward(const pde_emo_desc *d, const float *u0, const float *gout, const float *w6,
                                     const float *xs, const float *ys, float *gin, float *g_w6, void *workspace,
                                     size_t workspace_bytes, void *stream) {
-    int rc = emo_validate(d);
+    bool halo;
+    int rc = emo_route(d, &halo);
     if (rc) return rc;
     if (!g_w6) return PDE_ERR_INVALID;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -837,6 +838,8 @@ extern "C" int pde_emotion_backward(const pde_emo_desc *d, const float *u0, cons
     DeviceProps props;
     rc = query_props(&props);
     if (rc) return rc;
+    if (halo)
+        return halo::emo_halo_backward(d, u0, gout, w6, xs, ys, gin, g_w6, workspace, workspace_bytes, props, st);
     if (emo_use_tiled(d)) {
         if (!workspace || workspace_bytes < emo_tiled_workspace_bytes(d, props.sm_count)) return PDE_ERR_WORKSPACE;
         EmoArgs t{};

@@ -426,6 +426,14 @@ class EmoConfig:
         return _cabi.EmoDesc(B, self.N, self.Nt, f(0.5 * self.dt), f(self.dt), f(self.dx ** 2), f(self.dy ** 2), 0)
 
 
+def _emo_check(rc: int, d, what: str):
+    if rc == _cabi.ERR_UNSUPPORTED:
+        raise _cabi.PdeB200Error(
+            f"unsupported emotion PDELayer configuration (N={d.N}, Nt={d.Nt}); supported: N <= 64 with any Nt (the "
+            "backward pass while a sample's step states fit a block's shared memory); 65 ... 4096 with Nt <= 16")
+    _cabi.check(rc, what)
+
+
 @functools.lru_cache(maxsize=256)
 def _emo_plan(cfg: EmoConfig, B: int, generic: bool, device_index: int):
     """(descriptor, its byref, backward workspace bytes) of a call: depends on nothing else."""
@@ -447,8 +455,8 @@ class _EmotionFunction(torch.autograd.Function):
         d = plan[0]
         with _guard(u0.device):
             out = torch.empty_like(u0)
-            _cabi.check(L.pde_emotion_forward(plan[1], _ptr(u0), _ptr(w6c), _ptr(xs), _ptr(ys), _ptr(out), _stream(u0.device)),
-                        "pde_emotion_forward")
+            _emo_check(L.pde_emotion_forward(plan[1], _ptr(u0), _ptr(w6c), _ptr(xs), _ptr(ys), _ptr(out), _stream(u0.device)),
+                       d, "pde_emotion_forward")
         ctx.plan = plan   # the backward pass uses the same descriptor (tuning included)
         ctx.save_for_backward(u0, w6c, xs, ys)
         return out
@@ -468,8 +476,8 @@ class _EmotionFunction(torch.autograd.Function):
             ws = _bytes(ws_bytes, u0.device)
             gin = torch.empty_like(u0) if ctx.needs_input_grad[0] else None
             gw = torch.empty(6, dtype=torch.float32, device=u0.device)
-            _cabi.check(L.pde_emotion_backward(dref, _ptr(u0), _ptr(gout), _ptr(w6), _ptr(xs), _ptr(ys), _ptr(gin),
-                                               _ptr(gw), _ptr(ws), ws_bytes, _stream(u0.device)), "pde_emotion_backward")
+            _emo_check(L.pde_emotion_backward(dref, _ptr(u0), _ptr(gout), _ptr(w6), _ptr(xs), _ptr(ys), _ptr(gin),
+                                              _ptr(gw), _ptr(ws), ws_bytes, _stream(u0.device)), d, "pde_emotion_backward")
         return gin, gw, None, None, None
 
 

@@ -180,7 +180,7 @@ int pde_adi_multi_backward_saved(int n, const pde_adi_desc *d, const void *const
  * emotion_recognition.py:76-97.
  * ------------------------------------------------------------------------------------- */
 typedef struct pde_emo_desc {
-    int32_t B, N, Nt;         /* batch, plane edge (Nx == Ny == N <= 64), int(T/dt)           */
+    int32_t B, N, Nt;         /* batch, plane edge (Nx == Ny == N), int(T/dt); domain below      */
     float half_dt;            /* fp32(0.5*dt)      (scalar in alpha())                       */
     float dt;                 /* fp32(dt)          (scalar in beta())                        */
     float dx2, dy2;           /* fp32(dx**2), fp32(dy**2)                                    */
@@ -188,6 +188,12 @@ typedef struct pde_emo_desc {
                                  kernels where the register-tiled ones would serve            */
 } pde_emo_desc;
 #define PDE_EMO_TUNE_GENERIC 1
+/* Domain: N <= 64 with any Nt on the whole-plane kernels (the backward pass while a sample's step
+ * states fit a block's shared memory, else PDE_ERR_UNSUPPORTED); 65 <= N <= 4096 with Nt <= 16 on
+ * halo-tiled kernels.  Anything else is PDE_ERR_UNSUPPORTED, B = 0 included; B = 0 is a no-op
+ * inside the domain.  Elements need 4-byte alignment only.  The backward workspace is what
+ * pde_emotion_backward_workspace_bytes answers; above N = 64 it is about min(B, chunk) * Nt * N * N
+ * * 4 bytes (no state planes for Nt <= 1), samples running in chunks of at most 512 that fit 1 GiB. */
 
 size_t pde_emotion_backward_workspace_bytes(const pde_emo_desc *d);
 /* w6 = {alpha_w1, alpha_w2, alpha_w3, beta_w1, beta_w2, beta_w3}; xs, ys: the registered
