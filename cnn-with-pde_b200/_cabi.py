@@ -36,6 +36,8 @@ EXPORTS = (
     "pde_adi_checkpoint_bytes", "pde_adi_backward_saved_workspace_bytes", "pde_adi_forward_train",
     "pde_adi_backward_saved",
     "pde_adi_multi_prepare", "pde_adi_multi_forward_train", "pde_adi_multi_backward_saved",
+    "pde_adi_stream_forward_workspace_bytes", "pde_adi_stream_backward_workspace_bytes", "pde_adi_stream_forward",
+    "pde_adi_stream_backward",
     "pde_emotion_backward_workspace_bytes", "pde_emotion_forward", "pde_emotion_backward",
     "pde_tiny_backward_workspace_bytes", "pde_tiny_forward", "pde_tiny_backward",
     "pde_tiny_split", "pde_tiny_forward_bf16", "pde_tiny_backward_bf16",
@@ -114,6 +116,16 @@ def lib():
     L.pde_adi_multi_forward_train.argtypes = [c_int, pp, pp, fp, pp, pp, pp, pp, vp]
     L.pde_adi_multi_backward_saved.restype = c_int
     L.pde_adi_multi_backward_saved.argtypes = [c_int, pp, pp, fp, pp, pp, pp, pp, pp, pp, pp, pp, pp, pp, pp, pp, pp, vp]
+    L.pde_adi_stream_forward_workspace_bytes.restype = c_size_t
+    L.pde_adi_stream_forward_workspace_bytes.argtypes = [POINTER(AdiDesc)]
+    L.pde_adi_stream_backward_workspace_bytes.restype = c_size_t
+    L.pde_adi_stream_backward_workspace_bytes.argtypes = [POINTER(AdiDesc)]
+    L.pde_adi_stream_forward.restype = c_int
+    L.pde_adi_stream_forward.argtypes = [POINTER(AdiDesc), POINTER(AdiSchedule), fp, fp, fp, fp, fp, fp, fp, fp, vp, c_size_t,
+                                         vp]
+    L.pde_adi_stream_backward.restype = c_int
+    L.pde_adi_stream_backward.argtypes = [POINTER(AdiDesc), POINTER(AdiSchedule), fp, fp, fp, fp, fp, fp, fp, fp, fp, fp, fp,
+                                          fp, fp, fp, fp, vp, c_size_t, vp]
     L.pde_emotion_backward_workspace_bytes.restype = c_size_t
     L.pde_emotion_backward_workspace_bytes.argtypes = [POINTER(EmoDesc)]
     L.pde_emotion_forward.restype = c_int

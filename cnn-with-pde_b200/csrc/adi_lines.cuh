@@ -38,6 +38,46 @@ __device__ __forceinline__ void planes_to_tile(const float *__restrict__ g, floa
     }
 }
 
+// One line of one sweep's factor tables: coefficient maps -> clamp -> replicate smoothing -> r -> Thomas pivots,
+// one float4 (r, 1 / pivot, r / pivot, clamp mask) per cell at tq[i * N].  Reference arithmetic, without
+// contraction: get_alpha_beta_at_time mnist_test.py:33-42 / cifar10.py:53-63, smooth_coefficients
+// mnist_test.py:135-149, rows mnist_test.py:83-93, pivots mnist_test.py:169,177-181.  axis 0 reads the alpha maps
+// along row l, axis 1 the beta maps along column l.  This is gprepare_kernel's body (adi_generic.cu) op for op, used
+// by adi_stream.cu; gprepare_kernel keeps its inline copy because calling this routine changes its machine code
+// (register allocation), and the existing kernels' code is kept as it was.
+__device__ __forceinline__ void prepare_line(const pde_adi_desc &d, int axis, int c, int l, float tt, float dts, float h2,
+                                             const float *__restrict__ ab, const float *__restrict__ bb,
+                                             const float *__restrict__ atc, const float *__restrict__ btc, float4 *tq) {
+    const int N = d.N;
+    const float *base = axis ? bb : ab, *tc = axis ? btc : atc;
+    const float third = __fdiv_rn(1.0f, 3.0f);
+    auto coef = [&](int i, bool *inside) {
+        const size_t q = axis == 0 ? ((size_t)c * N + l) * N + i : ((size_t)c * N + i) * N + l;
+        const float raw = __fadd_rn(__ldg(base + q), __fmul_rn(__ldg(tc + q), tt));
+        bool m = raw >= d.cmin;
+        float k = raw < d.cmin ? d.cmin : raw;
+        if (d.has_max) {
+            m = m && raw <= d.cmax;
+            k = k > d.cmax ? d.cmax : k;
+        }
+        *inside = m;
+        return k;
+    };
+    bool m_cur, m_next = false;
+    float k_cur = coef(0, &m_cur), k_prev = k_cur, cst = 0.0f;
+    for (int i = 0; i < N; ++i) {
+        const float k_next = i + 1 < N ? coef(i + 1, &m_next) : k_cur;   // replicate padding at both ends
+        float ks = k_cur;
+        if (d.smooth) ks = __fadd_rn(__fadd_rn(__fmul_rn(k_prev, third), __fmul_rn(k_cur, third)), __fmul_rn(k_next, third));
+        const float r = __fdiv_rn(__fmul_rn(ks, dts), h2);
+        const float diag = (i == 0 || i == N - 1) ? __fadd_rn(1.0f, r) : __fadd_rn(1.0f, __fmul_rn(2.0f, r));
+        const float dn = i == 0 ? __fadd_rn(diag, d.eps) : __fadd_rn(__fsub_rn(diag, __fmul_rn(-r, cst)), d.eps);
+        cst = __fdiv_rn(-r, dn);
+        tq[i * N] = make_float4(r, __fdiv_rn(1.0f, dn), __fdiv_rn(r, dn), m_cur ? 1.0f : 0.0f);
+        k_prev = k_cur; k_cur = k_next; m_cur = m_next;
+    }
+}
+
 constexpr int kChunk = 4;   // cells whose loads are issued together, ahead of the dependent recurrence
 
 // L2 prefetch of a contiguous region by one thread (TMA bulk prefetch: no registers, no shared memory).  The

@@ -271,8 +271,105 @@ class _AdiFunction(torch.autograd.Function):
         return (gin, gmaps[0], gmaps[1], gmaps[2], gmaps[3], gchan, gskip, None, None)
 
 
+# ------------------------------- implicit ADI beyond one block's shared memory (pde_adi_stream_*)
+@functools.lru_cache(maxsize=256)
+def adi_route(cfg: AdiConfig) -> str:
+    """Which kernel family serves `cfg`: "tables" where the shared-memory kernels do (pde_adi_tables_bytes > 0: their
+    plans, table cache and checkpoints), "stream" where only the streaming kernels do (planes beyond one block's
+    shared memory).  Raises PdeB200Error outside both domains."""
+    L = _cabi.lib()
+    d = cfg.desc(1)
+    if L.pde_adi_tables_bytes(byref(d)):
+        return "tables"
+    if L.pde_adi_stream_forward_workspace_bytes(byref(d)):
+        return "stream"
+    raise _cabi.PdeB200Error(
+        f"unsupported implicit-layer configuration (size={cfg.N}, channels={cfg.C}, steps={cfg.steps}); supported: "
+        f"size 2 ... 4096, channels <= {_cabi.ADI_MAX_CHANNELS}, at most 64 Strang / 96 Lie steps")
+
+
+class _AdiStreamPlan:
+    """Descriptor, schedule and workspace sizes of a stream-routed call: (configuration, batch, device)."""
+    __slots__ = ("cfg", "desc", "dref", "sched", "sref", "fwd_bytes", "bwd_bytes")
+
+    def __init__(self, cfg: AdiConfig, B: int):
+        L = _cabi.lib()
+        self.cfg = cfg
+        self.desc = cfg.desc(B, 0)
+        self.dref = byref(self.desc)
+        self.sched = adi_schedule(cfg.steps, cfg.dt, cfg.hx, cfg.hy, cfg.lie)
+        self.sref = byref(self.sched)
+        self.fwd_bytes = L.pde_adi_stream_forward_workspace_bytes(self.dref)
+        self.bwd_bytes = L.pde_adi_stream_backward_workspace_bytes(self.dref)
+
+
+@functools.lru_cache(maxsize=256)
+def _adi_stream_plan(cfg: AdiConfig, B: int, device_index: int) -> _AdiStreamPlan:
+    return _AdiStreamPlan(cfg, B)
+
+
+class _AdiStreamFunction(torch.autograd.Function):
+    """The implicit layer on the streaming kernels: the factor tables are built inside each call, and the backward
+    pass replays the trajectory itself, so only the input and the parameters are kept between the passes."""
+
+    @staticmethod
+    def forward(ctx, u, alpha_base, beta_base, alpha_tc, beta_tc, chan, skipw, cfg: AdiConfig):
+        _require_cuda(u, "PDE layer input")
+        L = _cabi.lib()
+        u = _contig(u)
+        maps = [_contig(p.detach()) for p in (alpha_base, beta_base, alpha_tc, beta_tc)]
+        for p in maps:
+            _require_cuda(p, "PDE layer parameter")
+        chan_c = None if chan is None else _contig(chan.detach())
+        skip_c = None if skipw is None else _contig(skipw.detach())
+        dev = u.device
+        with _guard(dev):
+            plan = _adi_stream_plan(cfg, u.shape[0], dev.index if dev.index is not None else torch.cuda.current_device())
+            ws = _bytes(plan.fwd_bytes, dev)
+            out = torch.empty_like(u)
+            _cabi.check(L.pde_adi_stream_forward(plan.dref, plan.sref, *[p.data_ptr() for p in maps], _ptr(u), _ptr(chan_c),
+                                                 _ptr(skip_c), _ptr(out), ws.data_ptr(), plan.fwd_bytes, _stream(dev)),
+                        "pde_adi_stream_forward")
+        ctx.plan = plan
+        ctx.has_chan = chan is not None
+        ctx.has_skip = skipw is not None
+        ctx.save_for_backward(u, *maps, *(t for t in (chan_c, skip_c) if t is not None))
+        ctx.param_shapes = [p.shape for p in (alpha_base, beta_base, alpha_tc, beta_tc)]
+        return out
+
+    @staticmethod
+    def backward(ctx, gout):
+        _no_double_backward("PDE layer")
+        L = _cabi.lib()
+        plan = ctx.plan
+        saved = list(ctx.saved_tensors)
+        u, maps, rest = saved[0], saved[1:5], saved[5:]
+        chan = rest.pop(0) if ctx.has_chan else None
+        skipw = rest.pop(0) if ctx.has_skip else None
+        gout = _contig(gout)
+        if gout.dtype != torch.float32:
+            gout = gout.float()
+        dev = u.device
+        with _guard(dev):
+            ws = _bytes(plan.bwd_bytes, dev)
+            gin = torch.empty_like(u) if ctx.needs_input_grad[0] else None
+            C, N = plan.cfg.C, plan.cfg.N
+            gm = torch.empty((4,) + tuple(ctx.param_shapes[0]), dtype=torch.float32, device=dev)
+            base, plane = gm.data_ptr(), 4 * C * N * N
+            gchan = torch.empty((C, C), dtype=torch.float32, device=dev) if chan is not None else None
+            gskip = torch.empty((), dtype=torch.float32, device=dev) if skipw is not None else None
+            _cabi.check(L.pde_adi_stream_backward(plan.dref, plan.sref, *[m.data_ptr() for m in maps], _ptr(u), _ptr(gout),
+                                                  _ptr(chan), _ptr(skipw), _ptr(gin), base, base + plane, base + 2 * plane,
+                                                  base + 3 * plane, _ptr(gchan), _ptr(gskip), ws.data_ptr(), plan.bwd_bytes,
+                                                  _stream(dev)), "pde_adi_stream_backward")
+        gmaps = gm.unbind(0)
+        return (gin, gmaps[0], gmaps[1], gmaps[2], gmaps[3], gchan, gskip, None)
+
+
 def adi_layer(u, alpha_base, beta_base, alpha_tc, beta_tc, chan, skipw, cfg: AdiConfig):
     u = _autocast_to_fp32(u)
+    if isinstance(u, torch.Tensor) and u.is_cuda and adi_route(cfg) == "stream":
+        return _AdiStreamFunction.apply(u, alpha_base, beta_base, alpha_tc, beta_tc, chan, skipw, cfg)
     return _AdiFunction.apply(u, alpha_base, beta_base, alpha_tc, beta_tc, chan, skipw, cfg, torch.is_grad_enabled())
 
 
@@ -396,10 +493,12 @@ def adi_multi_layer(u, branches):
     """Apply n implicit layers to the same input.  branches: sequence of (alpha_base, beta_base,
     alpha_time_coeff, beta_time_coeff, chan, skip_weight, cfg).  Returns the n outputs.  Falls back to n
     single-layer calls when the layers cannot share a launch (different shapes / channel ops, plane sizes the
-    half-line kernels do not serve, inference)."""
+    half-line kernels do not serve, planes on the streaming kernels, inference)."""
     u = _autocast_to_fp32(u)
     cfgs = tuple(b[6] for b in branches)
     fused = u.is_cuda and torch.is_grad_enabled() and any(t is not None and t.requires_grad for b in branches for t in b[:6])
+    # the multi-branch launches are built on the shared-memory kernels: a stream-routed branch means one call per layer
+    fused = fused and all(adi_route(c) == "tables" for c in cfgs)
     if fused:
         dev = u.device
         with _guard(dev):

@@ -65,7 +65,8 @@ typedef struct pde_adi_desc {
                                  PDE_MAX_CHANNELS < C <= PDE_ADI_MAX_CHANNELS: any N in 2 ... 128
                                  while C * N * (N | 1) * 4 bytes <= 200 KB (e.g. C <= 48 at 32 x 32,
                                  12 at 64 x 64); no checkpoints (the backward pass replays), no
-                                 pde_adi_multi_* (PDE_ERR_UNSUPPORTED)                          */
+                                 pde_adi_multi_* (PDE_ERR_UNSUPPORTED).
+                                 Every other C <= 64, N <= 4096: pde_adi_stream_* below          */
     int32_t steps;            /* num_steps                                                   */
     int32_t lie;              /* 0 Strang x(dt/2) y(dt) x(dt/2); 1 Lie x(dt/2) y(dt/2)        */
     int32_t smooth;           /* 3-tap replicate smoothing of the clamped map along the sweep */
@@ -174,6 +175,44 @@ int pde_adi_multi_backward_saved(int n, const pde_adi_desc *d, const void *const
                                  float *const *g_alpha_time_coeff, float *const *g_beta_time_coeff,
                                  float *const *g_chan, float *const *g_skip_weight,
                                  void *const *workspace, const size_t *workspace_bytes, void *stream);
+
+/* ---------------------------------------------------------------------------------------
+ * Implicit ADI family, streaming kernels: the layers of the group above on planes beyond one block's
+ * shared memory.  Same descriptor, schedule and arguments; the factor tables are built inside the
+ * call (one sweep at a time, in the workspace), so there is no prepare step and no checkpoint buffer.
+ * Domain: every descriptor with 1 <= C <= PDE_ADI_MAX_CHANNELS, 2 <= N <= 4096 and at most
+ * PDE_MAX_SWEEPS sweeps, any B >= 0 -- including the configurations pde_adi_tables_bytes serves
+ * (callers use the group above there; outputs are equal bit for bit, gradients up to the fp32
+ * summation order).  N = 1, N > 4096, C > 64 or more sweeps: PDE_ERR_UNSUPPORTED, and both queries
+ * answer 0.  B = 0 is a no-op; the backward pass then zeroes the gradients.  u, out, gout, gin need
+ * 4-byte alignment only; the workspace must be 256-byte aligned and at least the queried size
+ * (PDE_ERR_WORKSPACE otherwise).  Workspace sizes, with S = steps * (lie ? 2 : 3) sweeps,
+ * P = (lie ? 2 : 3) sweeps a step and CNN = C * N * N:
+ *   forward:  16 * CNN                                       (one sweep's factor tables)
+ *   backward: 512 * C * C * (chan_op != 0) + 2048 * skip      (double partials of g_chan, g_skip)
+ *             + 16 * CNN                                      (one sweep's factor tables)
+ *             + K * (steps + P + 1) * CNN * 4                 (per sample in flight: the state at the end of
+ *                                                              every step, the replayed step's sweep outputs,
+ *                                                              the adjoint)
+ *   with K = min(max(B, 1), max(1, floor(2^30 / ((steps + P + 1) * CNN * 4)))) samples in flight.
+ * The backward pass replays the forward trajectory itself and overwrites the gradient outputs
+ * (gin may be NULL).  Coefficient gradients are bit-reproducible and independent of gin.
+ * ------------------------------------------------------------------------------------- */
+size_t pde_adi_stream_forward_workspace_bytes(const pde_adi_desc *d);
+size_t pde_adi_stream_backward_workspace_bytes(const pde_adi_desc *d);
+int pde_adi_stream_forward(const pde_adi_desc *d, const pde_adi_schedule *sched,
+                           const float *alpha_base, const float *beta_base,
+                           const float *alpha_time_coeff, const float *beta_time_coeff,
+                           const float *u, const float *chan, const float *skip_weight, float *out,
+                           void *workspace, size_t workspace_bytes, void *stream);
+int pde_adi_stream_backward(const pde_adi_desc *d, const pde_adi_schedule *sched,
+                            const float *alpha_base, const float *beta_base,
+                            const float *alpha_time_coeff, const float *beta_time_coeff,
+                            const float *u, const float *gout, const float *chan, const float *skip_weight,
+                            float *gin, float *g_alpha_base, float *g_beta_base,
+                            float *g_alpha_time_coeff, float *g_beta_time_coeff,
+                            float *g_chan, float *g_skip_weight,
+                            void *workspace, size_t workspace_bytes, void *stream);
 
 /* ---------------------------------------------------------------------------------------
  * Explicit family, frozen reflected ghost ring.  Replaces PDELayer.forward / alpha / beta
