@@ -20,8 +20,10 @@
 //     memory by TMA one phase ahead) to its half line of Q groups in turn; it optionally writes the
 //     state at the end of every step as a tile image (the "checkpoints": HBM is idle in these kernels).
 //   * Backward: starts from those checkpoints instead of recomputing the trajectory; checkpoint
-//     tiles arrive by TMA bulk copies one step ahead, the next item's gout planes by LDGSTS, the
+//     tiles arrive by TMA bulk copies one step ahead, the next item's gout planes by bulk copies too, the
 //     coefficients by TMA one sweep ahead; gradient accumulators live in tensor memory.
+//   * Plane I/O (u, out, gout, grad_input) is one TMA bulk copy per plane into / out of a tile slot in
+//     natural layout; the first and last sweeps convert in registers (nat_ld_half / nat_st_half).
 #include "adi_common.cuh"
 
 namespace pde {
@@ -45,6 +47,18 @@ struct SG {
                                                     // reading a column touches rows of both halves
     static constexpr int TILE = N * RS + HPAD;      // floats per tile: P sample pairs of one channel
     static constexpr int QS = N * 2;                // float4 stride between the chunks of a table row
+    // With four pairs, the planes of a group also sit in a tile slot in natural (NCHW) layout, one
+    // plane per sample, as bulk copies bring them in and take them out.  Plane pitch: N * N + 4 floats,
+    // so that the half-row reads of make_lane's lane map (LDS.64) spread over the banks: 2 wavefronts
+    // for 28 x 28 (N * N = 784 = 16 mod 32 puts the four pairs' sample a in one bank: 4 wavefronts);
+    // 32 x 32: 4 instead of 16, as two lines of a half warp then share their banks whatever the pitch.
+    static constexpr int NPITCH = N * N + 4;
+    // tile slot: a tile, or a group's planes if they need more (28 x 28, four pairs: 64 bytes more)
+    static constexpr int SLOT = TILE > 2 * P * NPITCH ? TILE : 2 * P * NPITCH;
+    // x sets keep the checkpoint image size: there the layer input goes unpadded when the pitch
+    // would not fit
+    static constexpr int XPITCH = 2 * P * NPITCH <= TILE ? NPITCH : N * N;
+    static_assert(TILE % 4 == 0 && SLOT % 4 == 0 && NPITCH % 4 == 0, "16-byte aligned tiles and planes");
 };
 
 // float offset of (mirrored) row R of a tile
@@ -116,7 +130,8 @@ __device__ __forceinline__ void st_half(float *tile, const Lane &t, const f2 (&x
     }
 }
 
-// planes of the block's P sample pairs (channel c) <-> tile.  A thread moves two adjacent cells of
+// Two pairs per group (one block per SM, nothing hides the barriers of the bulk-copy path): planes of the
+// block's P sample pairs (channel c) <-> tile by the threads.  A thread moves two adjacent cells of
 // both samples of a pair per step; consecutive lanes take consecutive pairs, then consecutive
 // cells.  All global loads of a thread are issued before the first one is used.
 template <int N, int P>
@@ -237,15 +252,104 @@ struct PlaneIO {
     }
 };
 
+// ------------------------------------------------------------------------------------------
+// Plane I/O with four pairs per group.  The 2P planes of a group travel between global memory and a tile
+// slot by TMA bulk copies, one per plane, in natural layout: sample s of channel c at
+// slot + c * cstride + s * pitch.  Samples beyond the batch are not copied; zero_tail clears them.
+// The sweep that first reads a group takes its half row from the natural layout (nat_ld_half) and,
+// after a barrier, stores it in tile layout; the last sweep does the reverse (nat_st_half).
+// ------------------------------------------------------------------------------------------
 template <int N, int P>
-__device__ __forceinline__ void planes_to_tile(const float *__restrict__ g, float *tile, int item, int c, int C, int B,
-                                               int tid_c, int) {
-    PlaneIO<N, P>::to_tile(g, tile, item, c, C, B, tid_c);
+__device__ __forceinline__ int group_valid(long long grp, int B) {   // samples of group grp inside the batch
+    const long long v = (long long)B - grp * 2 * P;
+    return v <= 0 ? 0 : (v >= 2 * P ? 2 * P : (int)v);
 }
+
+// one thread: bulk loads of the group's valid planes, completing on `bar` (the caller expects the bytes)
 template <int N, int P>
-__device__ __forceinline__ void tile_to_planes(const float *tile, float *__restrict__ g, int item, int c, int C, int B,
-                                               int tid_c, int, const float *__restrict__ w, float sig, float om) {
-    PlaneIO<N, P>::from_tile(tile, g, item, c, C, B, tid_c, w, sig, om);
+__device__ __forceinline__ void planes_load(float *slot, int cstride, int pitch, const float *__restrict__ g, long long grp,
+                                            int C, int B, uint64_t *bar) {
+    const int nv = group_valid<N, P>(grp, B);
+    for (int c = 0; c < C; ++c)
+        for (int s = 0; s < nv; ++s)
+            tma_load_1d(slot + c * cstride + s * pitch, g + ((size_t)(grp * 2 * P + s) * C + c) * (N * N),
+                        (uint32_t)(N * N * sizeof(float)), bar);
+}
+
+// one thread: bulk stores of the group's valid planes, as one bulk group
+template <int N, int P>
+__device__ __forceinline__ void planes_store(float *__restrict__ g, const float *slot, int cstride, int pitch, long long grp,
+                                             int C, int B) {
+    const int nv = group_valid<N, P>(grp, B);
+    for (int c = 0; c < C; ++c)
+        for (int s = 0; s < nv; ++s)
+            tma_store_1d(g + ((size_t)(grp * 2 * P + s) * C + c) * (N * N), slot + c * cstride + s * pitch,
+                         (uint32_t)(N * N * sizeof(float)));
+    bulk_commit();
+}
+
+// every thread of the block: zero planes nv .. 2P-1 of every channel (samples beyond the batch)
+template <int N, int P>
+__device__ __forceinline__ void zero_tail(float *slot, int cstride, int pitch, int C, int nv) {
+    constexpr int F4 = N * N / 4;
+    const int per_c = (2 * P - nv) * F4;
+    for (int i = threadIdx.x; i < C * per_c; i += blockDim.x) {
+        const int c = i / per_c, r = i - c * per_c;
+        *reinterpret_cast<float4 *>(slot + c * cstride + (nv + r / F4) * pitch + 4 * (r % F4)) = make_float4(0.f, 0.f, 0.f, 0.f);
+    }
+}
+
+// The thread's half row (row mirror(R), near or far half, cells from the plane edge) of its sample
+// pair, from / to the natural layout.  Cells 2m, 2m+1 are columns 2m, 2m+1 (near) or N-1-2m, N-2-2m (far).
+template <int N, int P, int PITCH>
+__device__ __forceinline__ void nat_ld_half(const float *slot, const Lane &t, f2 (&x)[N / 2]) {
+    const float *pa = slot + 2 * t.pp * PITCH + mirror(t.R, N) * N, *pb = pa + PITCH;
+#pragma unroll
+    for (int m = 0; m < N / 4; ++m) {
+        const int j = t.h ? N - 2 - 2 * m : 2 * m;
+        const float2 va = *reinterpret_cast<const float2 *>(pa + j), vb = *reinterpret_cast<const float2 *>(pb + j);
+        x[2 * m] = t.h ? f2_make(va.y, vb.y) : f2_make(va.x, vb.x);
+        x[2 * m + 1] = t.h ? f2_make(va.x, vb.x) : f2_make(va.y, vb.y);
+    }
+}
+// plane = x                   (w == nullptr)
+// plane = om * x + sig * w    (skip blend, w the same cells of a global plane set: out w = u, om = 1 - sig;
+//                              grad_input w = gout, om = 1)
+template <int N, int P, int PITCH>
+__device__ __forceinline__ void nat_st_half(float *slot, const Lane &t, const f2 (&x)[N / 2], const float *__restrict__ w,
+                                            long long grp, int c, int C, int B, float sig, float om) {
+    const int i = mirror(t.R, N);
+    float *pa = slot + 2 * t.pp * PITCH + i * N, *pb = pa + PITCH;
+    const long long ba = grp * 2 * P + 2 * t.pp, bb = ba + 1;
+    const float *wa = w + ((size_t)ba * C + c) * (N * N) + i * N, *wb = w + ((size_t)bb * C + c) * (N * N) + i * N;
+    const float2 zero = make_float2(0.f, 0.f);
+#pragma unroll
+    for (int m = 0; m < N / 4; ++m) {
+        const int j = t.h ? N - 2 - 2 * m : 2 * m;
+        const float lo_a = f2_lo(x[2 * m]), lo_b = f2_hi(x[2 * m]), hi_a = f2_lo(x[2 * m + 1]), hi_b = f2_hi(x[2 * m + 1]);
+        float2 a = t.h ? make_float2(hi_a, lo_a) : make_float2(lo_a, hi_a);
+        float2 b = t.h ? make_float2(hi_b, lo_b) : make_float2(lo_b, hi_b);
+        if (w) {
+            const float2 va = ba < B ? __ldg(reinterpret_cast<const float2 *>(wa + j)) : zero;
+            const float2 vb = bb < B ? __ldg(reinterpret_cast<const float2 *>(wb + j)) : zero;
+            a.x = fmaf(om, a.x, sig * va.x);
+            a.y = fmaf(om, a.y, sig * va.y);
+            b.x = fmaf(om, b.x, sig * vb.x);
+            b.y = fmaf(om, b.y, sig * vb.y);
+        }
+        *reinterpret_cast<float2 *>(pa + j) = a;
+        *reinterpret_cast<float2 *>(pb + j) = b;
+    }
+}
+
+// Rows of a tile slot that holds a group's planes -> the same slot in tile layout (the caller has
+// passed a barrier since the planes arrived; a barrier must follow before other threads read)
+template <int N, int P, int PITCH>
+__device__ __forceinline__ void planes_to_rows(float *slot, const Lane &t) {
+    f2 x[N / 2];
+    nat_ld_half<N, P, PITCH>(slot, t, x);
+    __syncthreads();   // every thread has read its rows in natural layout
+    if (t.active) st_half<N, P, 0>(slot, t, x);
 }
 
 // the thread's coefficients of one table for one sweep: HQ float4, the same address for the P
@@ -330,8 +434,8 @@ __device__ __forceinline__ Lane make_lane() {
     t.h = (lane / P) & 1;
     const int line = t.wi * G::LPW + lane / (2 * P);
     t.active = line < N;
-    t.R = t.active ? line : N - 1;
     t.tid_c = threadIdx.x - t.c * G::WPC * 32;
+    t.R = t.active ? line : N - 1;
     t.b0 = half_base_of<N, P, 0>(t.R, t.h, t.pp);
     t.b1 = half_base_of<N, P, 1>(t.R, t.h, t.pp);
     t.tab = (t.c * G::HQ * N + t.R) * 2 + t.h;
@@ -359,47 +463,6 @@ constexpr int max_threads() { return P >= 4 ? SG<N, P>::WPC * 32 : SG<N, P>::WPC
 // The closing half sweep of a Strang step and the opening one of the next run back to back on
 // the registers (same orientation).
 // ------------------------------------------------------------------------------------------
-// planes (u or gout) of group `grp` -> tile, asynchronously (LDGSTS): every 4-byte cell goes straight from
-// global memory to its slot in the interleaved / mirrored tile, no registers, no wait.  Samples
-// beyond the batch are zero-filled.  Completion: cp_async_wait_all() + a barrier.
-__device__ __forceinline__ void cp_async4(float *dst_smem, const float *src, bool valid) {
-    const int n = valid ? 4 : 0;
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 4, %2;" ::"r"(smem_u32(dst_smem)), "l"(src), "r"(n) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_group 0;" ::: "memory"); }
-
-template <int N, int P>
-__device__ __forceinline__ void planes_to_tile_async(const float *__restrict__ g, float *tile, int grp, int c, int C,
-                                                     int B, int tid_c) {
-    using IO = PlaneIO<N, P>;
-    const typename IO::Thread th = IO::thread(tid_c);
-#pragma unroll
-    for (int it = 0; it < IO::IT; ++it) {
-        const typename IO::Slot sl = IO::slot(th, tid_c, it);
-        if (sl.in) {
-            const int f = sl.f;
-            const bool hc = sl.hc;
-            const int ba = (grp * P + sl.pp) * 2, bb = ba + 1;
-            const bool va = ba < B, vb = bb < B;
-            const float *sa = g + ((size_t)(va ? ba : 0) * C + c) * (N * N) + 2 * f;
-            const float *sb = g + ((size_t)(vb ? bb : 0) * C + c) * (N * N) + 2 * f;
-            float *dst = tile + sl.off;
-            // chunk = {cell lo: a, b; cell hi: a, b}; in the far half the two columns swap.  The four
-            // 4-byte copies of a lane start at a component that rotates with the chunk index, so that the
-            // 32 lanes of one instruction hit 32 different banks (chunks are 16 floats apart for P == 4)
-            const int rot = (f >> 1) & 3;
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-                const int comp = (k + rot) & 3;               // 0: a lo-column, 1: b lo-column, 2: a hi, 3: b hi
-                const bool isb = comp & 1;
-                const float *src = (isb ? sb : sa) + (comp >> 1);
-                cp_async4(dst + (hc ? (comp ^ 2) : comp), src, isb ? vb : va);
-            }
-        }
-    }
-}
-
 // One warp folds the per-sweep header entries into the flags the backward kernel reads.  Not inlined:
 // the forward kernels' register allocation has no slack for it (12 - 24 bytes of spills when inlined).
 __device__ __noinline__ void write_ck_flags(const Header *hdr, int steps, int sps, CkFlags *out) {
@@ -416,15 +479,17 @@ __device__ __noinline__ void write_ck_flags(const Header *hdr, int steps, int sp
 template <int N, int P, int Q, bool MIX1>
 __device__ __forceinline__ void sfwd_body(const Args &a, const int bid, const int nblk) {
     using G = SG<N, P>;
-    constexpr int H = G::H, TILE = G::TILE, HQ4 = 4 * G::HQ;
+    constexpr int H = G::H, TILE = G::TILE, SLOT = G::SLOT, NPI = G::NPITCH, HQ4 = 4 * G::HQ;
+    constexpr bool BULK = P >= 4;   // plane I/O by bulk copies (see PlaneIO)
     extern __shared__ __align__(128) float smem[];
     __shared__ __align__(8) uint64_t cbar[2];
+    __shared__ __align__(8) uint64_t ubar;   // the planes of an item's Q groups
     __shared__ short h_slot[PDE_MAX_SWEEPS];
     const pde_adi_desc &d = a.d;
     const Lane t = make_lane<N, P>();
     const int C = d.C, nthr = blockDim.x;
     const bool far = t.h == 1;
-    const int SET = C * Q * TILE;   // floats per tile set: Q groups of every channel
+    const int SET = C * Q * SLOT;   // floats per tile set: Q groups of every channel
     // coefficient stage: 1/pivot and r/pivot of one sweep (all channels), double buffered, filled
     // by TMA one phase ahead
     const int CT = C * G::HQ * N * 2 * 4;
@@ -443,6 +508,7 @@ __device__ __forceinline__ void sfwd_body(const Args &a, const int bid, const in
     if (threadIdx.x == 0) {
         mbar_init(&cbar[0], 1);
         mbar_init(&cbar[1], 1);
+        mbar_init(&ubar, 1);
         mbar_fence_init();
     }
     __syncthreads();
@@ -457,13 +523,33 @@ __device__ __forceinline__ void sfwd_body(const Args &a, const int bid, const in
         }
     };
     const size_t plane = (size_t)N * N;
+    // thread 0: u planes of group q of item `it` -> tile slot q (natural layout); the fill of group 0
+    // expects the bytes of the whole item.  Call after a barrier that ends every use of slot q.
+    auto u_fill = [&](int it, int q) {
+        fence_proxy_async();
+        if (q == 0) {
+            const int nv = group_valid<N, Q * P>(it, d.B);   // samples of the item
+            mbar_expect_tx(&ubar, (uint32_t)(nv * C * plane * sizeof(float)));
+        }
+        planes_load<N, P>(smem + q * SLOT, Q * SLOT, NPI, a.u, (long long)it * Q + q, C, d.B, &ubar);
+    };
+    uint32_t uphase = 0u;
     int cb = 0;
-    if (bid < a.nitems) c_fill(0, 0);
+    if (bid < a.nitems) {
+        c_fill(0, 0);
+        if (BULK && threadIdx.x == 0)
+            for (int q = 0; q < Q; ++q) u_fill(bid, q);
+    }
+    // Four pairs per group serve only layers without channel ops (make_plan): the first sweep, on rows,
+    // reads the planes from the natural layout; a last sweep on rows (Strang) writes the output planes,
+    // the last column sweep of a Lie step leaves that to a pass of its own.
+    const bool nat_first = BULK;
+    const bool nat_last = BULK && sps == 3;
 
     for (int item = bid; item < a.nitems; item += nblk) {
         const int next_item = item + nblk;
         float *set = smem;
-        float *my = set + (size_t)t.c * Q * TILE;   // this channel's Q tiles
+        float *my = set + (size_t)t.c * Q * SLOT;   // this channel's Q tiles
         if (threadIdx.x == 0) {   // the next item's planes start their trip from HBM to L2 now
             const long long nb = (long long)next_item * Q * 2 * P;
             if (nb < d.B) {
@@ -471,18 +557,51 @@ __device__ __forceinline__ void sfwd_body(const Args &a, const int bid, const in
                 prefetch_region_l2(a.u + (size_t)nb * C * plane, (size_t)ns * C * plane * sizeof(float));
             }
         }
-        __syncthreads();   // the previous item's output has left the tiles
+        __syncthreads();   // the previous item's output planes have been read out of the tiles
+        if (!BULK) {
 #pragma unroll 1
-        for (int q = 0; q < Q; ++q) PlaneIO<N, P>::to_tile(a.u, my + q * TILE, item * Q + q, t.c, C, d.B, t.tid_c);
+            for (int q = 0; q < Q; ++q) PlaneIO<N, P>::to_tile(a.u, my + q * SLOT, item * Q + q, t.c, C, d.B, t.tid_c);
+        } else {
+            for (int q = 0; q < Q; ++q) {
+                const int nv = group_valid<N, P>((long long)item * Q + q, d.B);
+                if (nv < 2 * P) zero_tail<N, P>(set + q * SLOT, Q * SLOT, NPI, C, nv);
+            }
+            mbar_wait(&ubar, uphase);
+            uphase ^= 1u;
+        }
+        // tile q -> output planes: the thread's half row x of group q (row orientation) goes to the
+        // natural layout in place, then out by bulk stores; the slot is refilled with the next item's
+        // group as soon as the store has read it (refill of q - 1 behind the store of q)
+        auto emit = [&](int q, const f2 (&x)[H]) {
+            __syncthreads();   // every thread has read tile q
+            if (t.active)
+                nat_st_half<N, P, NPI>(my + q * SLOT, t, x, d.skip ? a.u : nullptr, (long long)item * Q + q, t.c, C, d.B, sig, om);
+            fence_proxy_async();
+            __syncthreads();
+            if (threadIdx.x == 0) {
+                if (a.out) planes_store<N, P>(a.out, set + q * SLOT, Q * SLOT, NPI, (long long)item * Q + q, C, d.B);
+                else bulk_commit();
+                if (next_item < a.nitems) {
+                    if (q > 0) {
+                        bulk_wait_read<1>();
+                        u_fill(next_item, q - 1);
+                    }
+                    if (q == Q - 1) {
+                        bulk_wait_read<0>();
+                        u_fill(next_item, q);
+                    }
+                }
+            }
+        };
         // u <- M u over the channels of every group (rows); leaves the tiles in row orientation
         auto mix_phase = [&]() {
             __syncthreads();
 #pragma unroll 1
             for (int q = 0; q < Q; ++q) {
                 f2 x[H];
-                mix_rows<N, P>(set + q * TILE, Q * TILE, C, a.chan + t.c * C, 1, t, x);
+                mix_rows<N, P>(set + q * SLOT, Q * SLOT, C, a.chan + t.c * C, 1, t, x);
                 __syncthreads();
-                if (t.active) st_half<N, P, 0>(my + q * TILE, t, x);
+                if (t.active) st_half<N, P, 0>(my + q * SLOT, t, x);
             }
         };
         int s = 0;
@@ -519,7 +638,7 @@ __device__ __forceinline__ void sfwd_body(const Args &a, const int bid, const in
             if (MIX1 && mix_first) {
                 f2 xm[Q][H];
 #pragma unroll
-                for (int q = 0; q < Q; ++q) mix_rows<N, P>(set + q * TILE, Q * TILE, C, a.chan + t.c * C, 1, t, xm[q]);
+                for (int q = 0; q < Q; ++q) mix_rows<N, P>(set + q * SLOT, Q * SLOT, C, a.chan + t.c * C, 1, t, xm[q]);
                 __syncthreads();   // every channel has read every tile of the item
 #pragma unroll
                 for (int q = 0; q < Q; ++q) {
@@ -527,16 +646,18 @@ __device__ __forceinline__ void sfwd_body(const Args &a, const int bid, const in
 #pragma unroll
                     for (int kk = 0; kk < H; ++kk) x[0][kk] = xm[q][kk];
                     solve<N, P, 1>(x, iv, e, far);
-                    if (t.active) st_half<N, P, 0>(my + q * TILE, t, x[0]);
+                    if (t.active) st_half<N, P, 0>(my + q * SLOT, t, x[0]);
                 }
                 s = s_next;
                 continue;
             }
+            const bool from_planes = nat_first && s == 0, to_planes = nat_last && s_next >= S;
 #pragma unroll 1
             for (int q = 0; q < Q; ++q) {
-                float *tile = my + q * TILE;
+                float *tile = my + q * SLOT;
                 f2 x[1][H];
-                if (ax == 0) ld_half<N, P, 0>(tile, t, x[0]);
+                if (from_planes) nat_ld_half<N, P, NPI>(tile, t, x[0]);
+                else if (ax == 0) ld_half<N, P, 0>(tile, t, x[0]);
                 else ld_half<N, P, 1>(tile, t, x[0]);
                 solve<N, P, 1>(x, iv, e, far);
                 if (k == sps - 1 && a.ckpt && t.active) {
@@ -558,6 +679,11 @@ __device__ __forceinline__ void sfwd_body(const Args &a, const int bid, const in
                     }
                 }
                 if (fuse) solve<N, P, 1>(x, iv, e, far);
+                if (to_planes) {
+                    emit(q, x[0]);
+                    continue;
+                }
+                if (from_planes) __syncthreads();   // every thread has read the group's planes
                 if (t.active) {
                     if (ax == 0) st_half<N, P, 0>(tile, t, x[0]);
                     else st_half<N, P, 1>(tile, t, x[0]);
@@ -566,14 +692,25 @@ __device__ __forceinline__ void sfwd_body(const Args &a, const int bid, const in
             if (k == sps - 1 && d.chan_op == 2) mix_phase();
             s = s_next;
         }
-        __syncthreads();
-        if (a.out) {
+        if (!BULK) {
+            __syncthreads();
+            if (a.out) {
 #pragma unroll 1
-            for (int q = 0; q < Q; ++q)
-                PlaneIO<N, P>::from_tile(my + q * TILE, a.out, item * Q + q, t.c, C, d.B, t.tid_c, d.skip ? a.u : nullptr,
-                                         sig, om);
+                for (int q = 0; q < Q; ++q)
+                    PlaneIO<N, P>::from_tile(my + q * SLOT, a.out, item * Q + q, t.c, C, d.B, t.tid_c, d.skip ? a.u : nullptr,
+                                             sig, om);
+            }
+        } else if (!nat_last) {
+            __syncthreads();
+#pragma unroll 1
+            for (int q = 0; q < Q; ++q) {
+                f2 x[H];
+                ld_half<N, P, 0>(my + q * SLOT, t, x);
+                emit(q, x);
+            }
         }
     }
+    if (BULK && threadIdx.x == 0) bulk_wait_all();   // the output stores are complete before the block ends
 }
 
 template <int N, int P, int Q, bool MIX1>
@@ -781,36 +918,44 @@ __device__ __forceinline__ void chan_adjoint(float *ggt, const float *gxt, int c
 // are double buffered and filled asynchronously one stage ahead:
 //   x tiles: TMA bulk copies of the checkpoints (the forward kernel wrote them as tile images),
 //            stream (item, last step) ... (item, step 0), (next item, last step) ...
-//   g tiles: the next item's gout planes by LDGSTS while the current item is reversed.
+//   g tiles: the next item's gout planes by TMA bulk copies while the current item is reversed.
 template <int N, int P, bool CHAN>
 __device__ __forceinline__ void sbwd_body(const Args &a, const int bid, const int nblk) {
     using G = SG<N, P>;
-    constexpr int H = G::H, TILE = G::TILE, HQ4 = 4 * G::HQ;
+    constexpr int H = G::H, TILE = G::TILE, SLOT = G::SLOT, NPI = G::NPITCH, XPI = G::XPITCH, HQ4 = 4 * G::HQ;
+    // the channel ops read x and g tile sets with one channel stride
+    static_assert(!CHAN || SLOT == TILE, "channel ops need tiles and g slots of one size");
     extern __shared__ __align__(128) float smem[];
     __shared__ uint32_t tmem_slot;
     __shared__ __align__(8) uint64_t xbar[2];
+    __shared__ __align__(8) uint64_t gbar[2];
     const pde_adi_desc &d = a.d;
     const Lane t = make_lane<N, P>();
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int C = d.C, nthr = blockDim.x;
     const bool far = t.h == 1;
-    const int CS = TILE;                 // channel stride inside a tile set
-    const int SET = C * TILE;            // floats per tile set
-    constexpr bool GDB = P >= 4;         // second g set: the next item's gout arrives while this one is reversed
+    const int CS = TILE;                 // channel stride inside an x tile set (a checkpoint image)
+    const int SET = C * TILE;            // floats per x tile set
+    const int GSET = C * SLOT;           // floats per g set (channel stride SLOT)
+    // four pairs: second g set, the next item's gout arrives while this one is reversed; plane I/O by bulk
+    // copies (see PlaneIO)
+    constexpr bool GDB = P >= 4;
     // tile sets by offset from the one shared-memory base (pointer arrays indexed at run time would
     // end up in local memory and turn every tile access into a generic load)
     auto xset = [&](int b) { return smem + b * SET; };
-    auto gset = [&](int b) { return smem + (2 + (GDB ? b : 0)) * SET; };
+    auto gset = [&](int b) { return smem + 2 * SET + (GDB ? b : 0) * GSET; };
     // coefficient stage: r and 1/pivot of one sweep (all channels), double buffered, filled by TMA
     // one sweep ahead -- the tables do not survive in what is left of L1 beside the tiles
     const int CT = C * G::HQ * N * 2 * 4;   // floats per table per sweep
-    float *cbuf = smem + (GDB ? 4 : 3) * SET;
+    float *cbuf = smem + 2 * SET + (GDB ? 2 : 1) * GSET;
     __shared__ __align__(8) uint64_t cbar[2];
 
     if (warp == 0) tmem_alloc(&tmem_slot, (uint32_t)a.tmem_cols);
     if (threadIdx.x == 0) {
         mbar_init(&xbar[0], 1);
         mbar_init(&xbar[1], 1);
+        mbar_init(&gbar[0], 1);
+        mbar_init(&gbar[1], 1);
         mbar_init(&cbar[0], 1);
         mbar_init(&cbar[1], 1);
         mbar_fence_init();
@@ -883,36 +1028,62 @@ __device__ __forceinline__ void sbwd_body(const Args &a, const int bid, const in
             tma_load_1d(cbuf + (size_t)(2 * b + 1) * CT, a.stab + T + (size_t)s * CT, bytes, &cbar[b]);
         }
     };
+    // the layer input of group `it`, natural layout (pitch XPI), into x set b: exact recomputation and
+    // the pre-step mix adjoint need it at step 0
+    auto u_xfill = [&](int b, int it) {   // call after a barrier that ends every use of buffer b
+        if (threadIdx.x == 0) {
+            fence_proxy_async();
+            mbar_expect_tx(&xbar[b], (uint32_t)(group_valid<N, P>(it, d.B) * C * plane * sizeof(float)));
+            planes_load<N, P>(xset(b), CS, XPI, a.u, it, C, d.B, &xbar[b]);
+        }
+        xpending |= 1u << b;
+    };
+    auto u_xrows = [&](int b, int it) {   // after x_wait(b): the layer input as rows of x set b
+        const int nv = group_valid<N, P>(it, d.B);
+        if (nv < 2 * P) zero_tail<N, P>(xset(b), CS, XPI, C, nv);
+        __syncthreads();
+        planes_to_rows<N, P, XPI>(xset(b) + (size_t)t.c * CS, t);
+        __syncthreads();
+    };
+    // gout planes of group `it` -> g set b, natural layout; the slot's previous grad_input store must
+    // have been read out first
+    uint32_t gphase = 0u;
+    auto g_fill = [&](int b, int it) {   // call after a barrier that ends every use of set b
+        if (threadIdx.x == 0) {
+            bulk_wait_read<0>();
+            fence_proxy_async();
+            mbar_expect_tx(&gbar[b], (uint32_t)(group_valid<N, P>(it, d.B) * C * plane * sizeof(float)));
+            planes_load<N, P>(gset(b), SLOT, NPI, a.gout, it, C, d.B, &gbar[b]);
+        }
+    };
     int xb = 0, gb = 0, cb = 0;
     if (bid < a.nitems) {
         x_fill(0, bid, d.steps - 1);
         c_fill(0, a.S - 1);
-        if (GDB) {
-            planes_to_tile_async<N, P>(a.gout, gset(0) + (size_t)t.c * CS, bid, t.c, C, d.B, t.tid_c);
-            cp_async_commit();
-        }
+        if (GDB) g_fill(0, bid);
     }
 
     for (int item = bid; item < a.nitems; item += nblk) {
         const int next_item = item + nblk;
-        float *ggt = gset(gb), *gt = ggt + (size_t)t.c * CS;
+        float *ggt = gset(gb), *gt = ggt + (size_t)t.c * SLOT;
+        __syncthreads();   // the previous item's grad_input has been written; nobody reads the other g set
         if (GDB) {
-            cp_async_wait_all();
-            __syncthreads();   // this item's gout tile is complete; nobody still reads the other g set
-            if (next_item < a.nitems) {
-                planes_to_tile_async<N, P>(a.gout, gset(gb ^ 1) + (size_t)t.c * CS, next_item, t.c, C, d.B, t.tid_c);
-                cp_async_commit();
-            }
+            if (next_item < a.nitems) g_fill(gb ^ 1, next_item);
+            const int nv = group_valid<N, P>(item, d.B);
+            if (nv < 2 * P) zero_tail<N, P>(ggt, SLOT, NPI, C, nv);
+            mbar_wait(&gbar[gb], (gphase >> gb) & 1u);
+            gphase ^= 1u << gb;
+            __syncthreads();
+            planes_to_rows<N, P, NPI>(gt, t);
         } else {
-            __syncthreads();   // the previous item's grad_input has left the g set
             PlaneIO<N, P>::to_tile(a.gout, gt, item, t.c, C, d.B, t.tid_c);
             __syncthreads();
         }
         // Which orientation last touched a tile set, and whether a barrier has passed since: a thread
         // only reads and writes its own half line within one orientation, so a barrier is needed
         // exactly when the orientation changes (2 = block-wide access pattern).
-        int x_last = 2, g_last = 2;
-        bool x_sync = true, g_sync = true;
+        int x_last = 2, g_last = GDB ? 0 : 2;
+        bool x_sync = true, g_sync = !GDB;
         auto bar = [&]() {
             __syncthreads();
             x_sync = true;
@@ -975,14 +1146,15 @@ __device__ __forceinline__ void sbwd_body(const Args &a, const int bid, const in
             // every use of the spare buffer (previous step) ends here; start the stage ahead
             bar();
             if (step > 0) x_fill(xb ^ 1, item, step - 1);
+            else if (GDB && defer_cross) u_xfill(xb ^ 1, item);
             else if (!defer_cross && next_item < a.nitems) x_fill(xb ^ 1, next_item, d.steps - 1);
             x_wait(xb);
             if (exact) {
                 // recompute the sweeps of this step from its input (spare buffer), keeping every sweep output
                 f2 x[1][H];
-                if (step > 0) {
-                    x_wait(xb ^ 1);
-                } else {
+                if (GDB || step > 0) x_wait(xb ^ 1);
+                if (GDB && step == 0) u_xrows(xb ^ 1, item);
+                if (!GDB && step == 0) {
                     PlaneIO<N, P>::to_tile(a.u, xs, item, t.c, C, d.B, t.tid_c);
                     __syncthreads();
                 }
@@ -1067,6 +1239,7 @@ __device__ __forceinline__ void sbwd_body(const Args &a, const int bid, const in
             }
             if (CHAN && d.chan_op == 1) {
                 // adjoint of the pre-step mix: needs g (rows) and the mix INPUT = state before this step
+                // (two pairs per group only: CHAN is never instantiated with four)
                 if (step > 0) {
                     x_wait(xb ^ 1);
                 } else {
@@ -1077,15 +1250,28 @@ __device__ __forceinline__ void sbwd_body(const Args &a, const int bid, const in
             }
             xb ^= 1;
         }
-        touch_g(2);
-        if (a.need_gin)
-            PlaneIO<N, P>::from_tile(gt, a.gin, item, t.c, C, d.B, t.tid_c, d.skip ? a.gout : nullptr, sig, 1.0f);
+        if (!GDB) {
+            touch_g(2);
+            if (a.need_gin)
+                PlaneIO<N, P>::from_tile(gt, a.gin, item, t.c, C, d.B, t.tid_c, d.skip ? a.gout : nullptr, sig, 1.0f);
+        } else if (a.need_gin) {   // the g rows -> natural layout (+ skip blend) -> bulk stores
+            touch_g(0);
+            f2 x[H];
+            ld_half<N, P, 0>(gt, t, x);
+            __syncthreads();   // every thread has read its rows of the g set
+            if (t.active) nat_st_half<N, P, NPI>(gt, t, x, d.skip ? a.gout : nullptr, item, t.c, C, d.B, sig, 1.0f);
+            fence_proxy_async();
+            __syncthreads();
+            if (threadIdx.x == 0) planes_store<N, P>(a.gin, ggt, SLOT, NPI, item, C, d.B);
+        }
         if (defer_cross && next_item < a.nitems) {
             __syncthreads();   // the layer input in the spare buffer has been consumed
             x_fill(xb, next_item, d.steps - 1);
         }
         if (GDB) gb ^= 1;
     }
+
+    if (GDB && threadIdx.x == 0) bulk_wait_all();   // the grad_input stores are complete before the block ends
 
     // ------------------------------ partials: TMEM -> sum over the P pairs -> global [row][col]
     tmem_wait_st();
@@ -1156,7 +1342,8 @@ constexpr int kMaxQ = 4;
 
 struct Plan {
     int P, Qf, Qb, threads, wpc, ngroups, tmem_cols;
-    size_t tile_bytes, scr_slot;   // one tile (P pairs of one channel); f2 per sweep output of a block (exact mode)
+    size_t tile_bytes, slot_bytes, scr_slot;   // one tile (P pairs of one channel); one tile slot (SG::SLOT); f2 per
+                                               // sweep output of a block (exact mode)
 };
 
 template <int N, int P>
@@ -1165,6 +1352,7 @@ static void fill_geo(const pde_adi_desc &d, Plan *p) {
     p->wpc = G::WPC;
     p->threads = G::WPC * 32 * d.C;
     p->tile_bytes = (size_t)G::TILE * sizeof(float);
+    p->slot_bytes = (size_t)G::SLOT * sizeof(float);
     p->scr_slot = (size_t)G::H * p->threads;
 }
 
@@ -1195,7 +1383,7 @@ static int make_plan(const pde_adi_desc &d, Plan *p) {
                                          : (size_t)227 * 1024 / blocks_per_sm - coef_stage - 2048;
     auto pick = [&](int qmax, size_t tiles_per_group, int forced) {
         int q = qmax;
-        while (q > 1 && ((p->ngroups + q - 1) / q < 2 * sm || (size_t)q * tiles_per_group * p->tile_bytes > tile_budget)) q >>= 1;
+        while (q > 1 && ((p->ngroups + q - 1) / q < 2 * sm || (size_t)q * tiles_per_group * p->slot_bytes > tile_budget)) q >>= 1;
         if (forced == 1 || forced == 2 || (forced == 4 && qmax == 4)) q = forced;
         return q;
     };
@@ -1282,8 +1470,8 @@ static int plan_bwd_grid(const pde_adi_desc &d, const Plan &p, BwdLaunch *b, con
     if (rc) return rc;
     const void *kern = kern_override ? kern_override : bwd_kernel_for(d.N, p.P, d.chan_op != 0);
     if (!kern) return PDE_ERR_UNSUPPORTED;
-    // x tile sets double buffered, g sets too for P == 4, two coefficient stages of two tables
-    b->smem = (size_t)(p.P >= 4 ? 4 : 3) * d.C * p.tile_bytes + (size_t)4 * d.C * ((d.N / 2 + 3) / 4) * d.N * 2 * 16;
+    // x tile sets double buffered, g sets (tile slots) too for P == 4, two coefficient stages of two tables
+    b->smem = (size_t)2 * d.C * p.tile_bytes + (size_t)(p.P >= 4 ? 2 : 1) * d.C * p.slot_bytes + (size_t)4 * d.C * ((d.N / 2 + 3) / 4) * d.N * 2 * 16;
     if (b->smem > (size_t)props.max_smem_optin) return PDE_ERR_UNSUPPORTED;
     // residency from first principles (the occupancy calculator answers 1 block / SM for kernels
     // that allocate tensor memory)
@@ -1347,6 +1535,7 @@ static void fill_args(const pde_adi_desc &d, const char *tables, Args *a) {
 
 int forward(const pde_adi_desc &d, const char *tables, const float *u, const float *chan, const float *skipw,
             float *out, float *ckpt, cudaStream_t st) {
+    if (!aligned16(u) || !aligned16(out)) return PDE_ERR_UNSUPPORTED;   // planes move by bulk copies
     Plan p;
     int rc = make_plan(d, &p);
     if (rc) return rc;
@@ -1356,7 +1545,7 @@ int forward(const pde_adi_desc &d, const char *tables, const float *u, const flo
     const void *kern = fwd_kernel_for(d.N, p.P, p.Qf, d.chan_op == 1);
     if (!kern) return PDE_ERR_UNSUPPORTED;
     // Qf groups of tiles, two coefficient stages of two tables
-    const size_t smem = (size_t)d.C * p.Qf * p.tile_bytes + (size_t)4 * d.C * ((d.N / 2 + 3) / 4) * d.N * 2 * 16;
+    const size_t smem = (size_t)d.C * p.Qf * p.slot_bytes + (size_t)4 * d.C * ((d.N / 2 + 3) / 4) * d.N * 2 * 16;
     if (smem > (size_t)props.max_smem_optin) return PDE_ERR_UNSUPPORTED;
     int per_sm = 1;
     rc = cached_occupancy(kern, p.threads, smem, &per_sm);
@@ -1383,6 +1572,7 @@ int forward(const pde_adi_desc &d, const char *tables, const float *u, const flo
 int backward(const pde_adi_desc &d, const char *tables, const float *u, const float *gout, const float *chan,
              const float *skipw, const float *ckpt, float *gin, float *g_ab, float *g_bb, float *g_atc, float *g_btc,
              float *g_chan, float *g_skip, void *workspace, size_t workspace_bytes_, cudaStream_t st) {
+    if (!aligned16(u) || !aligned16(gout) || !aligned16(gin)) return PDE_ERR_UNSUPPORTED;   // planes move by bulk copies
     Plan p;
     BwdLaunch b;
     int rc = make_plan(d, &p);
@@ -1475,6 +1665,9 @@ static float *ck_images(void *ckpt, CkFlags **flags) {   // [CkFlags, 256 bytes]
 
 int forward_multi(int n, const pde_adi_desc *d, const void *const *tables, const float *u, const float *const *chan,
                   const float *const *skipw, float *const *out, void *const *ckpt, cudaStream_t st) {
+    if (!aligned16(u)) return PDE_ERR_UNSUPPORTED;   // planes move by bulk copies
+    for (int i = 0; i < n; ++i)
+        if (!aligned16(out[i])) return PDE_ERR_UNSUPPORTED;
     Plan p;
     int rc = make_plan(d[0], &p);
     if (rc) return rc;
@@ -1483,7 +1676,7 @@ int forward_multi(int n, const pde_adi_desc *d, const void *const *tables, const
     if (rc) return rc;
     const void *kern = fwd_multi_kernel_for(d[0].N, p.P, p.Qf, d[0].chan_op == 1);
     if (!kern) return PDE_ERR_UNSUPPORTED;
-    const size_t smem = (size_t)d[0].C * p.Qf * p.tile_bytes + (size_t)4 * d[0].C * ((d[0].N / 2 + 3) / 4) * d[0].N * 2 * 16;
+    const size_t smem = (size_t)d[0].C * p.Qf * p.slot_bytes + (size_t)4 * d[0].C * ((d[0].N / 2 + 3) / 4) * d[0].N * 2 * 16;
     if (smem > (size_t)props.max_smem_optin) return PDE_ERR_UNSUPPORTED;
     int per_sm = 1;
     rc = cached_occupancy(kern, p.threads, smem, &per_sm);
@@ -1514,6 +1707,9 @@ int backward_multi(int n, const pde_adi_desc *d, const void *const *tables, cons
                    const float *const *chan, const float *const *skipw, const void *const *ckpt, float *const *gin,
                    float *const *g_ab, float *const *g_bb, float *const *g_atc, float *const *g_btc, float *const *g_chan,
                    float *const *g_skip, void *const *workspace, const size_t *workspace_bytes_, cudaStream_t st) {
+    if (!aligned16(u)) return PDE_ERR_UNSUPPORTED;   // planes move by bulk copies
+    for (int i = 0; i < n; ++i)
+        if (!aligned16(gout[i]) || (gin && !aligned16(gin[i]))) return PDE_ERR_UNSUPPORTED;
     Plan p;
     BwdLaunch b;
     int rc = make_plan(d[0], &p);

@@ -209,6 +209,21 @@ __device__ __forceinline__ void tma_load_1d(void *dst_smem, const void *src_gmem
                  : "memory");
 }
 
+// shared -> global, tracked in the issuing thread's bulk groups (commit, then wait_group)
+__device__ __forceinline__ void tma_store_1d(void *dst_gmem, const void *src_smem, uint32_t bytes) {
+    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst_gmem), "r"(smem_u32(src_smem)),
+                 "r"(bytes)
+                 : "memory");
+}
+__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
+// at most N of the thread's bulk groups still read shared memory (their source may then be refilled)
+template <int N>
+__device__ __forceinline__ void bulk_wait_read() {
+    asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory");
+}
+// every bulk group of the thread is complete (its global writes done)
+__device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
+
 // order prior generic-proxy accesses to shared memory before later async-proxy (TMA) accesses
 __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 

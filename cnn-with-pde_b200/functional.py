@@ -78,7 +78,11 @@ def _bytes(n: int, device) -> torch.Tensor:
 
 
 def _contig(t):
-    return t if t.is_contiguous() else t.contiguous()
+    """Contiguous and 16-byte aligned: the half-line ADI kernels move whole planes by bulk copies,
+    which need 16-byte-aligned addresses.  A view at an odd offset of its storage is copied."""
+    if t.is_contiguous() and t.data_ptr() % 16 == 0:
+        return t
+    return t.clone(memory_format=torch.contiguous_format)
 
 
 def env_tuning() -> int:

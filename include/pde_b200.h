@@ -111,7 +111,10 @@ int pde_adi_prepare(const pde_adi_desc *d, const pde_adi_schedule *sched,
                     const float *alpha_time_coeff, const float *beta_time_coeff,
                     void *tables, void *stream);
 
-/* u, out: [B][C][N][N].  chan: [C][C] or NULL (chan_op == 0).  skip_weight: 1 value or NULL. */
+/* u, out: [B][C][N][N].  chan: [C][C] or NULL (chan_op == 0).  skip_weight: 1 value or NULL.
+ * Where pde_adi_checkpoint_bytes(d) != 0, the training entry points below (pde_adi_forward_train,
+ * pde_adi_backward_saved, pde_adi_backward and the multi-layer ones) move whole planes by bulk copies:
+ * u, out, gout and gin must then be 16-byte aligned, and a misaligned one gives PDE_ERR_UNSUPPORTED. */
 int pde_adi_forward(const pde_adi_desc *d, const void *tables, const float *u,
                     const float *chan, const float *skip_weight, float *out, void *stream);
 
