@@ -17,6 +17,7 @@ There is no CPU path: inputs must be CUDA float tensors and the library must be 
 """
 from . import _cabi  # noqa: F401
 from .functional import AdiConfig, EmoConfig, TinyConfig, adi_layer, emotion_layer, tiny_layer  # noqa: F401
+from . import ops  # noqa: F401,E402  (registers the pde_b200:: custom ops that traced calls go through)
 from . import mnist_test, fashion_mnist, SVHN, cifar10, cifar_2version, emotion_recognition, tiny_imagenet  # noqa: F401,E402
 
 __all__ = ["mnist_test", "fashion_mnist", "SVHN", "cifar10", "cifar_2version", "emotion_recognition",

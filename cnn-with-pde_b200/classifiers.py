@@ -25,6 +25,8 @@ import torch
 import torch.nn as nn
 import torch.nn.functional as F
 
+from .functional import _traced
+
 
 # side streams of the branch-parallel extractors: per device, shared by all modules (kept out of the modules'
 # __dict__ so that copy.deepcopy / pickling of a model that has already run keeps working)
@@ -169,7 +171,9 @@ class MultiScaleExtractor(nn.Module):
 
     def forward(self, x):
         branches = ((self.pde1, self.attention1), (self.pde2, self.attention2), (self.pde3, self.attention3))
-        serial = bool(os.environ.get("PDE_B200_SERIAL_BRANCHES"))
+        # a traced call (torch.compile, torch.export, shape inference) takes the serial branch: the same values,
+        # without side streams or an environment read
+        serial = _traced(x) or bool(os.environ.get("PDE_B200_SERIAL_BRANCHES"))
         if x.is_cuda and self.fused_branches and not serial and torch.is_grad_enabled():
             from .cifar10 import apply_to_same_input
             ys = apply_to_same_input(x, [pde for pde, _ in branches])
@@ -345,7 +349,7 @@ class HybridPDEExtractor(nn.Module):
     fused_branches = False   # see MultiScaleExtractor
 
     def forward(self, x):
-        serial = bool(os.environ.get("PDE_B200_SERIAL_BRANCHES"))
+        serial = _traced(x) or bool(os.environ.get("PDE_B200_SERIAL_BRANCHES"))   # see MultiScaleExtractor
         if x.is_cuda and self.fused_branches and not serial and torch.is_grad_enabled():
             from .cifar10 import apply_to_same_input
             d1, d2 = apply_to_same_input(x, [self.diffusion1, self.diffusion2])   # one launch per pass for both

@@ -23,9 +23,17 @@ from ctypes import byref
 from dataclasses import dataclass
 
 import torch
+from torch._subclasses.fake_tensor import FakeTensor
 
 from . import _cabi
 from .schedule import adi_schedule
+
+
+def _traced(t) -> bool:
+    """Whether a layer call is traced rather than run: under torch.compile, or on FakeTensor / meta-device inputs
+    (torch.export, shape inference).  Such calls go through the custom ops of ops.py, which Dynamo and FakeTensor
+    mode can see through; a call on real tensors keeps the autograd.Functions below (less host time per call)."""
+    return torch.compiler.is_compiling() or isinstance(t, FakeTensor) or (isinstance(t, torch.Tensor) and t.is_meta)
 
 
 def _require_cuda(x: torch.Tensor, what: str):
@@ -106,6 +114,12 @@ def env_tuning() -> int:
     return _cabi.adi_tuning(impl, num("PDE_B200_SPLIT_P"), num("PDE_B200_SPLIT_QF"), num("PDE_B200_FWD_NP"))
 
 
+@torch.compiler.assume_constant_result
+def _traced_tuning() -> int:
+    """env_tuning() for a traced call: Dynamo takes the value as a constant of the graph."""
+    return env_tuning()
+
+
 _TUNING_KEYS = ("PDE_B200_ADI_LEGACY", "PDE_B200_ADI_SPLIT", "PDE_B200_SPLIT_P", "PDE_B200_SPLIT_QF", "PDE_B200_FWD_NP")
 _TUNING_KEYS_B = frozenset(k.encode() for k in _TUNING_KEYS)
 
@@ -128,12 +142,14 @@ class AdiConfig:
     cmax: float = 10.0
     eps: float = 1e-6
 
-    def __post_init__(self):
-        object.__setattr__(self, "_hash", hash((self.N, self.C, self.steps, self.dt, self.hx, self.hy, self.lie, self.smooth,
-                                                self.has_max, self.chan_op, self.skip, self.cmin, self.cmax, self.eps)))
-
-    def __hash__(self):   # computed once: the configuration keys the plan cache on every call
-        return self._hash
+    def __hash__(self):   # computed once (on first use, so that Dynamo can build a configuration): it keys the plan cache
+        try:
+            return self._hash
+        except AttributeError:
+            h = hash((self.N, self.C, self.steps, self.dt, self.hx, self.hy, self.lie, self.smooth, self.has_max,
+                      self.chan_op, self.skip, self.cmin, self.cmax, self.eps))
+            object.__setattr__(self, "_hash", h)
+            return h
 
     def desc(self, B: int, tuning: int = 0) -> "_cabi.AdiDesc":
         return _cabi.AdiDesc(B, self.C, self.N, self.steps, int(self.lie), int(self.smooth), int(self.has_max),
@@ -196,81 +212,109 @@ def _remember_tables(key, params, tables):
     _table_cache[key] = (tables, tuple(weakref.ref(p) for p in params), tuple(p._version for p in params))
 
 
+def _adi_tables_forward(u, params, chan, skipw, cfg: AdiConfig, tuning: int, training: bool, reuse_tables: bool):
+    """The forward pass on the shared-memory kernels: coefficient tables (or the cached ones of an inference call
+    while `reuse_tables`), then the forward kernel, writing step checkpoints while `training`.  Returns
+    (out, tables, ckpt or None, plan, u, chan, skip), the last three as the kernels read them."""
+    _require_cuda(u, "PDE layer input")
+    L = _cabi.lib()
+    u = _contig(u)
+    maps = [_contig(p) for p in params]
+    for p in maps:
+        _require_cuda(p, "PDE layer parameter")
+    chan_c = None if chan is None else _contig(chan.detach())
+    skip_c = None if skipw is None else _contig(skipw.detach())
+    dev = u.device
+    with _guard(dev):
+        # (the plan asks the library about the CURRENT device: built under the guard)
+        plan = _adi_plan(cfg, u.shape[0], tuning, dev.index if dev.index is not None else torch.cuda.current_device())
+        st = _stream(dev)
+        tables, key = None, None
+        if reuse_tables and not training and not torch.cuda.is_current_stream_capturing():
+            key, tables = _cached_tables(plan, params)
+        if tables is None:
+            # a traced call's tables are an output of its op: zeroed, so that the bytes prepare leaves unwritten
+            # (alignment padding) are the same in every run
+            tables = _bytes(plan.tables_bytes, dev) if reuse_tables else torch.zeros(plan.tables_bytes, dtype=torch.uint8,
+                                                                                     device=dev)
+            _cabi.check(L.pde_adi_prepare(plan.dref, plan.sref, *[p.data_ptr() for p in maps], tables.data_ptr(), st),
+                        "pde_adi_prepare")
+            if key is not None:
+                _remember_tables(key, params, tables)
+        out = torch.empty_like(u)
+        # under autograd the forward kernel also writes the state at the end of every step for
+        # the backward kernel (0 bytes when the configuration is served by the kernels that
+        # rebuild the trajectory on-chip).  PDE_B200_NO_CKPT=1 trades them for a recomputation
+        # inside pde_adi_backward (saves num_steps x the input in memory between the passes)
+        ck_bytes = plan.ckpt_bytes if training and not os.environ.get("PDE_B200_NO_CKPT") else 0
+        ckpt = _bytes(ck_bytes, dev) if ck_bytes else None
+        _cabi.check(L.pde_adi_forward_train(plan.dref, tables.data_ptr(), _ptr(u), _ptr(chan_c), _ptr(skip_c), _ptr(out),
+                                            _ptr(ckpt), st), "pde_adi_forward_train")
+    return out, tables, ckpt, plan, u, chan_c, skip_c
+
+
+def _adi_grad_buffers(cfg: AdiConfig, u, param_shape, has_chan: bool, has_skip: bool, need_gin: bool):
+    """grad_input (or None), the four coefficient-map gradients in one allocation, g_chan and g_skip (or None)."""
+    dev = u.device
+    gin = torch.empty_like(u) if need_gin else None
+    gm = torch.empty((4,) + tuple(param_shape), dtype=torch.float32, device=dev)
+    gchan = torch.empty((cfg.C, cfg.C), dtype=torch.float32, device=dev) if has_chan else None
+    gskip = torch.empty((), dtype=torch.float32, device=dev) if has_skip else None
+    return gin, gm, gchan, gskip
+
+
+def _float_grad(gout):
+    gout = _contig(gout)
+    return gout if gout.dtype == torch.float32 else gout.float()
+
+
+def _adi_tables_backward(plan, u, tables, chan, skipw, ckpt, gout, param_shape, need_gin: bool):
+    """The backward pass on the shared-memory kernels, from the checkpoints of the forward call or -- ckpt None --
+    recomputing them in a batch-sized workspace.  Returns (gin or None, the four map gradients as one (4, ...)
+    tensor, g_chan or None, g_skip or None)."""
+    L = _cabi.lib()
+    gout = _float_grad(gout)
+    dev = u.device
+    with _guard(dev):
+        ws_bytes = plan.ws_saved_bytes if ckpt is not None else plan.ws_bytes
+        ws = _bytes(ws_bytes, dev)
+        gin, gm, gchan, gskip = _adi_grad_buffers(plan.cfg, u, param_shape, chan is not None, skipw is not None, need_gin)
+        base, plane = gm.data_ptr(), plan.grad_numel
+        _cabi.check(L.pde_adi_backward_saved(plan.dref, tables.data_ptr(), _ptr(u), _ptr(gout), _ptr(chan), _ptr(skipw),
+                                             _ptr(ckpt), _ptr(gin), base, base + plane, base + 2 * plane, base + 3 * plane,
+                                             _ptr(gchan), _ptr(gskip), ws.data_ptr(), ws_bytes, _stream(dev)),
+                    "pde_adi_backward_saved")
+    return gin, gm, gchan, gskip
+
+
 class _AdiFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, u, alpha_base, beta_base, alpha_tc, beta_tc, chan, skipw, cfg: AdiConfig, grad_mode: bool = True):
-        _require_cuda(u, "PDE layer input")
-        L = _cabi.lib()
-        u = _contig(u)
-        maps = [_contig(p) for p in (alpha_base, beta_base, alpha_tc, beta_tc)]
-        for p in maps:
-            _require_cuda(p, "PDE layer parameter")
-        chan_c = None if chan is None else _contig(chan.detach())
-        skip_c = None if skipw is None else _contig(skipw.detach())
-        dev = u.device
         # needs_input_grad ignores torch.no_grad() and grad mode is always off inside forward(): the
         # caller passes the mode it saw
         training = grad_mode and any(ctx.needs_input_grad)
-        with _guard(dev):
-            # (the plan asks the library about the CURRENT device: built under the guard)
-            plan = _adi_plan(cfg, u.shape[0], env_tuning(), dev.index if dev.index is not None else torch.cuda.current_device())
-            st = _stream(dev)
-            tables, key = None, None
-            if not training and not torch.cuda.is_current_stream_capturing():
-                key, tables = _cached_tables(plan, (alpha_base, beta_base, alpha_tc, beta_tc))
-            if tables is None:
-                tables = _bytes(plan.tables_bytes, dev)
-                _cabi.check(L.pde_adi_prepare(plan.dref, plan.sref, *[p.data_ptr() for p in maps], tables.data_ptr(), st),
-                            "pde_adi_prepare")
-                if key is not None:
-                    _remember_tables(key, (alpha_base, beta_base, alpha_tc, beta_tc), tables)
-            out = torch.empty_like(u)
-            # under autograd the forward kernel also writes the state at the end of every step for
-            # the backward kernel (0 bytes when the configuration is served by the kernels that
-            # rebuild the trajectory on-chip).  PDE_B200_NO_CKPT=1 trades them for a recomputation
-            # inside pde_adi_backward (saves num_steps x the input in memory between the passes)
-            ck_bytes = plan.ckpt_bytes if training and not os.environ.get("PDE_B200_NO_CKPT") else 0
-            ckpt = _bytes(ck_bytes, dev) if ck_bytes else None
-            _cabi.check(L.pde_adi_forward_train(plan.dref, tables.data_ptr(), _ptr(u), _ptr(chan_c), _ptr(skip_c), _ptr(out),
-                                                _ptr(ckpt), st), "pde_adi_forward_train")
+        params = (alpha_base, beta_base, alpha_tc, beta_tc)
+        out, tables, ckpt, plan, u, chan_c, skip_c = _adi_tables_forward(u, params, chan, skipw, cfg, env_tuning(), training,
+                                                                         True)
         ctx.plan = plan   # the descriptor (tuning included) the backward pass must use as well
         ctx.has_chan = chan is not None
         ctx.has_skip = skipw is not None
         ctx.has_ckpt = ckpt is not None
         ctx.save_for_backward(u, tables, *(t for t in (chan_c, skip_c, ckpt) if t is not None))
-        ctx.param_shapes = [p.shape for p in (alpha_base, beta_base, alpha_tc, beta_tc)]
+        ctx.param_shape = alpha_base.shape
         return out
 
     @staticmethod
     def backward(ctx, gout):
         _no_double_backward("PDE layer")
-        L = _cabi.lib()
-        plan = ctx.plan
-        cfg = plan.cfg
         saved = list(ctx.saved_tensors)
         u, tables = saved[0], saved[1]
         rest = saved[2:]
         chan = rest.pop(0) if ctx.has_chan else None
         skipw = rest.pop(0) if ctx.has_skip else None
         ckpt = rest.pop(0) if ctx.has_ckpt else None
-        gout = _contig(gout)
-        if gout.dtype != torch.float32:
-            gout = gout.float()
-        dev = u.device
-        with _guard(dev):
-            ws_bytes = plan.ws_saved_bytes if ckpt is not None else plan.ws_bytes
-            ws = _bytes(ws_bytes, dev)
-            gin = torch.empty_like(u) if ctx.needs_input_grad[0] else None
-            # the four coefficient-map gradients share one allocation (one unbind instead of four views)
-            C, N = cfg.C, cfg.N
-            gm = torch.empty((4,) + tuple(ctx.param_shapes[0]), dtype=torch.float32, device=dev)
-            base, plane = gm.data_ptr(), 4 * C * N * N
-            gchan = torch.empty((C, C), dtype=torch.float32, device=dev) if chan is not None else None
-            gskip = torch.empty((), dtype=torch.float32, device=dev) if skipw is not None else None
-            _cabi.check(L.pde_adi_backward_saved(plan.dref, tables.data_ptr(), _ptr(u), _ptr(gout), _ptr(chan), _ptr(skipw),
-                                                 _ptr(ckpt), _ptr(gin), base, base + plane, base + 2 * plane, base + 3 * plane,
-                                                 _ptr(gchan), _ptr(gskip), ws.data_ptr(), ws_bytes, _stream(dev)),
-                        "pde_adi_backward_saved")
+        gin, gm, gchan, gskip = _adi_tables_backward(ctx.plan, u, tables, chan, skipw, ckpt, gout, ctx.param_shape,
+                                                     ctx.needs_input_grad[0])
         gmaps = gm.unbind(0)
         return (gin, gmaps[0], gmaps[1], gmaps[2], gmaps[3], gchan, gskip, None, None)
 
@@ -312,66 +356,83 @@ def _adi_stream_plan(cfg: AdiConfig, B: int, device_index: int) -> _AdiStreamPla
     return _AdiStreamPlan(cfg, B)
 
 
+def _adi_stream_forward(u, params, chan, skipw, cfg: AdiConfig):
+    """The forward pass on the streaming kernels.  Returns (out, plan, u, maps, chan, skip), the last four as the
+    kernels read them."""
+    _require_cuda(u, "PDE layer input")
+    L = _cabi.lib()
+    u = _contig(u)
+    maps = [_contig(p.detach()) for p in params]
+    for p in maps:
+        _require_cuda(p, "PDE layer parameter")
+    chan_c = None if chan is None else _contig(chan.detach())
+    skip_c = None if skipw is None else _contig(skipw.detach())
+    dev = u.device
+    with _guard(dev):
+        plan = _adi_stream_plan(cfg, u.shape[0], dev.index if dev.index is not None else torch.cuda.current_device())
+        ws = _bytes(plan.fwd_bytes, dev)
+        out = torch.empty_like(u)
+        _cabi.check(L.pde_adi_stream_forward(plan.dref, plan.sref, *[p.data_ptr() for p in maps], _ptr(u), _ptr(chan_c),
+                                             _ptr(skip_c), _ptr(out), ws.data_ptr(), plan.fwd_bytes, _stream(dev)),
+                    "pde_adi_stream_forward")
+    return out, plan, u, maps, chan_c, skip_c
+
+
+def _adi_stream_backward(plan, u, maps, chan, skipw, gout, param_shape, need_gin: bool):
+    """The backward pass on the streaming kernels (it replays the trajectory itself).  Returns what
+    _adi_tables_backward returns."""
+    L = _cabi.lib()
+    gout = _float_grad(gout)
+    dev = u.device
+    with _guard(dev):
+        ws = _bytes(plan.bwd_bytes, dev)
+        gin, gm, gchan, gskip = _adi_grad_buffers(plan.cfg, u, param_shape, chan is not None, skipw is not None, need_gin)
+        C, N = plan.cfg.C, plan.cfg.N
+        base, plane = gm.data_ptr(), 4 * C * N * N
+        _cabi.check(L.pde_adi_stream_backward(plan.dref, plan.sref, *[m.data_ptr() for m in maps], _ptr(u), _ptr(gout),
+                                              _ptr(chan), _ptr(skipw), _ptr(gin), base, base + plane, base + 2 * plane,
+                                              base + 3 * plane, _ptr(gchan), _ptr(gskip), ws.data_ptr(), plan.bwd_bytes,
+                                              _stream(dev)), "pde_adi_stream_backward")
+    return gin, gm, gchan, gskip
+
+
 class _AdiStreamFunction(torch.autograd.Function):
     """The implicit layer on the streaming kernels: the factor tables are built inside each call, and the backward
     pass replays the trajectory itself, so only the input and the parameters are kept between the passes."""
 
     @staticmethod
     def forward(ctx, u, alpha_base, beta_base, alpha_tc, beta_tc, chan, skipw, cfg: AdiConfig):
-        _require_cuda(u, "PDE layer input")
-        L = _cabi.lib()
-        u = _contig(u)
-        maps = [_contig(p.detach()) for p in (alpha_base, beta_base, alpha_tc, beta_tc)]
-        for p in maps:
-            _require_cuda(p, "PDE layer parameter")
-        chan_c = None if chan is None else _contig(chan.detach())
-        skip_c = None if skipw is None else _contig(skipw.detach())
-        dev = u.device
-        with _guard(dev):
-            plan = _adi_stream_plan(cfg, u.shape[0], dev.index if dev.index is not None else torch.cuda.current_device())
-            ws = _bytes(plan.fwd_bytes, dev)
-            out = torch.empty_like(u)
-            _cabi.check(L.pde_adi_stream_forward(plan.dref, plan.sref, *[p.data_ptr() for p in maps], _ptr(u), _ptr(chan_c),
-                                                 _ptr(skip_c), _ptr(out), ws.data_ptr(), plan.fwd_bytes, _stream(dev)),
-                        "pde_adi_stream_forward")
+        out, plan, u, maps, chan_c, skip_c = _adi_stream_forward(u, (alpha_base, beta_base, alpha_tc, beta_tc), chan, skipw,
+                                                                 cfg)
         ctx.plan = plan
         ctx.has_chan = chan is not None
         ctx.has_skip = skipw is not None
         ctx.save_for_backward(u, *maps, *(t for t in (chan_c, skip_c) if t is not None))
-        ctx.param_shapes = [p.shape for p in (alpha_base, beta_base, alpha_tc, beta_tc)]
+        ctx.param_shape = alpha_base.shape
         return out
 
     @staticmethod
     def backward(ctx, gout):
         _no_double_backward("PDE layer")
-        L = _cabi.lib()
-        plan = ctx.plan
         saved = list(ctx.saved_tensors)
         u, maps, rest = saved[0], saved[1:5], saved[5:]
         chan = rest.pop(0) if ctx.has_chan else None
         skipw = rest.pop(0) if ctx.has_skip else None
-        gout = _contig(gout)
-        if gout.dtype != torch.float32:
-            gout = gout.float()
-        dev = u.device
-        with _guard(dev):
-            ws = _bytes(plan.bwd_bytes, dev)
-            gin = torch.empty_like(u) if ctx.needs_input_grad[0] else None
-            C, N = plan.cfg.C, plan.cfg.N
-            gm = torch.empty((4,) + tuple(ctx.param_shapes[0]), dtype=torch.float32, device=dev)
-            base, plane = gm.data_ptr(), 4 * C * N * N
-            gchan = torch.empty((C, C), dtype=torch.float32, device=dev) if chan is not None else None
-            gskip = torch.empty((), dtype=torch.float32, device=dev) if skipw is not None else None
-            _cabi.check(L.pde_adi_stream_backward(plan.dref, plan.sref, *[m.data_ptr() for m in maps], _ptr(u), _ptr(gout),
-                                                  _ptr(chan), _ptr(skipw), _ptr(gin), base, base + plane, base + 2 * plane,
-                                                  base + 3 * plane, _ptr(gchan), _ptr(gskip), ws.data_ptr(), plan.bwd_bytes,
-                                                  _stream(dev)), "pde_adi_stream_backward")
+        gin, gm, gchan, gskip = _adi_stream_backward(ctx.plan, u, maps, chan, skipw, gout, ctx.param_shape,
+                                                     ctx.needs_input_grad[0])
         gmaps = gm.unbind(0)
         return (gin, gmaps[0], gmaps[1], gmaps[2], gmaps[3], gchan, gskip, None)
 
 
 def adi_layer(u, alpha_base, beta_base, alpha_tc, beta_tc, chan, skipw, cfg: AdiConfig):
     u = _autocast_to_fp32(u)
+    if _traced(u):
+        # the condition under which _AdiFunction writes checkpoints: it also selects the forward kernel
+        training = torch.is_grad_enabled() and any(t is not None and t.requires_grad
+                                                   for t in (u, alpha_base, beta_base, alpha_tc, beta_tc, chan, skipw))
+        return torch.ops.pde_b200.adi_fwd(u, alpha_base, beta_base, alpha_tc, beta_tc, chan, skipw, cfg.N, cfg.C, cfg.steps,
+                                          cfg.dt, cfg.hx, cfg.hy, cfg.lie, cfg.smooth, cfg.has_max, cfg.chan_op, cfg.skip,
+                                          cfg.cmin, cfg.cmax, cfg.eps, _traced_tuning(), training)[0]
     if isinstance(u, torch.Tensor) and u.is_cuda and adi_route(cfg) == "stream":
         return _AdiStreamFunction.apply(u, alpha_base, beta_base, alpha_tc, beta_tc, chan, skipw, cfg)
     return _AdiFunction.apply(u, alpha_base, beta_base, alpha_tc, beta_tc, chan, skipw, cfg, torch.is_grad_enabled())
@@ -500,7 +561,8 @@ def adi_multi_layer(u, branches):
     half-line kernels do not serve, planes on the streaming kernels, inference)."""
     u = _autocast_to_fp32(u)
     cfgs = tuple(b[6] for b in branches)
-    fused = u.is_cuda and torch.is_grad_enabled() and any(t is not None and t.requires_grad for b in branches for t in b[:6])
+    # (a traced call takes one op per layer: whether the layers can share a launch is a library query)
+    fused = not _traced(u) and u.is_cuda and torch.is_grad_enabled() and any(t is not None and t.requires_grad for b in branches for t in b[:6])
     # the multi-branch launches are built on the shared-memory kernels: a stream-routed branch means one call per layer
     fused = fused and all(adi_route(c) == "tables" for c in cfgs)
     if fused:
@@ -545,21 +607,45 @@ def _emo_plan(cfg: EmoConfig, B: int, generic: bool, device_index: int):
     return d, byref(d), _cabi.lib().pde_emotion_backward_workspace_bytes(byref(d))
 
 
+def _emotion_forward(u0, w6, xs, ys, cfg: EmoConfig, generic: bool):
+    """The emotion layer's forward pass.  Returns (out, plan, u0, w6, xs, ys), the last four as the kernels read them."""
+    _require_cuda(u0, "PDELayer input")
+    L = _cabi.lib()
+    dev = u0.device
+    plan = _emo_plan(cfg, u0.shape[0], generic, dev.index if dev.index is not None else torch.cuda.current_device())
+    u0 = _contig(u0)
+    w6c, xs, ys = _contig(w6.detach()), _contig(xs), _contig(ys)
+    with _guard(u0.device):
+        out = torch.empty_like(u0)
+        _emo_check(L.pde_emotion_forward(plan[1], _ptr(u0), _ptr(w6c), _ptr(xs), _ptr(ys), _ptr(out), _stream(u0.device)),
+                   plan[0], "pde_emotion_forward")
+    return out, plan, u0, w6c, xs, ys
+
+
+def _emotion_backward(plan, u0, w6, xs, ys, gout, need_gin: bool):
+    """The emotion layer's backward pass.  Returns (gin or None, g_w6)."""
+    L = _cabi.lib()
+    gout = _float_grad(gout)
+    d, dref, ws_bytes = plan
+    if ws_bytes == 0:
+        raise _tiny_refused(d)
+    with _guard(u0.device):
+        ws = _bytes(ws_bytes, u0.device)
+        gin = torch.empty_like(u0) if need_gin else None
+        gw = torch.empty(6, dtype=torch.float32, device=u0.device)
+        _emo_check(L.pde_emotion_backward(dref, _ptr(u0), _ptr(gout), _ptr(w6), _ptr(xs), _ptr(ys), _ptr(gin),
+                                          _ptr(gw), _ptr(ws), ws_bytes, _stream(u0.device)), d, "pde_emotion_backward")
+    return gin, gw
+
+
+def _emo_generic() -> bool:
+    return os.environ.get("PDE_B200_EMO_TILED") == "0"
+
+
 class _EmotionFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, u0, w6, xs, ys, cfg: EmoConfig):
-        _require_cuda(u0, "PDELayer input")
-        L = _cabi.lib()
-        u0 = _contig(u0)
-        w6c, xs, ys = _contig(w6.detach()), _contig(xs), _contig(ys)
-        dev = u0.device
-        plan = _emo_plan(cfg, u0.shape[0], os.environ.get("PDE_B200_EMO_TILED") == "0",
-                         dev.index if dev.index is not None else torch.cuda.current_device())
-        d = plan[0]
-        with _guard(u0.device):
-            out = torch.empty_like(u0)
-            _emo_check(L.pde_emotion_forward(plan[1], _ptr(u0), _ptr(w6c), _ptr(xs), _ptr(ys), _ptr(out), _stream(u0.device)),
-                       d, "pde_emotion_forward")
+        out, plan, u0, w6c, xs, ys = _emotion_forward(u0, w6, xs, ys, cfg, _emo_generic())
         ctx.plan = plan   # the backward pass uses the same descriptor (tuning included)
         ctx.save_for_backward(u0, w6c, xs, ys)
         return out
@@ -567,25 +653,21 @@ class _EmotionFunction(torch.autograd.Function):
     @staticmethod
     def backward(ctx, gout):
         _no_double_backward("PDELayer")
-        L = _cabi.lib()
         u0, w6, xs, ys = ctx.saved_tensors
-        gout = _contig(gout)
-        if gout.dtype != torch.float32:
-            gout = gout.float()
-        d, dref, ws_bytes = ctx.plan
-        if ws_bytes == 0:
-            raise _tiny_refused(d)
-        with _guard(u0.device):
-            ws = _bytes(ws_bytes, u0.device)
-            gin = torch.empty_like(u0) if ctx.needs_input_grad[0] else None
-            gw = torch.empty(6, dtype=torch.float32, device=u0.device)
-            _emo_check(L.pde_emotion_backward(dref, _ptr(u0), _ptr(gout), _ptr(w6), _ptr(xs), _ptr(ys), _ptr(gin),
-                                              _ptr(gw), _ptr(ws), ws_bytes, _stream(u0.device)), d, "pde_emotion_backward")
+        gin, gw = _emotion_backward(ctx.plan, u0, w6, xs, ys, gout, ctx.needs_input_grad[0])
         return gin, gw, None, None, None
 
 
+@torch.compiler.assume_constant_result
+def _traced_emo_generic() -> bool:
+    return _emo_generic()
+
+
 def emotion_layer(u0, w6, xs, ys, cfg: EmoConfig):
-    return _EmotionFunction.apply(_autocast_to_fp32(u0), _autocast_to_fp32(w6), xs, ys, cfg)
+    u0, w6 = _autocast_to_fp32(u0), _autocast_to_fp32(w6)
+    if _traced(u0):
+        return torch.ops.pde_b200.emotion_fwd(u0, w6, xs, ys, cfg.N, cfg.Nt, cfg.dt, cfg.dx, cfg.dy, _traced_emo_generic())
+    return _EmotionFunction.apply(u0, w6, xs, ys, cfg)
 
 
 # ----------------------------------------------------------------------- explicit, zero ghosts
@@ -620,29 +702,54 @@ def _tiny_plan(cfg: TinyConfig, shape, device_index: int):
     return d, byref(d), _cabi.lib().pde_tiny_backward_workspace_bytes(byref(d))
 
 
+def _tiny_forward(u, alpha_base, channel_scaling, cfg: TinyConfig):
+    """The tiny_imagenet layer's forward pass, fp32 or bf16 planes after the input's dtype.  Returns
+    (out, plan, u, alpha_base, channel_scaling), the last three as the kernels read them."""
+    bf16 = isinstance(u, torch.Tensor) and u.is_cuda and u.dtype == torch.bfloat16
+    if not bf16:
+        _require_cuda(u, "ImprovedDiffusionLayer input")
+    L = _cabi.lib()
+    u = _contig(u)
+    al, sc = _contig(alpha_base.detach()), _contig(channel_scaling.detach())
+    if al.dtype != torch.float32 or sc.dtype != torch.float32:   # a module converted with .bfloat16(): the kernels take fp32 scalars
+        al, sc = al.float(), sc.float()
+    dev = u.device
+    plan = _tiny_plan(cfg, tuple(u.shape), dev.index if dev.index is not None else torch.cuda.current_device())
+    fwd = L.pde_tiny_forward_bf16 if bf16 else L.pde_tiny_forward
+    with _guard(u.device):
+        out = torch.empty_like(u)
+        _tiny_check(fwd(plan[1], _ptr(u), _ptr(al), _ptr(sc), _ptr(out), _stream(u.device)), plan[0], "pde_tiny_forward")
+    return out, plan, u, al, sc
+
+
+def _tiny_backward(plan, u, al, sc, gout, need_gin: bool):
+    """The tiny_imagenet layer's backward pass in u's dtype.  Returns (gin or None, g_alpha_base, g_channel_scaling)."""
+    L = _cabi.lib()
+    gout = _contig(gout)
+    if gout.dtype != u.dtype:
+        gout = gout.to(u.dtype)
+    C = u.shape[1]
+    d, dref, ws_bytes = plan
+    if ws_bytes == 0:
+        raise _tiny_refused(d)
+    with _guard(u.device):
+        ws = _bytes(ws_bytes, u.device)
+        gin = torch.empty_like(u) if need_gin else None
+        ga = torch.empty(C, dtype=torch.float32, device=u.device)
+        gs = torch.empty(C, dtype=torch.float32, device=u.device)
+        bwd = L.pde_tiny_backward_bf16 if u.dtype == torch.bfloat16 else L.pde_tiny_backward
+        _tiny_check(bwd(dref, _ptr(u), _ptr(gout), _ptr(al), _ptr(sc), _ptr(gin), _ptr(ga),
+                        _ptr(gs), _ptr(ws), ws_bytes, _stream(u.device)), d, "pde_tiny_backward")
+    return gin, ga, gs
+
+
 class _TinyFunction(torch.autograd.Function):
     """fp32 planes in, fp32 planes out -- or bfloat16 in, bfloat16 out (pde_tiny_*_bf16: the arithmetic, the
     parameters and their gradients stay fp32; the one bandwidth-bound layer of the reference moves half the bytes)."""
 
     @staticmethod
     def forward(ctx, u, alpha_base, channel_scaling, cfg: TinyConfig):
-        if isinstance(u, torch.Tensor) and u.is_cuda and u.dtype == torch.bfloat16:
-            ctx.bf16 = True
-        else:
-            ctx.bf16 = False
-            _require_cuda(u, "ImprovedDiffusionLayer input")
-        L = _cabi.lib()
-        u = _contig(u)
-        al, sc = _contig(alpha_base.detach()), _contig(channel_scaling.detach())
-        if al.dtype != torch.float32 or sc.dtype != torch.float32:   # a module converted with .bfloat16(): the kernels take fp32 scalars
-            al, sc = al.float(), sc.float()
-        dev = u.device
-        plan = _tiny_plan(cfg, tuple(u.shape), dev.index if dev.index is not None else torch.cuda.current_device())
-        fwd = L.pde_tiny_forward_bf16 if ctx.bf16 else L.pde_tiny_forward
-        with _guard(u.device):
-            out = torch.empty_like(u)
-            _tiny_check(fwd(plan[1], _ptr(u), _ptr(al), _ptr(sc), _ptr(out), _stream(u.device)), plan[0],
-                        "pde_tiny_forward")
+        out, plan, u, al, sc = _tiny_forward(u, alpha_base, channel_scaling, cfg)
         ctx.plan = plan
         ctx.save_for_backward(u, al, sc)
         return out
@@ -650,28 +757,15 @@ class _TinyFunction(torch.autograd.Function):
     @staticmethod
     def backward(ctx, gout):
         _no_double_backward("ImprovedDiffusionLayer")
-        L = _cabi.lib()
         u, al, sc = ctx.saved_tensors
-        gout = _contig(gout)
-        if gout.dtype != u.dtype:
-            gout = gout.to(u.dtype)
-        C = u.shape[1]
-        d, dref, ws_bytes = ctx.plan
-        if ws_bytes == 0:
-            raise _tiny_refused(d)
-        with _guard(u.device):
-            ws = _bytes(ws_bytes, u.device)
-            gin = torch.empty_like(u) if ctx.needs_input_grad[0] else None
-            ga = torch.empty(C, dtype=torch.float32, device=u.device)
-            gs = torch.empty(C, dtype=torch.float32, device=u.device)
-            bwd = L.pde_tiny_backward_bf16 if ctx.bf16 else L.pde_tiny_backward
-            _tiny_check(bwd(dref, _ptr(u), _ptr(gout), _ptr(al), _ptr(sc), _ptr(gin), _ptr(ga),
-                            _ptr(gs), _ptr(ws), ws_bytes, _stream(u.device)), d, "pde_tiny_backward")
-        return gin, ga, gs, None
+        return (*_tiny_backward(ctx.plan, u, al, sc, gout, ctx.needs_input_grad[0]), None)
 
 
 def tiny_layer(u, alpha_base, channel_scaling, cfg: TinyConfig):
-    return _TinyFunction.apply(_autocast_to_fp32(u), alpha_base, channel_scaling, cfg)
+    u = _autocast_to_fp32(u)
+    if _traced(u):
+        return torch.ops.pde_b200.tiny_fwd(u, alpha_base, channel_scaling, cfg.steps, cfg.dt, cfg.cmin, cfg.cmax, cfg.blend)
+    return _TinyFunction.apply(u, alpha_base, channel_scaling, cfg)
 
 
 # --------------------------------------------- tiny_imagenet's dormant scalar-coefficient methods
@@ -703,30 +797,28 @@ def _tiny_split_desc(mode: int, B: int, H: int, W: int, coeff_x: float, coeff_y:
     return d
 
 
+def _tiny_split_run(desc, u, what: str):
+    """One pde_tiny_split call on planes u; the forward pass and (on the upstream gradient) the backward pass."""
+    _require_cuda(u, what)
+    u = _contig(u)
+    out = torch.empty_like(u)
+    with _guard(u.device):
+        _cabi.check(_cabi.lib().pde_tiny_split(byref(desc), _ptr(u), _ptr(out), _stream(u.device)), "pde_tiny_split")
+    return out
+
+
 class _TinySplitFunction(torch.autograd.Function):
     """All five maps are linear in u with symmetric bands: backward is the same kernel on the gradient."""
 
     @staticmethod
     def forward(ctx, u, desc):
-        _require_cuda(u, "ImprovedDiffusionLayer dormant-path input")
-        u = _contig(u)
-        out = torch.empty_like(u)
-        with _guard(u.device):
-            _cabi.check(_cabi.lib().pde_tiny_split(byref(desc), _ptr(u), _ptr(out), _stream(u.device)), "pde_tiny_split")
         ctx.desc = desc
-        return out
+        return _tiny_split_run(desc, u, "ImprovedDiffusionLayer dormant-path input")
 
     @staticmethod
     def backward(ctx, gout):
         _no_double_backward("ImprovedDiffusionLayer dormant path")
-        gout = _contig(gout)
-        if gout.dtype != torch.float32:
-            gout = gout.float()
-        gin = torch.empty_like(gout)
-        with _guard(gout.device):
-            _cabi.check(_cabi.lib().pde_tiny_split(byref(ctx.desc), _ptr(gout), _ptr(gin), _stream(gout.device)),
-                        "pde_tiny_split")
-        return gin, None
+        return _tiny_split_run(ctx.desc, _float_grad(gout), "ImprovedDiffusionLayer dormant-path gradient"), None
 
 
 def tiny_split(method: str, u, coeff_x: float = 0.0, coeff_y: float = 0.0, dt: float = 0.01, eps: float = 1e-6):
@@ -738,5 +830,8 @@ def tiny_split(method: str, u, coeff_x: float = 0.0, coeff_y: float = 0.0, dt: f
     if H > 4096 or W > 4096:
         raise _cabi.PdeB200Error(f"{method}: planes up to 4096 x 4096 are built, got {H} x {W}")
     u = _autocast_to_fp32(u)
+    if _traced(u):
+        return torch.ops.pde_b200.tiny_split(u, TINY_SPLIT_MODES[method], float(coeff_x), float(coeff_y), float(dt),
+                                             float(eps))
     d = _tiny_split_desc(TINY_SPLIT_MODES[method], B, H, W, float(coeff_x), float(coeff_y), float(dt), float(eps))
     return _TinySplitFunction.apply(u, d)

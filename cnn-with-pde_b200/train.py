@@ -32,6 +32,9 @@ the all-reduce inside ONE graph instead (thread-local capture mode, after a warm
 capture stream); it takes the same optimiser steps (tests/test_gpu_multi.py) and the same time
 (1.264 ms), but a 220-step run of it stopped making progress on the two-GPU box here, so it is opt-in.
 
+--compile trains torch.compile(model, fullgraph=True) instead (the PDE layers are pde_b200:: custom ops in the
+graph, ops.py); it excludes --graph and works with --amp and the flat all-reduce.
+
 --amp reproduces the CIFAR scripts' mixed-precision recipe (cifar10.py:440,458-467): autocast,
 GradScaler.scale(loss).backward(), unscale_, clip_grad_norm_, scaler.step, scaler.update -- the PDE
 layers themselves stay fp32 (custom_fwd(cast_inputs=float32)).
@@ -138,10 +141,17 @@ def _dist_env():
 
 def run(model_name: str, batch: int, steps: int, warmup: int, graph: bool = False, amp: bool = False,
         seed: int = 1234, pool: int = 4, quiet: bool = False, sync: str = "flat", nccl_in_graph: bool = False,
-        no_dropout: bool = False, keep_model: bool = False, image_size: int | None = None):
+        no_dropout: bool = False, keep_model: bool = False, image_size: int | None = None, compile: bool = False):
     """Train `steps` timed steps (after `warmup`) of `model_name` at per-GPU batch `batch` on the
     current rank's GPU; returns a dict with whole-job img/s (max-over-ranks device time).
-    `image_size` (tiny only) trains on image_size x image_size images instead of the recipe's 64 x 64."""
+    `image_size` (tiny only) trains on image_size x image_size images instead of the recipe's 64 x 64.
+    `compile` trains torch.compile(model, fullgraph=True): the PDE layers enter the graph as pde_b200:: custom ops
+    (ops.py), the stock layers are Inductor's; the first warm-up step compiles."""
+    if compile and graph:
+        raise ValueError("--compile and --graph are exclusive: --compile traces the model with torch.compile, "
+                         "--graph captures the eager step in CUDA graphs")
+    if compile and sync == "ddp":
+        raise ValueError("--compile needs --sync flat")
     r = _recipes()[model_name]
     shape = r.shape
     if image_size is not None:
@@ -175,6 +185,8 @@ def run(model_name: str, batch: int, steps: int, warmup: int, graph: bool = Fals
         use_ddp = world > 1 and sync == "ddp"
         net = nn.parallel.DistributedDataParallel(model, device_ids=[local], gradient_as_bucket_view=True) \
             if use_ddp else model
+        if compile:
+            net = torch.compile(model, fullgraph=True)
         flat = None if use_ddp else FlatGradSync(model, world)
         opt = make_optimizer(model, r, capturable=graph)
     torch.cuda.current_stream().wait_stream(side)
@@ -278,7 +290,7 @@ def run(model_name: str, batch: int, steps: int, warmup: int, graph: bool = Fals
         "model": model_name, "image_shape": list(shape), "n_gpus": world, "batch_per_gpu": batch, "global_batch": batch * world,
         "steps": steps, "warmup": warmup, "ms_per_step": ms / max(steps, 1),
         "img_per_s": batch * world * steps / (ms * 1e-3) if ms > 0 else 0.0,
-        "loss": float(loss_out.item()), "cuda_graph": bool(graphs), "autocast": amp, "optimizer_steps": state["done"],
+        "loss": float(loss_out.item()), "cuda_graph": bool(graphs), "compiled": compile, "autocast": amp, "optimizer_steps": state["done"],
         "grad_sync": "none" if world == 1 else ("ddp" if use_ddp else (
             "flat all-reduce inside the CUDA graph" if len(graphs) == 1 else "flat all-reduce")),
         "grad_scaler": bool(amp),
@@ -301,6 +313,8 @@ def main(argv=None):
     ap.add_argument("--steps", type=int, default=50)
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--graph", action="store_true", help="capture the whole step in a CUDA graph")
+    ap.add_argument("--compile", action="store_true",
+                    help="train torch.compile(model, fullgraph=True); not with --graph (compiled in the first warm-up step)")
     ap.add_argument("--amp", action="store_true", help="autocast as in cifar10.py:459 (the PDE layer stays fp32)")
     ap.add_argument("--sync", choices=("flat", "ddp"), default="flat", help="gradient sync for N > 1")
     ap.add_argument("--nccl-in-graph", action="store_true", help="capture the all-reduce inside the CUDA graph (opt-in)")
@@ -310,7 +324,7 @@ def main(argv=None):
     batch = a.batch or _recipes()[a.model].batch
     t0 = time.time()
     out = run(a.model, batch, a.steps, a.warmup, graph=a.graph, amp=a.amp, seed=a.seed, sync=a.sync,
-              nccl_in_graph=a.nccl_in_graph, image_size=a.image_size)
+              nccl_in_graph=a.nccl_in_graph, image_size=a.image_size, compile=a.compile)
     if int(os.environ.get("RANK", "0")) == 0:
         print(f"# {out['img_per_s']:.0f} img/s on {out['n_gpus']} GPU(s), {out['ms_per_step']:.3f} ms/step, "
               f"wall {time.time() - t0:.1f} s", flush=True)
