@@ -41,6 +41,7 @@ EXPORTS = (
     "pde_emotion_backward_workspace_bytes", "pde_emotion_forward", "pde_emotion_backward",
     "pde_tiny_backward_workspace_bytes", "pde_tiny_forward", "pde_tiny_backward",
     "pde_tiny_split", "pde_tiny_forward_bf16", "pde_tiny_backward_bf16",
+    "pde_emotion_backward_workspace_bytes_bf16", "pde_emotion_forward_bf16", "pde_emotion_backward_bf16",
 )
 
 
@@ -132,6 +133,12 @@ def lib():
     L.pde_emotion_forward.argtypes = [POINTER(EmoDesc), fp, fp, fp, fp, fp, vp]
     L.pde_emotion_backward.restype = c_int
     L.pde_emotion_backward.argtypes = [POINTER(EmoDesc), fp, fp, fp, fp, fp, fp, fp, vp, c_size_t, vp]
+    L.pde_emotion_backward_workspace_bytes_bf16.restype = c_size_t
+    L.pde_emotion_backward_workspace_bytes_bf16.argtypes = [POINTER(EmoDesc)]
+    L.pde_emotion_forward_bf16.restype = c_int
+    L.pde_emotion_forward_bf16.argtypes = [POINTER(EmoDesc), fp, fp, fp, fp, fp, vp]
+    L.pde_emotion_backward_bf16.restype = c_int
+    L.pde_emotion_backward_bf16.argtypes = [POINTER(EmoDesc), fp, fp, fp, fp, fp, fp, fp, vp, c_size_t, vp]
     L.pde_tiny_backward_workspace_bytes.restype = c_size_t
     L.pde_tiny_backward_workspace_bytes.argtypes = [POINTER(TinyDesc)]
     L.pde_tiny_forward.restype = c_int

@@ -1,11 +1,30 @@
 // The row / column coefficient profiles of emotion_recognition.PDELayer, shared by every emotion kernel
-// (explicit.cu, emotion_tiled.cuh, emotion_halo.cu) so that all plane sizes use identical coefficient arithmetic.
+// (explicit.cu, emotion_tiled.cuh, emotion_halo.cu) so that all plane sizes use identical coefficient arithmetic,
+// and the plane loads / stores of those kernels in either I/O type.
 #pragma once
+
+#include <cuda_bf16.h>
 
 #include "common.cuh"
 
 namespace pde {
 namespace expl {
+
+// Plane I/O of the emotion kernels: fp32 or bf16 planes in HBM, fp32 everywhere else.  A bf16 value is widened
+// exactly on load; a result is rounded once, to nearest even, on its store.
+__device__ __forceinline__ float io_widen(float v) { return v; }
+__device__ __forceinline__ float io_widen(__nv_bfloat16 v) { return __bfloat162float(v); }
+template <typename T>
+__device__ __forceinline__ T io_round(float v) {
+    if constexpr (sizeof(T) == 4) return v;
+    else return __float2bfloat16_rn(v);
+}
+template <typename T>
+__device__ __forceinline__ float io_ldg(const T *p) { return io_widen(__ldg(p)); }
+template <typename T>
+__device__ __forceinline__ float io_ldcs(const T *p) { return io_widen(__ldcs(p)); }
+template <typename T>
+__device__ __forceinline__ void io_stcs(T *p, float v) { __stcs(p, io_round<T>(v)); }
 
 // a_i = 0.5 dt (w1 + w2 sin 2 pi y_i + w3 sin 4 pi y_i) / dx^2     emotion_recognition.py:76-77
 // b_j =     dt (w1 + w2 cos 2 pi x_j + w3 cos 4 pi x_j) / dy^2     emotion_recognition.py:79-80

@@ -20,7 +20,14 @@
 //      that one block owns per (sample slot, tile), summed in a fixed order across tiles, slots and chunks, then
 //      weighted by {1, sin 2 pi y, sin 4 pi y} / {1, cos 2 pi x, cos 4 pi x} in double: bit-reproducible.
 // Coefficients come from emo_profile, the routine every emotion kernel uses.  Indices into planes are 64-bit.
+//
+// I/O type T (fp32 or bf16) is that of u0, gout, out and grad_input only: windows, replayed states, adjoint planes,
+// edge sums and partials are fp32 / double in both.  In bf16 the adjoint kernel meets T at k = Nt - 1 (lambda^Nt =
+// gout) and at k = 0 (u^0, and lambda^0 = grad_input).  lambda^0 is rounded on its store except at the cells the
+// fold adds ghost-ring terms to (rows and columns 1 and N - 2): their fp32 values wait in a side buffer
+// [slot][4][N] until the fold adds those terms and rounds, so grad_input is rounded once, as in the fp32 order.
 #include <cstdio>
+#include <type_traits>
 
 #include "common.cuh"
 #include "emo_profile.cuh"
@@ -30,6 +37,9 @@ namespace pde {
 namespace halo {
 
 using expl::emo_profile;
+using expl::io_ldg;
+using expl::io_round;
+using expl::io_stcs;
 
 constexpr int kThreads = 256, kWarps = kThreads / 32;
 constexpr int kTH = 32, kTW = 64;      // output tile: a warp per row, 64 fp32 columns = two 128-byte lines
@@ -37,8 +47,9 @@ constexpr int kMaxChunk = 512;         // sample slots per backward chunk (bound
 
 struct FwdArgs {
     pde_emo_desc d;
-    const float *u0, *w6, *xs, *ys;
-    float *out;            // forward: u^K
+    const void *u0;        // I/O type
+    const float *w6, *xs, *ys;
+    void *out;             // forward: u^K, I/O type
     float *hist;           // replay: u^s of slot b at hist + (s - 1) * hstride + b * N^2, s = 1 ... K
     size_t hstride;
     int K, ntw, ntiles;
@@ -48,11 +59,12 @@ struct FwdArgs {
 struct AdjArgs {
     pde_emo_desc d;
     const float *w6, *xs, *ys;
-    const float *u0;       // the chunk's layer input: the ghost ring of every state
-    const float *uk;       // u^k of the chunk's slots (slot stride N^2)
-    const float *lin;      // lambda^{k+1}
-    float *lout;           // lambda^k (NULL: not needed)
+    const void *u0;        // the chunk's layer input: the ghost ring of every state (I/O type)
+    const void *uk;        // u^k of the chunk's slots (slot stride N^2): u0 at k = 0, else an fp32 plane
+    const void *lin;       // lambda^{k+1}: gout at k = Nt - 1, else an fp32 plane
+    void *lout;            // lambda^k (NULL: not needed): grad_input at k = 0, else an fp32 plane
     float *edge;           // [slot][top | bottom | left | right][N] (NULL: no grad_input)
+    float *side;           // bf16 grad_input: [slot][row 1 | row N - 2 | column 1 | column N - 2][N] fp32 lambda^0
     double *pa, *pb;       // [slot][tile column][N] row sums, [slot][tile row][N] column sums
     int ntw, nth, ntiles;
     long long nitems;
@@ -72,7 +84,8 @@ __device__ __forceinline__ void load_coeffs(const pde_emo_desc &d, const float *
 
 // window cell (i, j) <- plane cell (gr0 + i, gc0 + j): plane cells from `in`, ghost-ring cells (corners excluded)
 // reflected from `ring`, or zero where `ring` is NULL; every other cell zero.  Into w0, and w1 when set.
-__device__ __forceinline__ void load_window(float *w0, float *w1, const float *in, const float *ring, int gr0, int gc0,
+template <typename TI, typename TR>
+__device__ __forceinline__ void load_window(float *w0, float *w1, const TI *in, const TR *ring, int gr0, int gc0,
                                             int WH, int WW, int N) {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     for (int i = warp; i < WH; i += kWarps) {
@@ -84,8 +97,8 @@ __device__ __forceinline__ void load_window(float *w0, float *w1, const float *i
             const bool cin = (unsigned)gc < (unsigned)N, cg = gc == -1 || gc == N;
             const int sc = gc == -1 ? 1 : (gc == N ? N - 2 : gc);
             float v = 0.0f;
-            if (rin && cin) v = __ldg(in + (size_t)gr * N + gc);
-            else if (ring && ((rin && cg) || (rg && cin))) v = __ldg(ring + (size_t)sr * N + sc);
+            if (rin && cin) v = io_ldg(in + (size_t)gr * N + gc);
+            else if (ring && ((rin && cg) || (rg && cin))) v = io_ldg(ring + (size_t)sr * N + sc);
             w0[i * WW + j] = v;
             if (w1) w1[i * WW + j] = v;
         }
@@ -95,8 +108,8 @@ __device__ __forceinline__ void load_window(float *w0, float *w1, const float *i
 // one explicit step of the plane cells among window cells [lo, WH - lo) x [lo, WW - lo), in emo_step's
 // arithmetic: into dst when set, and the tile's cells (window cells [K, K + kTH) x [K, K + kTW)) into the plane g
 // when set (streaming stores for the layer output)
-template <bool kStream>
-__device__ __forceinline__ void fwd_step(const float *src, float *dst, float *g, int lo, int K, int WH, int WW, int gr0,
+template <bool kStream, typename TG>
+__device__ __forceinline__ void fwd_step(const float *src, float *dst, TG *g, int lo, int K, int WH, int WW, int gr0,
                                          int gc0, int N, const float *sa, const float *sb) {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     for (int i = lo + warp; i < WH - lo; i += kWarps) {
@@ -114,16 +127,16 @@ __device__ __forceinline__ void fwd_step(const float *src, float *dst, float *g,
             const float v = fmaf(sb[j], dc, fmaf(ai, dr, ct));
             if (dst) dst[i * WW + j] = v;
             if (g && row_tile && j >= K && j < K + kTW) {
-                if (kStream) __stcs(g + (size_t)gr * N + gc, v);
-                else g[(size_t)gr * N + gc] = v;
+                if (kStream) io_stcs(g + (size_t)gr * N + gc, v);
+                else g[(size_t)gr * N + gc] = io_round<TG>(v);
             }
         }
     }
 }
 
 // kReplay = false: the layer forward (K = Nt >= 1 steps into out); true: the backward's replay (K = Nt - 1 >= 1
-// steps, every state into hist)
-template <bool kReplay>
+// steps, every state into hist, fp32).  T: the I/O type of u0 and out
+template <bool kReplay, typename T>
 __global__ void __launch_bounds__(kThreads) emo_halo_fwd_kernel(const FwdArgs a) {
     extern __shared__ __align__(16) float smem[];
     const int N = a.d.N, K = a.K, WH = kTH + 2 * K, WW = kTW + 2 * K;
@@ -133,7 +146,7 @@ __global__ void __launch_bounds__(kThreads) emo_halo_fwd_kernel(const FwdArgs a)
         const long long b = item / a.ntiles;
         const int tile = (int)(item - b * a.ntiles);
         const int gr0 = (tile / a.ntw) * kTH - K, gc0 = (tile % a.ntw) * kTW - K;
-        const float *u = a.u0 + (size_t)b * NN;
+        const T *u = static_cast<const T *>(a.u0) + (size_t)b * NN;
         __syncthreads();   // the previous item is done with shared memory
         load_coeffs(a.d, a.w6, a.xs, a.ys, gr0, gc0, WH, WW, sa, sb);
         load_window(w0, K > 1 ? w1 : nullptr, u, u, gr0, gc0, WH, WW, N);
@@ -141,9 +154,13 @@ __global__ void __launch_bounds__(kThreads) emo_halo_fwd_kernel(const FwdArgs a)
         const float *src = w0;
         float *dst = w1;
         for (int s = 1; s <= K; ++s) {
-            float *g = kReplay ? a.hist + (size_t)(s - 1) * a.hstride + (size_t)b * NN
-                               : (s == K ? a.out + (size_t)b * NN : nullptr);
-            fwd_step<!kReplay>(src, s < K ? dst : nullptr, g, s, K, WH, WW, gr0, gc0, N, sa, sb);
+            if constexpr (kReplay) {
+                float *g = a.hist + (size_t)(s - 1) * a.hstride + (size_t)b * NN;
+                fwd_step<false>(src, s < K ? dst : nullptr, g, s, K, WH, WW, gr0, gc0, N, sa, sb);
+            } else {
+                T *g = s == K ? static_cast<T *>(a.out) + (size_t)b * NN : nullptr;
+                fwd_step<true>(src, s < K ? dst : nullptr, g, s, K, WH, WW, gr0, gc0, N, sa, sb);
+            }
             if (s < K) {
                 __syncthreads();
                 float *t = const_cast<float *>(src);
@@ -155,8 +172,14 @@ __global__ void __launch_bounds__(kThreads) emo_halo_fwd_kernel(const FwdArgs a)
 }
 
 // One reversed step on a tile: lambda^k = M^T lambda^{k+1} with lambda zero outside the plane, what flows into the
-// ghost ring, and this step's dA / dB terms.  Arithmetic of emo_bwd_kernel.
+// ghost ring, and this step's dA / dB terms.  Arithmetic of emo_bwd_kernel.  T: the I/O type; kLinIO: lambda^{k+1}
+// is gout (k = Nt - 1); kFirst: k = 0 (u^k is u0, lambda^k is grad_input).  fp32 I/O uses <float, false, false> for
+// every k: all its planes have one type.
+template <typename T, bool kLinIO, bool kFirst>
 __global__ void __launch_bounds__(kThreads) emo_halo_adj_kernel(const AdjArgs a) {
+    using TL = std::conditional_t<kLinIO, T, float>;
+    using TU = std::conditional_t<kFirst, T, float>;
+    constexpr bool kSide = kFirst && sizeof(T) == 2;   // lambda^0's fold cells stay fp32 until the fold
     constexpr int WH = kTH + 2, WW = kTW + 2;
     __shared__ float L[WH * WW], U[WH * WW], sa[WH], sb[WW];
     __shared__ float red[kWarps][kTW];
@@ -168,8 +191,9 @@ __global__ void __launch_bounds__(kThreads) emo_halo_adj_kernel(const AdjArgs a)
         const int gr0 = tr * kTH - 1, gc0 = tc * kTW - 1;
         __syncthreads();   // the previous item is done with shared memory
         load_coeffs(a.d, a.w6, a.xs, a.ys, gr0, gc0, WH, WW, sa, sb);
-        load_window(L, nullptr, a.lin + (size_t)b * NN, nullptr, gr0, gc0, WH, WW, N);
-        load_window(U, nullptr, a.uk + (size_t)b * NN, a.u0 + (size_t)b * NN, gr0, gc0, WH, WW, N);
+        load_window<TL, TL>(L, nullptr, static_cast<const TL *>(a.lin) + (size_t)b * NN, nullptr, gr0, gc0, WH, WW, N);
+        load_window(U, nullptr, static_cast<const TU *>(a.uk) + (size_t)b * NN, static_cast<const T *>(a.u0) + (size_t)b * NN,
+                    gr0, gc0, WH, WW, N);
         __syncthreads();
         float *e = a.edge ? a.edge + (size_t)b * 4 * N : nullptr;
         float fB[2] = {0.0f, 0.0f};
@@ -194,7 +218,17 @@ __global__ void __launch_bounds__(kThreads) emo_halo_adj_kernel(const AdjArgs a)
                     nv = fmaf(ap, pl[WW], nv);
                     nv = fmaf(sb[j - 1], pl[-1], nv);
                     nv = fmaf(sb[j + 1], pl[1], nv);
-                    if (a.lout) a.lout[(size_t)b * NN + (size_t)gr * N + gc] = nv;
+                    if (a.lout) {
+                        if (kSide && a.side && (gr == 1 || gr == N - 2 || gc == 1 || gc == N - 2)) {
+                            float *sd = a.side + (size_t)b * 4 * N;
+                            if (gr == 1) sd[gc] = nv;
+                            if (gr == N - 2) sd[N + gc] = nv;
+                            if (gc == 1) sd[2 * N + gr] = nv;
+                            if (gc == N - 2) sd[3 * N + gr] = nv;
+                        } else {
+                            static_cast<TU *>(a.lout)[(size_t)b * NN + (size_t)gr * N + gc] = io_round<TU>(nv);
+                        }
+                    }
                     if (e) {   // a_0 lam(0, j) / a_{N-1} lam(N-1, j) / b_0 lam(i, 0) / b_{N-1} lam(i, N-1): ghost ring
                         if (gr == 0) e[gc] += al;
                         if (gr == N - 1) e[N + gc] += al;
@@ -221,29 +255,36 @@ __global__ void __launch_bounds__(kThreads) emo_halo_adj_kernel(const AdjArgs a)
 }
 
 // grad_input += the ghost ring's adjoint through the reflection: rows 1 / N - 2 first, then columns 1 / N - 2
-// (the order of emo_bwd_kernel); a thread per edge cell
-__global__ void emo_halo_fold_kernel(int N, long long ncells, const float *__restrict__ edge, float *gin) {
+// (the order of emo_bwd_kernel); a thread per edge cell.  fp32 adds to grad_input in place; bf16 takes lambda^0 of
+// the cell from the side buffer and rounds the sum on its store
+template <typename T>
+__global__ void emo_halo_fold_kernel(int N, long long ncells, const float *__restrict__ edge,
+                                     const float *__restrict__ side, T *gin) {
     const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= ncells) return;
     const long long b = idx / (4 * N);
-    const int t = (int)(idx - b * 4 * N), side = t / N, q = t - side * N;
+    const int t = (int)(idx - b * 4 * N), sd = t / N, q = t - sd * N;
     const float *e = edge + (size_t)b * 4 * N;
-    float *g = gin + (size_t)b * N * N;
+    T *g = gin + (size_t)b * N * N;
+    auto lam0 = [&](int i, int j) {
+        if constexpr (sizeof(T) == 4) return g[(size_t)i * N + j];
+        else return side[(size_t)b * 4 * N + t];
+    };
     int i, j;
     float v;
-    if (side < 2) {
-        i = side == 0 ? 1 : N - 2;
+    if (sd < 2) {
+        i = sd == 0 ? 1 : N - 2;
         j = q;
-        v = g[(size_t)i * N + j] + e[side * N + j];
+        v = lam0(i, j) + e[sd * N + j];
         if (j == 1) v += e[2 * N + i];
         if (j == N - 2) v += e[3 * N + i];
     } else {
         if (q == 1 || q == N - 2) return;   // done with the rows above
         i = q;
-        j = side == 2 ? 1 : N - 2;
-        v = g[(size_t)i * N + j] + e[side * N + i];
+        j = sd == 2 ? 1 : N - 2;
+        v = lam0(i, j) + e[sd * N + i];
     }
-    g[(size_t)i * N + j] = v;
+    g[(size_t)i * N + j] = io_round<T>(v);
 }
 
 // tot[i] = dA_i (i < N), tot[N + j] = dB_j: double, summed over slots then tiles in a fixed order
@@ -289,15 +330,17 @@ __global__ void __launch_bounds__(kFinishThreads) emo_halo_finish_kernel(pde_emo
 
 // ------------------------------------------------------------------------------------------ host
 // Backward workspace, from a 256-byte aligned base: tot [2N] doubles, pa [chunk][ntw][N] and pb [chunk][nth][N]
-// doubles, edges [chunk][4][N] floats, state / adjoint planes [Nt][chunk][N][N] floats (none for Nt <= 1).
-// chunk = the sample slots whose share fits kHaloWorkspaceCap, at least 1, at most min(B, kMaxChunk).
+// doubles, edges [chunk][4][N] floats, state / adjoint planes [Nt][chunk][N][N] floats (none for Nt <= 1), and for
+// bf16 I/O the side buffer [chunk][4][N] floats.  chunk = the sample slots whose share of the fp32 layout fits
+// kHaloWorkspaceCap, at least 1, at most min(B, kMaxChunk): the same in both I/O types, so that the partial sums
+// are added in the same order.
 struct Layout {
     int ntw, nth, ntiles, planes;
     long long chunk;
-    size_t pa, pb, edge, plane, bytes;
+    size_t pa, pb, edge, plane, side, bytes;
 };
 
-static Layout layout(const pde_emo_desc *d) {
+static Layout layout(const pde_emo_desc *d, int io_bytes) {
     Layout l;
     const size_t N = (size_t)d->N, NN = N * N;
     l.ntw = (d->N + kTW - 1) / kTW;
@@ -314,11 +357,12 @@ static Layout layout(const pde_emo_desc *d) {
     l.pb = l.pa + (size_t)c * l.ntw * N * sizeof(double);
     l.edge = l.pb + (size_t)c * l.nth * N * sizeof(double);
     l.plane = l.edge + (size_t)c * 4 * N * sizeof(float);
-    l.bytes = 256 + l.plane + (size_t)c * l.planes * NN * sizeof(float);
+    l.side = l.plane + (size_t)c * l.planes * NN * sizeof(float);
+    l.bytes = 256 + l.side + (io_bytes == 2 ? (size_t)c * 4 * N * sizeof(float) : 0);
     return l;
 }
 
-size_t emo_halo_workspace_bytes(const pde_emo_desc *d) { return layout(d).bytes; }
+size_t emo_halo_workspace_bytes(const pde_emo_desc *d, int io_bytes) { return layout(d, io_bytes).bytes; }
 
 struct Launch {
     const void *kern;
@@ -341,11 +385,12 @@ static int plan_launch(const void *kern, size_t smem, long long nitems, const De
     return PDE_OK;
 }
 
+template <typename T>
 static int plan_fwd(const FwdArgs &a, bool replay, const DeviceProps &props, Launch *p) {
     const size_t WH = kTH + 2 * a.K, WW = kTW + 2 * a.K;
     const size_t smem = (WH + WW + (a.K > 1 ? 2 : 1) * WH * WW) * sizeof(float);
-    const void *kern = replay ? reinterpret_cast<const void *>(emo_halo_fwd_kernel<true>)
-                              : reinterpret_cast<const void *>(emo_halo_fwd_kernel<false>);
+    const void *kern = replay ? reinterpret_cast<const void *>(emo_halo_fwd_kernel<true, T>)
+                              : reinterpret_cast<const void *>(emo_halo_fwd_kernel<false, T>);
     return plan_launch(kern, smem, a.nitems, props, p);
 }
 
@@ -355,7 +400,7 @@ static int launch(const Launch &p, void *args, cudaStream_t st) {
     return cuda_last_error();
 }
 
-static FwdArgs fwd_args(const pde_emo_desc *d, const float *u0, const float *w6, const float *xs, const float *ys, int K,
+static FwdArgs fwd_args(const pde_emo_desc *d, const void *u0, const float *w6, const float *xs, const float *ys, int K,
                         long long nsamples) {
     FwdArgs a{};
     a.d = *d; a.u0 = u0; a.w6 = w6; a.xs = xs; a.ys = ys; a.K = K;
@@ -365,9 +410,23 @@ static FwdArgs fwd_args(const pde_emo_desc *d, const float *u0, const float *w6,
     return a;
 }
 
-int emo_halo_forward(const pde_emo_desc *d, const float *u0, const float *w6, const float *xs, const float *ys,
-                     float *out, const DeviceProps &props, cudaStream_t st) {
-    const size_t bytes = (size_t)d->B * d->N * d->N * sizeof(float);
+// the adjoint kernel of reversed step k: fp32 I/O has one for every k
+template <typename T>
+static const void *adj_kernel(bool lin_io, bool first) {
+    if constexpr (sizeof(T) == 4) {
+        return reinterpret_cast<const void *>(emo_halo_adj_kernel<float, false, false>);
+    } else {
+        if (lin_io) return first ? reinterpret_cast<const void *>(emo_halo_adj_kernel<T, true, true>)
+                                 : reinterpret_cast<const void *>(emo_halo_adj_kernel<T, true, false>);
+        return first ? reinterpret_cast<const void *>(emo_halo_adj_kernel<T, false, true>)
+                     : reinterpret_cast<const void *>(emo_halo_adj_kernel<T, false, false>);
+    }
+}
+
+template <typename T>
+int emo_halo_forward(const pde_emo_desc *d, const T *u0, const float *w6, const float *xs, const float *ys, T *out,
+                     const DeviceProps &props, cudaStream_t st) {
+    const size_t bytes = (size_t)d->B * d->N * d->N * sizeof(T);
     if (d->Nt == 0) {
         if (debug_enabled()) fprintf(stderr, "[pde_b200] emotion halo fwd plan: B=%d N=%d Nt=0 copy\n", d->B, d->N);
         PDE_CUDA_TRY(cudaMemcpyAsync(out, u0, bytes, cudaMemcpyDeviceToDevice, st));
@@ -376,7 +435,7 @@ int emo_halo_forward(const pde_emo_desc *d, const float *u0, const float *w6, co
     FwdArgs a = fwd_args(d, u0, w6, xs, ys, d->Nt, d->B);
     a.out = out;
     Launch p;
-    int rc = plan_fwd(a, false, props, &p);
+    int rc = plan_fwd<T>(a, false, props, &p);
     if (rc) return rc;
     if (debug_enabled())
         fprintf(stderr, "[pde_b200] emotion halo fwd plan: B=%d N=%d Nt=%d tile=%dx%d window=%dx%d smem=%zu regs=%d "
@@ -385,21 +444,23 @@ int emo_halo_forward(const pde_emo_desc *d, const float *u0, const float *w6, co
     return launch(p, &a, st);
 }
 
-int emo_halo_backward(const pde_emo_desc *d, const float *u0, const float *gout, const float *w6, const float *xs,
-                      const float *ys, float *gin, float *g_w6, void *workspace, size_t workspace_bytes,
+template <typename T>
+int emo_halo_backward(const pde_emo_desc *d, const T *u0, const T *gout, const float *w6, const float *xs,
+                      const float *ys, T *gin, float *g_w6, void *workspace, size_t workspace_bytes,
                       const DeviceProps &props, cudaStream_t st) {
-    const Layout l = layout(d);
+    const Layout l = layout(d, (int)sizeof(T));
     if (!workspace || workspace_bytes < l.bytes) return PDE_ERR_WORKSPACE;
     char *base = reinterpret_cast<char *>((reinterpret_cast<uintptr_t>(workspace) + 255u) & ~(uintptr_t)255u);
     double *tot = reinterpret_cast<double *>(base), *pa = reinterpret_cast<double *>(base + l.pa),
            *pb = reinterpret_cast<double *>(base + l.pb);
     float *edge = reinterpret_cast<float *>(base + l.edge), *planes = reinterpret_cast<float *>(base + l.plane);
+    float *side = sizeof(T) == 2 ? reinterpret_cast<float *>(base + l.side) : nullptr;
     const int N = d->N, Nt = d->Nt;
     const size_t NN = (size_t)N * N;
     const long long B = d->B, chunk = l.chunk;
     int rc;
     PDE_CUDA_TRY(cudaMemsetAsync(pa, 0, (size_t)chunk * (l.ntw + l.nth) * N * sizeof(double), st));   // pa, pb
-    if (Nt == 0 && gin) PDE_CUDA_TRY(cudaMemcpyAsync(gin, gout, (size_t)B * NN * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    if (Nt == 0 && gin) PDE_CUDA_TRY(cudaMemcpyAsync(gin, gout, (size_t)B * NN * sizeof(T), cudaMemcpyDeviceToDevice, st));
     auto plane = [&](int p) { return planes + (size_t)p * chunk * NN; };
     Launch rp{}, ap{};
     AdjArgs q{};
@@ -407,29 +468,30 @@ int emo_halo_backward(const pde_emo_desc *d, const float *u0, const float *gout,
     q.ntw = l.ntw; q.nth = l.nth; q.ntiles = l.ntiles;
     for (long long b0 = 0; Nt > 0 && b0 < B; b0 += chunk) {
         const long long nb = B - b0 < chunk ? B - b0 : chunk;
-        const float *u = u0 + (size_t)b0 * NN, *g = gout + (size_t)b0 * NN;
-        float *gi = gin ? gin + (size_t)b0 * NN : nullptr;
+        const T *u = u0 + (size_t)b0 * NN, *g = gout + (size_t)b0 * NN;
+        T *gi = gin ? gin + (size_t)b0 * NN : nullptr;
         if (gi) PDE_CUDA_TRY(cudaMemsetAsync(edge, 0, (size_t)nb * 4 * N * sizeof(float), st));
         if (Nt >= 2) {   // u^1 ... u^{Nt-1} into planes 0 ... Nt - 2
             FwdArgs r = fwd_args(d, u, w6, xs, ys, Nt - 1, nb);
             r.hist = planes;
             r.hstride = (size_t)chunk * NN;
-            if ((rc = plan_fwd(r, true, props, &rp))) return rc;
+            if ((rc = plan_fwd<T>(r, true, props, &rp))) return rc;
             if ((rc = launch(rp, &r, st))) return rc;
         }
         q.u0 = u;
         q.edge = gi ? edge : nullptr;
+        q.side = gi ? side : nullptr;
         q.nitems = nb * l.ntiles;
-        if ((rc = plan_launch(reinterpret_cast<const void *>(emo_halo_adj_kernel), 0, q.nitems, props, &ap))) return rc;
         for (int k = Nt - 1; k >= 0; --k) {
-            q.uk = k == 0 ? u : plane(k - 1);
-            q.lin = k + 1 == Nt ? g : plane(k + 1 == Nt - 1 ? Nt - 1 : k + 1);
-            q.lout = k == 0 ? gi : plane(k == Nt - 1 ? Nt - 1 : k);
+            q.uk = k == 0 ? static_cast<const void *>(u) : plane(k - 1);
+            q.lin = k + 1 == Nt ? static_cast<const void *>(g) : plane(k + 1 == Nt - 1 ? Nt - 1 : k + 1);
+            q.lout = k == 0 ? static_cast<void *>(gi) : plane(k == Nt - 1 ? Nt - 1 : k);
+            if ((rc = plan_launch(adj_kernel<T>(k + 1 == Nt, k == 0), 0, q.nitems, props, &ap))) return rc;
             if ((rc = launch(ap, &q, st))) return rc;
         }
         if (gi) {
             const long long ncells = nb * 4 * N;
-            emo_halo_fold_kernel<<<(unsigned)((ncells + 255) / 256), 256, 0, st>>>(N, ncells, edge, gi);
+            emo_halo_fold_kernel<T><<<(unsigned)((ncells + 255) / 256), 256, 0, st>>>(N, ncells, edge, side, gi);
             if ((rc = cuda_last_error())) return rc;
         }
     }
@@ -445,6 +507,16 @@ int emo_halo_backward(const pde_emo_desc *d, const float *u0, const float *gout,
     emo_halo_finish_kernel<<<1, kFinishThreads, 0, st>>>(*d, tot, xs, ys, g_w6);
     return cuda_last_error();
 }
+
+template int emo_halo_forward<float>(const pde_emo_desc *, const float *, const float *, const float *, const float *,
+                                     float *, const DeviceProps &, cudaStream_t);
+template int emo_halo_forward<__nv_bfloat16>(const pde_emo_desc *, const __nv_bfloat16 *, const float *, const float *,
+                                             const float *, __nv_bfloat16 *, const DeviceProps &, cudaStream_t);
+template int emo_halo_backward<float>(const pde_emo_desc *, const float *, const float *, const float *, const float *,
+                                      const float *, float *, float *, void *, size_t, const DeviceProps &, cudaStream_t);
+template int emo_halo_backward<__nv_bfloat16>(const pde_emo_desc *, const __nv_bfloat16 *, const __nv_bfloat16 *,
+                                              const float *, const float *, const float *, __nv_bfloat16 *, float *, void *,
+                                              size_t, const DeviceProps &, cudaStream_t);
 
 }  // namespace halo
 }  // namespace pde

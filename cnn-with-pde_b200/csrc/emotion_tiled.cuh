@@ -21,6 +21,10 @@
 // in fp32 within a step and in double across steps and planes.  What flows into the frozen ghost ring is summed
 // over the steps (top / bottom rows in registers, left / right columns in shared memory by the edge
 // lanes) and folded back through the reflection at the end.
+//
+// Planes in HBM (u0, gout, out, gin) are fp32 or bf16 (template T): a bf16 cell is widened on load (the frozen
+// ghosts with it), a result is rounded once on its store (grad_input after the ghost-ring fold); registers, the
+// history and every sum are fp32 / double in both instantiations.
 #pragma once
 
 namespace pde {
@@ -69,14 +73,14 @@ struct Tile {
 
 // load a lane's block of the plane and capture the frozen ghosts (reflect padding of u^0):
 // gedge = top ghost row (= row 1) in the upper half, bottom ghost row (= row N - 2) in the lower
-template <int N>
-__device__ __forceinline__ void tile_load(const float *__restrict__ src, int half, int sub, int r0, int j0,
+template <int N, typename T>
+__device__ __forceinline__ void tile_load(const T *__restrict__ src, int half, int sub, int r0, int j0,
                                           float (&u)[N / 2][N / 16], float (&gedge)[N / 16], float *gl, float *gr) {
     constexpr int CW = Tile<N>::CW, RH = Tile<N>::RH;
 #pragma unroll
     for (int r = 0; r < RH; ++r)
 #pragma unroll
-        for (int c = 0; c < CW; ++c) u[r][c] = __ldg(src + (r0 + r) * N + j0 + c);
+        for (int c = 0; c < CW; ++c) u[r][c] = io_ldg(src + (r0 + r) * N + j0 + c);
 #pragma unroll
     for (int c = 0; c < CW; ++c) gedge[c] = half == 0 ? u[1][c] : u[RH - 2][c];
     // left ghost = column 1, right ghost = column N - 2 of u^0
@@ -140,7 +144,7 @@ __device__ __forceinline__ void tile_step(float (&u)[N / 2][N / 16], const float
     }
 }
 
-template <int N>
+template <int N, typename T>
 __global__ void __launch_bounds__(kTileWarps * 32) emo_fwd_tiled(const EmoArgs a) {
     constexpr int CW = Tile<N>::CW, RH = Tile<N>::RH;
     __shared__ __align__(16) TileShared sh;
@@ -157,19 +161,19 @@ __global__ void __launch_bounds__(kTileWarps * 32) emo_fwd_tiled(const EmoArgs a
     for (int plane = blockIdx.x * kTileWarps + warp; plane < a.d.B; plane += gridDim.x * kTileWarps) {
         const size_t off = (size_t)plane * N * N;
         float u[RH][CW], gedge[CW];
-        tile_load<N>(a.u0 + off, half, sub, r0, j0, u, gedge, gl, gr);
+        tile_load<N>(static_cast<const T *>(a.u0) + off, half, sub, r0, j0, u, gedge, gl, gr);
 #pragma unroll 1
         for (int k = 0; k < a.d.Nt; ++k) tile_step<N>(u, gedge, b, sh.a + 1 + r0, gl + r0, gr + r0, half, sub);
-        float *o = a.out + off;
+        T *o = static_cast<T *>(a.out) + off;
 #pragma unroll
         for (int r = 0; r < RH; ++r)
 #pragma unroll
-            for (int c = 0; c < CW; ++c) __stcs(o + (r0 + r) * N + j0 + c, u[r][c]);
+            for (int c = 0; c < CW; ++c) io_stcs(o + (r0 + r) * N + j0 + c, u[r][c]);
         __syncwarp();   // the ghost columns are rewritten by the next plane
     }
 }
 
-template <int N>
+template <int N, typename T>
 __global__ void __launch_bounds__(kTileWarps * 32) emo_bwd_tiled(const EmoArgs a, float *hist_all, double *part) {
     constexpr int CW = Tile<N>::CW, RH = Tile<N>::RH;
     constexpr int HROW = CW * 32;               // floats per history row
@@ -227,7 +231,7 @@ __global__ void __launch_bounds__(kTileWarps * 32) emo_bwd_tiled(const EmoArgs a
         }
         {   // ------------------------------ replay: u^kb .. u^{ke-1} into the history
             float u[RH][CW];
-            tile_load<N>(a.u0 + off, half, sub, r0, j0, u, gedge, gl, gr);
+            tile_load<N>(static_cast<const T *>(a.u0) + off, half, sub, r0, j0, u, gedge, gl, gr);
 #pragma unroll 1
             for (int k = 0; k < ke; ++k) {
                 if (k >= kb) {
@@ -246,11 +250,11 @@ __global__ void __launch_bounds__(kTileWarps * 32) emo_bwd_tiled(const EmoArgs a
 #pragma unroll
                 for (int c = 0; c < CW; ++c) lam[r][c] = __ldcg(park + (r * CW + c) * 32);
         } else {
-            const float *go = a.gout + off;
+            const T *go = static_cast<const T *>(a.gout) + off;
 #pragma unroll
             for (int r = 0; r < RH; ++r)
 #pragma unroll
-                for (int c = 0; c < CW; ++c) lam[r][c] = __ldcs(go + (r0 + r) * N + j0 + c);
+                for (int c = 0; c < CW; ++c) lam[r][c] = io_ldcs(go + (r0 + r) * N + j0 + c);
         }
         // ------------------------------ reverse over the segment
 #pragma unroll 1   // the body is 24 unrolled rows; more copies only thrash the instruction cache
@@ -353,7 +357,7 @@ __global__ void __launch_bounds__(kTileWarps * 32) emo_bwd_tiled(const EmoArgs a
         }
         __syncwarp();
         if (a.need_gin) {
-            float *gi = a.gin + off;
+            T *gi = static_cast<T *>(a.gin) + off;
 #pragma unroll
             for (int r = 0; r < RH; ++r)
 #pragma unroll
@@ -369,7 +373,7 @@ __global__ void __launch_bounds__(kTileWarps * 32) emo_bwd_tiled(const EmoArgs a
                         const float e = sh.gadj[warp][r][half * 16 + 15];
                         v += (sub == (N - 2) / CW) ? e : 0.0f;
                     }
-                    __stcs(gi + (r0 + r) * N + j0 + c, v);
+                    io_stcs(gi + (r0 + r) * N + j0 + c, v);
                 }
         }
         __syncwarp();
@@ -440,36 +444,38 @@ static size_t emo_tiled_workspace_bytes(const pde_emo_desc *d, int sm_count) {
     return emo_tiled_hist_floats(d, grid) * sizeof(float) + (size_t)grid * kTileWarps * kTilePartDoubles * sizeof(double) + 512;
 }
 
-template <int N>
+template <int N, typename T>
 static int emo_tiled_forward_n(const EmoArgs &a, int sm_count, cudaStream_t st) {
     int per_sm = 1;   // persistent grid: the blocks resident at once (register bound)
-    int rc = cached_occupancy(reinterpret_cast<const void *>(emo_fwd_tiled<N>), kTileWarps * 32, 0, &per_sm);
+    int rc = cached_occupancy(reinterpret_cast<const void *>(emo_fwd_tiled<N, T>), kTileWarps * 32, 0, &per_sm);
     if (rc) return rc;
     const int want = (a.d.B + kTileWarps - 1) / kTileWarps;
     int grid = sm_count * per_sm;
     if (grid > want) grid = want;
-    emo_fwd_tiled<N><<<grid, kTileWarps * 32, 0, st>>>(a);
+    emo_fwd_tiled<N, T><<<grid, kTileWarps * 32, 0, st>>>(a);
     return cuda_last_error();
 }
 
+template <typename T>
 static int emo_tiled_forward(const EmoArgs &a, int sm_count, cudaStream_t st) {
     switch (a.d.N) {
-        case 16: return emo_tiled_forward_n<16>(a, sm_count, st);
-        case 32: return emo_tiled_forward_n<32>(a, sm_count, st);
-        case 48: return emo_tiled_forward_n<48>(a, sm_count, st);
+        case 16: return emo_tiled_forward_n<16, T>(a, sm_count, st);
+        case 32: return emo_tiled_forward_n<32, T>(a, sm_count, st);
+        case 48: return emo_tiled_forward_n<48, T>(a, sm_count, st);
         default: return PDE_ERR_UNSUPPORTED;
     }
 }
 
+template <typename T>
 static int emo_tiled_backward(const EmoArgs &a, int sm_count, void *workspace, const float *xs, float *g_w6,
                               cudaStream_t st) {
     const int grid = emo_tiled_bwd_grid(&a.d, sm_count);
     float *hist = reinterpret_cast<float *>((reinterpret_cast<uintptr_t>(workspace) + 255u) & ~(uintptr_t)255u);
     double *part = reinterpret_cast<double *>(hist + emo_tiled_hist_floats(&a.d, grid));
     switch (a.d.N) {
-        case 16: emo_bwd_tiled<16><<<grid, kTileWarps * 32, 0, st>>>(a, hist, part); break;
-        case 32: emo_bwd_tiled<32><<<grid, kTileWarps * 32, 0, st>>>(a, hist, part); break;
-        case 48: emo_bwd_tiled<48><<<grid, kTileWarps * 32, 0, st>>>(a, hist, part); break;
+        case 16: emo_bwd_tiled<16, T><<<grid, kTileWarps * 32, 0, st>>>(a, hist, part); break;
+        case 32: emo_bwd_tiled<32, T><<<grid, kTileWarps * 32, 0, st>>>(a, hist, part); break;
+        case 48: emo_bwd_tiled<48, T><<<grid, kTileWarps * 32, 0, st>>>(a, hist, part); break;
         default: return PDE_ERR_UNSUPPORTED;
     }
     int rc = cuda_last_error();

@@ -399,20 +399,25 @@ static bool tiny_aligned(const void *p, bool tiled, int io_bytes) {
 constexpr int kEmoRows = 8;       // rows per thread strip
 constexpr int kEmoMaxN = 64;
 
+// u0, gout, out, gin: fp32 or bf16 planes (every emotion kernel is instantiated for both I/O types); the six
+// weights, the x / y buffers, the arithmetic and the weight gradients are fp32 either way
 struct EmoArgs {
     pde_emo_desc d;
-    const float *u0, *gout, *w6, *xs, *ys;
-    float *out, *gin, *part;
+    const void *u0, *gout;
+    const float *w6, *xs, *ys;
+    void *out, *gin;
+    float *part;
     int need_gin;
 };
 
 // interior of the padded plane <- global plane (coalesced), then the reflected ghost ring
-__device__ __forceinline__ void emo_load_padded(const float *__restrict__ g, float *buf, float *buf2, int N,
+template <typename T>
+__device__ __forceinline__ void emo_load_padded(const T *__restrict__ g, float *buf, float *buf2, int N,
                                                 int tid, int nthreads) {
     const int M = N + 2;
     for (int idx = tid; idx < N * N; idx += nthreads) {
         const int i = idx / N, j = idx - i * N;
-        buf[(i + 1) * M + j + 1] = __ldcs(g + idx);
+        buf[(i + 1) * M + j + 1] = io_ldcs(g + idx);
     }
     __syncthreads();
     if (tid < N) {
@@ -445,6 +450,7 @@ __device__ __forceinline__ void emo_step(const float *src, float *dst, const flo
     }
 }
 
+template <typename T>
 __global__ void emo_fwd_kernel(const EmoArgs a) {
     extern __shared__ __align__(16) float smem[];
     const pde_emo_desc &d = a.d;
@@ -457,17 +463,17 @@ __global__ void emo_fwd_kernel(const EmoArgs a) {
     const bool active = r0 < N;
     const float bj = sb[j];
     for (int plane = blockIdx.x; plane < d.B; plane += gridDim.x) {
-        emo_load_padded(a.u0 + (size_t)plane * N * N, buf0, buf1, N, tid, nthreads);
+        emo_load_padded(static_cast<const T *>(a.u0) + (size_t)plane * N * N, buf0, buf1, N, tid, nthreads);
         float *src = buf0, *dst = buf1;
         for (int k = 0; k < d.Nt; ++k) {
             if (active) emo_step(src, dst, sa, N, j, r0, r1, bj);
             __syncthreads();
             float *tmp = src; src = dst; dst = tmp;
         }
-        float *o = a.out + (size_t)plane * N * N;
+        T *o = static_cast<T *>(a.out) + (size_t)plane * N * N;
         for (int idx = tid; idx < N * N; idx += nthreads) {
             const int i = idx / N, jj = idx - i * N;
-            __stcs(o + idx, src[(i + 1) * M + jj + 1]);
+            io_stcs(o + idx, src[(i + 1) * M + jj + 1]);
         }
         __syncthreads();
     }
@@ -479,6 +485,7 @@ __global__ void emo_fwd_kernel(const EmoArgs a) {
 // on a padded lam plane whose ring stays zero; what would flow into the (frozen, input-derived)
 // ghost ring is summed over all steps in four edge vectors and folded back through the
 // reflection at the end.  dA_i += lam * d2_row u, dB_j += lam * d2_col u per thread.
+template <typename T>
 __global__ void emo_bwd_kernel(const EmoArgs a) {
     extern __shared__ __align__(16) float smem[];
     const pde_emo_desc &d = a.d;
@@ -508,7 +515,7 @@ __global__ void emo_bwd_kernel(const EmoArgs a) {
 
     for (int plane = blockIdx.x; plane < d.B; plane += gridDim.x) {
         // forward states: hist[k] = u^k, k = 0..Nt-1 (hist[Nt] receives u^Nt, unused)
-        emo_load_padded(a.u0 + (size_t)plane * N * N, hist, hist + PP, N, tid, nthreads);
+        emo_load_padded(static_cast<const T *>(a.u0) + (size_t)plane * N * N, hist, hist + PP, N, tid, nthreads);
         for (int k = 0; k < Nt; ++k) {
             float *nxt = hist + (size_t)(k + 1) * PP;
             if (k > 0 && tid < N) {  // ring of the next plane (hist[1] already has it)
@@ -519,10 +526,10 @@ __global__ void emo_bwd_kernel(const EmoArgs a) {
             if (active) emo_step(hist + (size_t)k * PP, nxt, sa + 1, N, j, r0, r1, bj);
             __syncthreads();
         }
-        const float *go = a.gout + (size_t)plane * N * N;
+        const T *go = static_cast<const T *>(a.gout) + (size_t)plane * N * N;
         for (int idx = tid; idx < N * N; idx += nthreads) {
             const int i = idx / N, jj = idx - i * N;
-            lam0[(i + 1) * M + jj + 1] = __ldcs(go + idx);
+            lam0[(i + 1) * M + jj + 1] = io_ldcs(go + idx);
         }
         if (tid < 4 * kEmoMaxN) edge[tid] = 0.f;
         for (int idx = tid + nthreads; idx < 4 * kEmoMaxN; idx += nthreads) edge[idx] = 0.f;
@@ -563,7 +570,7 @@ __global__ void emo_bwd_kernel(const EmoArgs a) {
             float *tmp = lsrc; lsrc = ldst; ldst = tmp;
         }
         if (a.need_gin) {
-            float *gi = a.gin + (size_t)plane * N * N;
+            T *gi = static_cast<T *>(a.gin) + (size_t)plane * N * N;
             for (int idx = tid; idx < N * N; idx += nthreads) {
                 const int i = idx / N, jj = idx - i * N;
                 float v = lsrc[(i + 1) * M + jj + 1];
@@ -571,7 +578,7 @@ __global__ void emo_bwd_kernel(const EmoArgs a) {
                 if (i == N - 2) v += edge[kEmoMaxN + jj];
                 if (jj == 1) v += edge[2 * kEmoMaxN + i];
                 if (jj == N - 2) v += edge[3 * kEmoMaxN + i];
-                __stcs(gi + idx, v);
+                io_stcs(gi + idx, v);   // rounded once, after the ghost-ring fold
             }
         }
         __syncthreads();
@@ -783,10 +790,12 @@ extern "C" int pde_tiny_backward_bf16(const pde_tiny_desc *d, const void *u, con
 }
 
 // --------------------------------------------------------------------------------------- emotion
-extern "C" size_t pde_emotion_backward_workspace_bytes(const pde_emo_desc *d) {
+// Both I/O types take the same route, grid and chunking for a descriptor, so their fp32 arithmetic and summation
+// order are the same: a bf16 call gives bit for bit the fp32 call on the widened planes, rounded to bf16.
+static size_t emo_workspace_bytes(const pde_emo_desc *d, int io_bytes) {
     bool halo;
     if (emo_route(d, &halo) != PDE_OK) return 0;
-    if (halo) return halo::emo_halo_workspace_bytes(d);
+    if (halo) return halo::emo_halo_workspace_bytes(d, io_bytes);
     DeviceProps props;
     if (query_props(&props) != PDE_OK) return 0;
     const size_t generic = (size_t)props.sm_count * 4 * 2 * kEmoMaxN * sizeof(float) + 256;
@@ -797,34 +806,49 @@ extern "C" size_t pde_emotion_backward_workspace_bytes(const pde_emo_desc *d) {
     return generic;
 }
 
-extern "C" int pde_emotion_forward(const pde_emo_desc *d, const float *u0, const float *w6, const float *xs,
-                                   const float *ys, float *out, void *stream) {
+extern "C" size_t pde_emotion_backward_workspace_bytes(const pde_emo_desc *d) { return emo_workspace_bytes(d, 4); }
+
+extern "C" size_t pde_emotion_backward_workspace_bytes_bf16(const pde_emo_desc *d) { return emo_workspace_bytes(d, 2); }
+
+// planes need their element alignment only (bf16: 2 bytes)
+template <typename T>
+static bool emo_aligned(const void *p) {
+    return (reinterpret_cast<uintptr_t>(p) % sizeof(T)) == 0;
+}
+
+template <typename T>
+static int emotion_forward_impl(const pde_emo_desc *d, const void *u0, const float *w6, const float *xs, const float *ys,
+                                void *out, void *stream) {
     bool halo;
     int rc = emo_route(d, &halo);
     if (rc) return rc;
     if (d->B == 0) return PDE_OK;   // empty batch: a no-op, its tensor pointers may be NULL
     if (!u0 || !w6 || !xs || !ys || !out) return PDE_ERR_INVALID;
+    if (!emo_aligned<T>(u0) || !emo_aligned<T>(out)) return PDE_ERR_INVALID;
     DeviceProps props;
     rc = query_props(&props);
     if (rc) return rc;
-    if (halo) return halo::emo_halo_forward(d, u0, w6, xs, ys, out, props, static_cast<cudaStream_t>(stream));
+    if (halo)
+        return halo::emo_halo_forward<T>(d, static_cast<const T *>(u0), w6, xs, ys, static_cast<T *>(out), props,
+                                         static_cast<cudaStream_t>(stream));
     EmoArgs a{};
     a.d = *d; a.u0 = u0; a.w6 = w6; a.xs = xs; a.ys = ys; a.out = out;
     if (emo_use_tiled(d))
-        return emo_tiled_forward(a, props.sm_count, static_cast<cudaStream_t>(stream));
+        return emo_tiled_forward<T>(a, props.sm_count, static_cast<cudaStream_t>(stream));
     const size_t smem = emo_fwd_smem(d);
     const int threads = emo_threads(d->N);
     long grid = (long)props.sm_count * 6;
     if (grid > d->B) grid = d->B;
-    rc = kernel_info(reinterpret_cast<const void *>(emo_fwd_kernel), smem, nullptr);
+    rc = kernel_info(reinterpret_cast<const void *>(emo_fwd_kernel<T>), smem, nullptr);
     if (rc) return rc;
-    emo_fwd_kernel<<<(int)grid, threads, smem, static_cast<cudaStream_t>(stream)>>>(a);
+    emo_fwd_kernel<T><<<(int)grid, threads, smem, static_cast<cudaStream_t>(stream)>>>(a);
     return cuda_last_error();
 }
 
-extern "C" int pde_emotion_backward(const pde_emo_desc *d, const float *u0, const float *gout, const float *w6,
-                                    const float *xs, const float *ys, float *gin, float *g_w6, void *workspace,
-                                    size_t workspace_bytes, void *stream) {
+template <typename T>
+static int emotion_backward_impl(const pde_emo_desc *d, const void *u0, const void *gout, const float *w6, const float *xs,
+                                 const float *ys, void *gin, float *g_w6, void *workspace, size_t workspace_bytes,
+                                 void *stream) {
     bool halo;
     int rc = emo_route(d, &halo);
     if (rc) return rc;
@@ -835,17 +859,19 @@ extern "C" int pde_emotion_backward(const pde_emo_desc *d, const float *u0, cons
         return PDE_OK;
     }
     if (!u0 || !gout || !w6 || !xs || !ys) return PDE_ERR_INVALID;
+    if (!emo_aligned<T>(u0) || !emo_aligned<T>(gout) || !emo_aligned<T>(gin)) return PDE_ERR_INVALID;
     DeviceProps props;
     rc = query_props(&props);
     if (rc) return rc;
     if (halo)
-        return halo::emo_halo_backward(d, u0, gout, w6, xs, ys, gin, g_w6, workspace, workspace_bytes, props, st);
+        return halo::emo_halo_backward<T>(d, static_cast<const T *>(u0), static_cast<const T *>(gout), w6, xs, ys,
+                                          static_cast<T *>(gin), g_w6, workspace, workspace_bytes, props, st);
     if (emo_use_tiled(d)) {
         if (!workspace || workspace_bytes < emo_tiled_workspace_bytes(d, props.sm_count)) return PDE_ERR_WORKSPACE;
         EmoArgs t{};
         t.d = *d; t.u0 = u0; t.gout = gout; t.w6 = w6; t.xs = xs; t.ys = ys; t.gin = gin;
         t.need_gin = gin != nullptr;
-        return emo_tiled_backward(t, props.sm_count, workspace, xs, g_w6, st);
+        return emo_tiled_backward<T>(t, props.sm_count, workspace, xs, g_w6, st);
     }
     const size_t smem = emo_bwd_smem(d);
     if (smem > (size_t)props.max_smem_optin) return PDE_ERR_UNSUPPORTED;
@@ -856,11 +882,33 @@ extern "C" int pde_emotion_backward(const pde_emo_desc *d, const float *u0, cons
     a.d = *d; a.u0 = u0; a.gout = gout; a.w6 = w6; a.xs = xs; a.ys = ys; a.gin = gin;
     a.need_gin = gin != nullptr;
     a.part = reinterpret_cast<float *>((reinterpret_cast<uintptr_t>(workspace) + 255u) & ~(uintptr_t)255u);
-    rc = kernel_info(reinterpret_cast<const void *>(emo_bwd_kernel), smem, nullptr);
+    rc = kernel_info(reinterpret_cast<const void *>(emo_bwd_kernel<T>), smem, nullptr);
     if (rc) return rc;
-    emo_bwd_kernel<<<grid, emo_threads(d->N), smem, st>>>(a);
+    emo_bwd_kernel<T><<<grid, emo_threads(d->N), smem, st>>>(a);
     rc = cuda_last_error();
     if (rc) return rc;
     emo_finish_kernel<<<1, kEmoMaxN, 0, st>>>(*d, grid, a.part, xs, ys, g_w6);
     return cuda_last_error();
+}
+
+extern "C" int pde_emotion_forward(const pde_emo_desc *d, const float *u0, const float *w6, const float *xs,
+                                   const float *ys, float *out, void *stream) {
+    return emotion_forward_impl<float>(d, u0, w6, xs, ys, out, stream);
+}
+
+extern "C" int pde_emotion_backward(const pde_emo_desc *d, const float *u0, const float *gout, const float *w6,
+                                    const float *xs, const float *ys, float *gin, float *g_w6, void *workspace,
+                                    size_t workspace_bytes, void *stream) {
+    return emotion_backward_impl<float>(d, u0, gout, w6, xs, ys, gin, g_w6, workspace, workspace_bytes, stream);
+}
+
+extern "C" int pde_emotion_forward_bf16(const pde_emo_desc *d, const void *u0, const float *w6, const float *xs,
+                                        const float *ys, void *out, void *stream) {
+    return emotion_forward_impl<__nv_bfloat16>(d, u0, w6, xs, ys, out, stream);
+}
+
+extern "C" int pde_emotion_backward_bf16(const pde_emo_desc *d, const void *u0, const void *gout, const float *w6,
+                                         const float *xs, const float *ys, void *gin, float *g_w6, void *workspace,
+                                         size_t workspace_bytes, void *stream) {
+    return emotion_backward_impl<__nv_bfloat16>(d, u0, gout, w6, xs, ys, gin, g_w6, workspace, workspace_bytes, stream);
 }

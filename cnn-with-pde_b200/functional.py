@@ -591,50 +591,76 @@ class EmoConfig:
         return _cabi.EmoDesc(B, self.N, self.Nt, f(0.5 * self.dt), f(self.dt), f(self.dx ** 2), f(self.dy ** 2), 0)
 
 
+def _emo_refused(d) -> "_cabi.PdeB200Error":
+    return _cabi.PdeB200Error(
+        f"unsupported emotion PDELayer configuration (N={d.N}, Nt={d.Nt}); supported: N <= 64 with any Nt (the "
+        "backward pass while a sample's step states fit a block's shared memory); 65 ... 4096 with Nt <= 16")
+
+
 def _emo_check(rc: int, d, what: str):
     if rc == _cabi.ERR_UNSUPPORTED:
-        raise _cabi.PdeB200Error(
-            f"unsupported emotion PDELayer configuration (N={d.N}, Nt={d.Nt}); supported: N <= 64 with any Nt (the "
-            "backward pass while a sample's step states fit a block's shared memory); 65 ... 4096 with Nt <= 16")
+        raise _emo_refused(d)
     _cabi.check(rc, what)
 
 
 @functools.lru_cache(maxsize=256)
-def _emo_plan(cfg: EmoConfig, B: int, generic: bool, device_index: int):
-    """(descriptor, its byref, backward workspace bytes) of a call: depends on nothing else."""
+def _emo_plan(cfg: EmoConfig, B: int, generic: bool, device_index: int, bf16: bool = False):
+    """(descriptor, its byref, backward workspace bytes for the planes' dtype) of a call: depends on nothing else."""
     d = cfg.desc(B)
     d.tuning = _cabi.EMO_TUNE_GENERIC if generic else 0
-    return d, byref(d), _cabi.lib().pde_emotion_backward_workspace_bytes(byref(d))
+    L = _cabi.lib()
+    ws = L.pde_emotion_backward_workspace_bytes_bf16 if bf16 else L.pde_emotion_backward_workspace_bytes
+    return d, byref(d), ws(byref(d))
+
+
+def _emo_bf16(u0) -> bool:
+    """Whether the emotion layer's planes take the bf16 entry points; anything but fp32 or bf16 CUDA planes is refused."""
+    if isinstance(u0, torch.Tensor) and u0.is_cuda and u0.dtype != torch.float32:
+        if u0.dtype == torch.bfloat16:
+            return True
+        raise RuntimeError(f"PDELayer input: expected float32 or bfloat16, got {u0.dtype}")
+    _require_cuda(u0, "PDELayer input")
+    return False
+
+
+def _fp32(t):
+    """The six weights and the x / y buffers as the kernels read them, whatever the module's dtype: fp32, contiguous."""
+    return _contig(t if t.dtype == torch.float32 else t.float())
 
 
 def _emotion_forward(u0, w6, xs, ys, cfg: EmoConfig, generic: bool):
-    """The emotion layer's forward pass.  Returns (out, plan, u0, w6, xs, ys), the last four as the kernels read them."""
-    _require_cuda(u0, "PDELayer input")
+    """The emotion layer's forward pass, fp32 or bf16 planes after the input's dtype.  Returns (out, plan, u0, w6, xs,
+    ys), the last four as the kernels read them."""
+    bf16 = _emo_bf16(u0)
     L = _cabi.lib()
     dev = u0.device
-    plan = _emo_plan(cfg, u0.shape[0], generic, dev.index if dev.index is not None else torch.cuda.current_device())
+    plan = _emo_plan(cfg, u0.shape[0], generic, dev.index if dev.index is not None else torch.cuda.current_device(), bf16)
     u0 = _contig(u0)
-    w6c, xs, ys = _contig(w6.detach()), _contig(xs), _contig(ys)
+    w6c, xs, ys = _fp32(w6.detach()), _fp32(xs), _fp32(ys)
+    fwd = L.pde_emotion_forward_bf16 if bf16 else L.pde_emotion_forward
     with _guard(u0.device):
         out = torch.empty_like(u0)
-        _emo_check(L.pde_emotion_forward(plan[1], _ptr(u0), _ptr(w6c), _ptr(xs), _ptr(ys), _ptr(out), _stream(u0.device)),
+        _emo_check(fwd(plan[1], _ptr(u0), _ptr(w6c), _ptr(xs), _ptr(ys), _ptr(out), _stream(u0.device)),
                    plan[0], "pde_emotion_forward")
     return out, plan, u0, w6c, xs, ys
 
 
 def _emotion_backward(plan, u0, w6, xs, ys, gout, need_gin: bool):
-    """The emotion layer's backward pass.  Returns (gin or None, g_w6)."""
+    """The emotion layer's backward pass in u0's dtype (plan for that dtype).  Returns (gin or None, g_w6 in fp32)."""
     L = _cabi.lib()
-    gout = _float_grad(gout)
+    gout = _contig(gout)
+    if gout.dtype != u0.dtype:
+        gout = gout.to(u0.dtype)
     d, dref, ws_bytes = plan
     if ws_bytes == 0:
-        raise _tiny_refused(d)
+        raise _emo_refused(d)
+    bwd = L.pde_emotion_backward_bf16 if u0.dtype == torch.bfloat16 else L.pde_emotion_backward
     with _guard(u0.device):
         ws = _bytes(ws_bytes, u0.device)
         gin = torch.empty_like(u0) if need_gin else None
         gw = torch.empty(6, dtype=torch.float32, device=u0.device)
-        _emo_check(L.pde_emotion_backward(dref, _ptr(u0), _ptr(gout), _ptr(w6), _ptr(xs), _ptr(ys), _ptr(gin),
-                                          _ptr(gw), _ptr(ws), ws_bytes, _stream(u0.device)), d, "pde_emotion_backward")
+        _emo_check(bwd(dref, _ptr(u0), _ptr(gout), _ptr(w6), _ptr(xs), _ptr(ys), _ptr(gin), _ptr(gw), _ptr(ws), ws_bytes,
+                       _stream(u0.device)), d, "pde_emotion_backward")
     return gin, gw
 
 
@@ -643,6 +669,9 @@ def _emo_generic() -> bool:
 
 
 class _EmotionFunction(torch.autograd.Function):
+    """fp32 planes in, fp32 planes out -- or bfloat16 in, bfloat16 out (pde_emotion_*_bf16: the weights, the buffers,
+    the arithmetic and the weight gradient stay fp32)."""
+
     @staticmethod
     def forward(ctx, u0, w6, xs, ys, cfg: EmoConfig):
         out, plan, u0, w6c, xs, ys = _emotion_forward(u0, w6, xs, ys, cfg, _emo_generic())
@@ -664,7 +693,12 @@ def _traced_emo_generic() -> bool:
 
 
 def emotion_layer(u0, w6, xs, ys, cfg: EmoConfig):
-    u0, w6 = _autocast_to_fp32(u0), _autocast_to_fp32(w6)
+    u0 = _autocast_to_fp32(u0)
+    # the kernels read the weights and the x / y buffers as fp32 whatever the module's dtype; w6 is widened under
+    # autograd, so a converted module's weight gradients come back in its own dtype
+    if w6.dtype != torch.float32:
+        w6 = w6.float()
+    xs, ys = (t if t.dtype == torch.float32 else t.float() for t in (xs, ys))
     if _traced(u0):
         return torch.ops.pde_b200.emotion_fwd(u0, w6, xs, ys, cfg.N, cfg.Nt, cfg.dt, cfg.dx, cfg.dy, _traced_emo_generic())
     return _EmotionFunction.apply(u0, w6, xs, ys, cfg)

@@ -2,7 +2,7 @@
 FakeTensor / meta-device shape inference see of the layers.
 
     adi_fwd / adi_bwd            implicit layers (both kernel families: the route is chosen inside the op)
-    emotion_fwd / emotion_bwd    emotion_recognition.PDELayer
+    emotion_fwd / emotion_bwd    emotion_recognition.PDELayer (fp32 or bf16 planes, after the input)
     tiny_fwd / tiny_bwd          tiny_imagenet.ImprovedDiffusionLayer (fp32 or bf16 planes, after the input)
     tiny_split                   its dormant split methods (self-adjoint: the backward pass is the same op)
 
@@ -132,15 +132,17 @@ def _(u0, w6, xs, ys, N, Nt, dt, dx, dy, generic):
 @torch.library.custom_op("pde_b200::emotion_bwd", mutates_args=())
 def emotion_bwd(gout: Tensor, u0: Tensor, w6: Tensor, xs: Tensor, ys: Tensor, N: int, Nt: int, dt: float, dx: float,
                 dy: float, generic: bool, need_gin: bool) -> tuple[Tensor, Tensor]:
-    """(grad_input or an empty tensor, the gradient of the six weights)."""
-    plan = F._emo_plan(F.EmoConfig(N=N, Nt=Nt, dt=dt, dx=dx, dy=dy), u0.shape[0], generic, _device_index(u0.device))
-    gin, gw = F._emotion_backward(plan, F._contig(u0), F._contig(w6), F._contig(xs), F._contig(ys), gout, need_gin)
+    """(grad_input or an empty tensor, the gradient of the six weights); grad_input in u0's dtype, the weight
+    gradient fp32."""
+    plan = F._emo_plan(F.EmoConfig(N=N, Nt=Nt, dt=dt, dx=dx, dy=dy), u0.shape[0], generic, _device_index(u0.device),
+                       u0.dtype == torch.bfloat16)
+    gin, gw = F._emotion_backward(plan, F._contig(u0), F._fp32(w6), F._fp32(xs), F._fp32(ys), gout, need_gin)
     return (u0.new_empty(0) if gin is None else gin), gw
 
 
 @emotion_bwd.register_fake
 def _(gout, u0, w6, xs, ys, N, Nt, dt, dx, dy, generic, need_gin):
-    return u0.new_empty(u0.shape if need_gin else (0,)), u0.new_empty((6,))
+    return u0.new_empty(u0.shape if need_gin else (0,)), u0.new_empty((6,), dtype=torch.float32)
 
 
 def _emotion_setup(ctx, inputs, output):

@@ -246,6 +246,21 @@ int pde_emotion_backward(const pde_emo_desc *d, const float *u0, const float *go
                          const float *xs, const float *ys, float *gin, float *g_w6,
                          void *workspace, size_t workspace_bytes, void *stream);
 
+/* bf16-I/O variants: u0, out, gout, gin are bfloat16 planes in the same layout, 2-byte aligned on every
+ * route; w6, xs, ys and g_w6 stay fp32, and so does all arithmetic.  Every value is widened on load and
+ * every result rounded once, to nearest even, on its final store (grad_input after the ghost-ring
+ * terms are added), and a descriptor takes the same kernels, grid and chunking as in fp32, so a bf16
+ * call gives bit for bit the fp32 call on the widened planes, rounded to bf16.  Same domain, same
+ * PDE_ERR_UNSUPPORTED, B = 0 a no-op (the backward then zeroes g_w6).  The backward workspace is what
+ * pde_emotion_backward_workspace_bytes_bf16 answers: above N = 64 the fp32 size plus chunk * 4 * N
+ * floats, where grad_input's cells on rows and columns 1 and N - 2 wait in fp32 for the fold. */
+size_t pde_emotion_backward_workspace_bytes_bf16(const pde_emo_desc *d);
+int pde_emotion_forward_bf16(const pde_emo_desc *d, const void *u0, const float *w6, const float *xs,
+                             const float *ys, void *out, void *stream);
+int pde_emotion_backward_bf16(const pde_emo_desc *d, const void *u0, const void *gout, const float *w6,
+                              const float *xs, const float *ys, void *gin, float *g_w6,
+                              void *workspace, size_t workspace_bytes, void *stream);
+
 /* ---------------------------------------------------------------------------------------
  * Explicit family, zero ghosts, per-channel scalars.  Replaces ImprovedDiffusionLayer.forward
  * and simple_diffusion_step, tiny_imagenet.py:34-72.
