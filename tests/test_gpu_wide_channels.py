@@ -46,9 +46,9 @@ def _tame(c, params, gain=0.2):
 ORACLE_MAX_C = 8   # the oracle's adjoint holds the channel-matrix gradient in an 8 x 8 array
 
 
-def _expected(c, params, io, need_gin, dtype):
+def _expected(c, params, io, need_gin, dtype, nthreads=0):
     if c.shape[0] <= ORACLE_MAX_C:
-        return runners.run_oracle(c, params=params, io=io, dtype=dtype, need_gin=need_gin)
+        return runners.run_oracle(c, params=params, io=io, dtype=dtype, need_gin=need_gin, nthreads=nthreads)
     want = AR.run(c, params=params, io=io, dtype=dtype, need_gin=need_gin, device="cuda")
     if dtype == np.float32:   # and the outputs against the oracle's forward, which takes any C
         y = runners.run_oracle(c, params=params, io=io, dtype=np.float32, forward_only=True)["y"]
@@ -57,9 +57,10 @@ def _expected(c, params, io, need_gin, dtype):
     return want
 
 
-def _judge(got, c, params, io, need_gin, what):
-    want32 = _expected(c, params, io, need_gin, np.float32)
-    want64 = _expected(c, params, io, need_gin, np.float64)
+def _judge(got, c, params, io, need_gin, what, nthreads=0):
+    """Returns the error of every key against the fp32 reference."""
+    want32 = _expected(c, params, io, need_gin, np.float32, nthreads)
+    want64 = _expected(c, params, io, need_gin, np.float64, nthreads)
     got = {k: v for k, v in got.items() if v is not None}
     want32 = {k: want32[k] for k in got}
     errs = runners.compare(got, want32)
@@ -71,6 +72,7 @@ def _judge(got, c, params, io, need_gin, what):
         else:
             assert k in SCALARS, (what, k, errs[k])
             assert e64[k] <= 3.0 * r64[k] + TOL, (what, k, errs[k], e64[k], r64[k])
+    return errs
 
 
 def _check(c, params=None, need_gin=True):
